@@ -2,7 +2,7 @@
 """Headline benchmark: NDMPS encode + truncate-to-chi + reconstruct voxels/s on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload cfg1|cfg2|cfg3|cfg4|cfg5b|cfg5] [--chi 64]
+                    [--workload cfg1|cfg2|cfg3|cfg4|cfg5b|cfg5] [--chi 64] [--dump-outputs DIR]
 
 A step is one pass of the hot path over one BATCH of independent synthetic tensors (the reference's
 benchmark loop walks a list of tensors, ``evaluation/benchmark.py:73-76,117-118``); ``--in-flight``
@@ -33,6 +33,8 @@ streams).  Workloads (BASELINE.json configs, SURVEY section 8d):
 * ``--impl reference``: the CPU oracle (numpy/LAPACK float64 restatement of the reference path - the
   reference itself cannot be imported without quimb / scikit-image) on the SAME workload, one tensor
   per step, all host threads, rank 0 only; the number of steps is bounded by ``--ref-budget`` seconds.
+* ``--dump-outputs DIR``: what the device-resident path computed in its last timed step, as .npy files (see
+  ``write_outputs``).  Inputs are seeded, so two builds run with the same arguments can be compared file by file.
 """
 from __future__ import annotations
 
@@ -56,6 +58,8 @@ for _p in (str(ROOT), str(ROOT / "img-compression-mps_b200")):
 METRIC = "ndmps_encode_truncate_reconstruct_voxels_per_s"
 UNIT = "voxels/s"
 L2_BYTES = 126 << 20          # B200 L2: timed iterations either flush it or work on inputs several times larger
+DUMP_LIMIT = 64 << 20         # --dump-outputs writes at most this many bytes
+DUMP_SEED = 0
 
 CHI_SWEEP = (128, 64, 32, 16, 8)
 WORKLOADS = {
@@ -345,6 +349,38 @@ def device_unit(workload, chi):
         return None, out
 
     return {"cfg1": with_metrics, "cfg2": chi_sweep, "cfg3": plain, "cfg4": with_metrics, "cfg5b": plain}[workload]
+
+
+def dump_positions(nvox, batch):
+    """Flat voxel positions of each reconstruction that --dump-outputs keeps: all of them when a step's tensors fit in
+    3/4 of DUMP_LIMIT (counted as float64), otherwise the same subset for every tensor: one position drawn from
+    numpy's default_rng(DUMP_SEED) in each of `keep` equal strata of the flat index, so two runs or two builds keep
+    the same voxels, spread over the whole tensor, without materialising a permutation of all of them."""
+    keep = max(1, (DUMP_LIMIT * 3 // 4) // (8 * batch))
+    if keep >= nvox:
+        return np.arange(nvox)
+    edges = np.arange(keep + 1, dtype=np.int64) * nvox // keep
+    return edges[:-1] + (np.random.default_rng(DUMP_SEED).random(keep) * np.diff(edges)).astype(np.int64)
+
+
+def write_outputs(out_dir, results):
+    """--dump-outputs: ``results`` holds, for each tensor of the last timed step, (its kept reconstruction voxels or
+    None, the unit's scalars).  One DIR/<name>.npy per name with the step's tensors along axis 0: ``reconstruction``
+    (float32), then every scalar and bond list of the unit as float64 (``<name>_chi<c>`` for the chi sweep's entries)."""
+    arrays = {}
+    if results[0][0] is not None:
+        arrays["reconstruction"] = np.stack([r.cpu().numpy() for r, _ in results])
+    for key, first in results[0][1].items():
+        for sub in (list(first) if isinstance(first, dict) else [None]):
+            vals = [s[key] if sub is None else s[key][sub] for _, s in results]
+            arrays[key if sub is None else f"{key}_chi{sub}"] = np.asarray(vals, dtype=np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT}-byte limit (fewer --volumes)")
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out / f"{name}.npy", a)
 
 
 def oracle_unit(workload, chi):
@@ -659,9 +695,19 @@ def run_ours(args):
     flush_buf = torch.empty(512 * 1024 * 1024, dtype=torch.uint8, device="cuda")   # > 126 MB L2
     pipe = VolumePipeline(workers=in_flight)
     unit = device_unit(workload, chi)
+    keep = torch.from_numpy(dump_positions(nvox, batch)).cuda() if args.dump_outputs else None
 
-    def step():
-        pipe.map(lambda v: unit(v)[1], vols)
+    def timed(item):
+        if isinstance(item, tuple):  # last step with --dump-outputs: the unit + one gather of the kept voxels
+            rec, scal = unit(item[0])
+            return (None if rec is None else rec.reshape(-1).index_select(0, keep)), scal
+        return unit(item)[1]
+
+    def step_items(last_step):
+        return [(v,) for v in vols] if last_step and keep is not None else vols
+
+    def step(last_step=False):
+        return pipe.map(timed, step_items(last_step))
 
     info = None
     for _ in range(max(args.warmup, 3)):
@@ -687,22 +733,25 @@ def run_ours(args):
         if back_to_back:
             flush_buf.fill_(0)
             starts[0].record()
-            pipe.map(lambda v: unit(v)[1], vols * args.steps)
+            last = pipe.map(timed, vols * (args.steps - 1) + step_items(True))[-batch:]
             stops[0].record()
         else:
             for i in range(args.steps):
                 flush_buf.fill_(i & 0xFF)                            # evict L2 (outside the event pair)
                 starts[i].record()
-                step()                                               # workers wait for the submitting stream, then are joined
+                last = step(i == args.steps - 1)                     # workers wait for the submitting stream, then are joined
                 stops[i].record()
         barrier()
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, last)
+    del last
     n_pairs = 1 if back_to_back else args.steps
     total_ms = max_over_ranks(sum(s.elapsed_time(e) for s, e in zip(starts[:n_pairs], stops[:n_pairs])))
     launches = pipe.launch_count() - launches0
     value = world * batch * nvox * passes * args.steps / (total_ms * 1e-3)
 
     # ---- one tensor at a time, stage profiler on: latency and the per-stage rooflines ----------------------
-    p_steps = max(1, min(args.steps, 5))
+    p_steps = args.steps
     p_starts = [torch.cuda.Event(enable_timing=True) for _ in range(p_steps)]
     p_stops = [torch.cuda.Event(enable_timing=True) for _ in range(p_steps)]
     ctx.profile(True)
@@ -822,6 +871,10 @@ def run_ours(args):
     }
     if sharded is not None:
         result["sharded"] = sharded
+    if keep is not None:
+        result["run"]["dump_outputs"] = {
+            "dir": args.dump_outputs, "voxels_kept_per_tensor": int(keep.numel()),
+            "note": "the last timed step also gathered the kept voxels of every reconstruction (one small kernel per tensor)"}
     if world == 1 and not args.no_cpu:
         rate, per, n_run = time_oracle(workload, chi, hosts[0], 1, 0.0)
         result["cpu_baseline"] = {
@@ -868,7 +921,7 @@ def sharded_volume_record(args, chi, torch, dist, ctx, flush_buf, world, rank, l
     if world > 1:
         dist.all_reduce(err2)
     err = float(torch.sqrt(err2[0] / err2[1]))
-    steps = max(3, min(args.steps, 10))
+    steps = args.steps
     starts = [torch.cuda.Event(enable_timing=True) for _ in range(steps)]
     stops = [torch.cuda.Event(enable_timing=True) for _ in range(steps)]
     launches0 = ctx.launch_count()
@@ -914,7 +967,9 @@ def sharded_volume_record(args, chi, torch, dist, ctx, flush_buf, world, rank, l
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5,
+                    help="timed steps of every record; --impl reference stops sooner when --ref-budget runs out and "
+                         "reports the steps it ran")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="cfg3", choices=sorted(WORKLOADS))
@@ -925,7 +980,15 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--per-step", action="store_true", help="one event pair and an L2 flush per step (drains the pipeline between steps)")
     ap.add_argument("--ref-budget", type=float, default=150.0, help="--impl reference: seconds of timed oracle work")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write what the last one computed (rank 0) as DIR/<name>.npy, at most 64 MB: "
+                         "each tensor's reconstruction (a fixed seeded sample of its voxels when the step's are too many) "
+                         "and the unit's scalars and bond dimensions")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "cfg5"):
+        ap.error("--dump-outputs needs --impl ours and a timed workload (not cfg5)")
     if args.workload == "cfg5":
         if int(os.environ.get("RANK", "0")) == 0:
             degenerate_report(args)

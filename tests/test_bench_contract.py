@@ -86,3 +86,56 @@ def test_roofline_entries_follow_the_contract():
     assert "latency-bound" in roof["eig"]["bound_note"]
     tiles = bench.build_rooflines(per_call, 11.2, work, nvox, peaks, 35.3, 1.1e9, True, False)
     assert "permute_tiled_kernel" in tiles["permute"]["kernel"]
+
+
+def test_dump_outputs_layout_and_size_limit(tmp_path):
+    """--dump-outputs: the kept voxels are fixed by a seed, every workload's default step fits in 64 MB, and each
+    output of the unit becomes one float32 / float64 .npy with the step's tensors along axis 0."""
+    import numpy as np
+    import torch
+
+    import bench
+    for key, wl in bench.WORKLOADS.items():
+        pos = bench.dump_positions(int(np.prod(wl["shape"])), wl["batch"])
+        assert 8 * wl["batch"] * pos.size <= bench.DUMP_LIMIT, key
+        assert np.all(np.diff(pos) > 0) and np.array_equal(pos, bench.dump_positions(int(np.prod(wl["shape"])), wl["batch"]))
+    assert np.array_equal(bench.dump_positions(1000, 4), np.arange(1000))
+    rec = torch.arange(12, dtype=torch.float32)
+    bench.write_outputs(tmp_path / "plain", [(rec + i, {"bond_dims": [8, 64, 8], "site_dims": [8, 8, 8, 8]}) for i in range(3)])
+    got = {p.stem: np.load(p) for p in (tmp_path / "plain").iterdir() if p.suffix == ".npy"}
+    assert sorted(p.name for p in (tmp_path / "plain").iterdir()) == ["bond_dims.npy", "reconstruction.npy", "site_dims.npy"]
+    assert got["reconstruction"].dtype == np.float32 and got["reconstruction"].shape == (3, 12) and got["reconstruction"][2, 0] == 2
+    assert got["bond_dims"].dtype == np.float64 and got["bond_dims"].tolist() == [[8, 64, 8]] * 3
+    sweep = {"site_dims": [8] * 8, "bond_dims": {128: [8, 64], 8: [8, 8]}, "fidelity": {128: 1.0, 8: 0.9}, "psnr": {128: 50.0, 8: 30.0}}
+    bench.write_outputs(tmp_path / "sweep", [(None, sweep)] * 2)
+    assert sorted(p.name for p in (tmp_path / "sweep").iterdir()) == [
+        "bond_dims_chi128.npy", "bond_dims_chi8.npy", "fidelity_chi128.npy", "fidelity_chi8.npy", "psnr_chi128.npy", "psnr_chi8.npy",
+        "site_dims.npy"]
+    with pytest.raises(SystemExit):
+        bench.write_outputs(tmp_path / "big", [(torch.zeros(bench.DUMP_LIMIT // 4 + 1), {})])
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_what_the_timed_path_computed(tmp_path):
+    """bench.py --dump-outputs on the default workload: the kept voxels of the last timed step are those of the same
+    volume reconstructed on its own, and the bond dimensions are the step's."""
+    import numpy as np
+    import torch
+
+    import bench
+    from imgcompressionmps.core.ndmps import NDMPS
+    out = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--volumes", "1", "--in-flight", "1", "--steps", "2", "--warmup", "1",
+                          "--no-cpu", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900, cwd=str(ROOT))
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads([ln for ln in out.stdout.splitlines() if ln.startswith("{")][0])
+    assert sum(p.stat().st_size for p in tmp_path.iterdir()) <= bench.DUMP_LIMIT + 4096
+    rec, bonds = np.load(tmp_path / "reconstruction.npy"), np.load(tmp_path / "bond_dims.npy")
+    pos = bench.dump_positions(512 ** 3, 1)
+    assert rec.shape == (1, pos.size) and rec.dtype == np.float32
+    assert line["run"]["dump_outputs"]["voxels_kept_per_tensor"] == pos.size
+    assert bonds.tolist() == [line["run"]["bond_dims"]]
+    x = torch.from_numpy(bench.make_input("cfg3", 0, 0)).cuda()
+    obj = NDMPS.from_tensor(x, max_bond=64)
+    want = obj.to_tensor_device().reshape(-1)[torch.from_numpy(pos).cuda()].cpu().numpy()
+    assert bonds.tolist() == [obj.bond_sizes()]
+    assert np.linalg.norm(rec[0] - want) <= 1e-5 * np.linalg.norm(want)
