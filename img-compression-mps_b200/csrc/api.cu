@@ -149,7 +149,7 @@ __global__ void __launch_bounds__(256) readback_kernel(const unsigned* __restric
 int copy_small(ndmps_ctx* ctx, void* dev_dst, const void* dev_src, size_t bytes) {
     if (bytes == 0) return NDMPS_OK;
     const bool words = bytes % 4 == 0 && reinterpret_cast<uintptr_t>(dev_dst) % 4 == 0 && reinterpret_cast<uintptr_t>(dev_src) % 4 == 0;
-    if (ctx->opt_readback == 0 && words && bytes <= (size_t(8) << 20)) {
+    if (words && bytes <= (size_t(8) << 20)) {
         const int64_t n = (int64_t)(bytes / 4);
         int64_t grid = (n + 1023) / 1024;
         if (grid > 64) grid = 64;
@@ -166,7 +166,7 @@ int readback(ndmps_ctx* ctx, void* pinned_dst, const void* dev_src, size_t bytes
     const bool in_scratch = ctx->pinned && (const char*)pinned_dst >= (const char*)ctx->pinned &&
                             (const char*)pinned_dst + bytes <= (const char*)(ctx->pinned + ctx->pinned_doubles);
     const bool words = bytes % 4 == 0 && reinterpret_cast<uintptr_t>(pinned_dst) % 4 == 0 && reinterpret_cast<uintptr_t>(dev_src) % 4 == 0;
-    if (ctx->opt_readback == 0 && in_scratch && words && bytes <= (size_t(8) << 20)) {
+    if (in_scratch && words && bytes <= (size_t(8) << 20)) {
         const int64_t n = (int64_t)(bytes / 4);
         int64_t grid = (n + 1023) / 1024;
         if (grid > 32) grid = 32;
@@ -224,25 +224,8 @@ static cudaError_t flag_wait(ndmps_ctx* ctx) {
 }
 
 cudaError_t stream_wait(ndmps_ctx* ctx) {
-    if (!ctx->opt_blocking_sync) return cudaStreamSynchronize(ctx->stream);
     if (ctx->opt_blocking_sync == 3) return flag_wait(ctx);
-    if (!ctx->sync_event) {
-        cudaError_t e = cudaEventCreateWithFlags(&ctx->sync_event, cudaEventBlockingSync | cudaEventDisableTiming);
-        if (e != cudaSuccess) return e;
-    }
-    cudaError_t e = cudaEventRecord(ctx->sync_event, ctx->stream);
-    if (e != cudaSuccess) return e;
-    if (ctx->opt_blocking_sync == 2) {
-        // polite polling: the waits of the sweep are 5 - 500 us long; sleeping in the driver costs a wake-up (50 - 100 us)
-        // per wait, spinning needs a core per waiter.  Poll, and hand the core over between polls.
-        for (int spins = 0;; spins++) {
-            e = cudaEventQuery(ctx->sync_event);
-            if (e != cudaErrorNotReady) return e;
-            if (spins < 64) continue;
-            std::this_thread::yield();
-        }
-    }
-    return cudaEventSynchronize(ctx->sync_event);
+    return cudaStreamSynchronize(ctx->stream);
 }
 
 // ---- gate for concurrent cooperative launches (see common.cuh) ---------------------------------
@@ -341,7 +324,6 @@ int ndmps_ctx_destroy(ndmps_ctx_t* ctx) {
     if (!ctx) return NDMPS_OK;
     stream_wait(ctx);
     ctx->ws.release();
-    if (ctx->sync_event) cudaEventDestroy(ctx->sync_event);
     if (ctx->wait_flag) cudaFreeHost(const_cast<unsigned*>(ctx->wait_flag));
     if (ctx->pinned) cudaFreeHost(ctx->pinned);
     delete ctx;
@@ -418,34 +400,22 @@ int ndmps_ctx_get_stat(ndmps_ctx_t* ctx, const char* name, double* value_out, in
 int ndmps_ctx_set_option(ndmps_ctx_t* ctx, const char* name, int64_t value) {
     NDMPS_REQUIRE(ctx != nullptr && name != nullptr, "ndmps_ctx_set_option: NULL argument");
     if (!strcmp(name, "gram_path")) ctx->opt_gram_path = value;
-    else if (!strcmp(name, "jacobi_block")) ctx->opt_jacobi_block = value;
     else if (!strcmp(name, "gemm_path")) ctx->opt_gemm_path = value;
-    else if (!strcmp(name, "permute_path")) ctx->opt_permute_path = value;
-    else if (!strcmp(name, "permute_ctas")) ctx->opt_permute_ctas = value;
-    else if (!strcmp(name, "merge_cap")) ctx->opt_merge_cap = value;
-    else if (!strcmp(name, "jacobi_max_sweeps")) ctx->opt_jacobi_max_sweeps = value;
-    else if (!strcmp(name, "eig_cholesky")) ctx->opt_eig_cholesky = value;
-    else if (!strcmp(name, "eig_small")) ctx->opt_eig_small = value;
-    else if (!strcmp(name, "chol_blocked")) ctx->opt_chol_blocked = value;
-    else if (!strcmp(name, "chol_cluster")) ctx->opt_chol_cluster = value;
-    else if (!strcmp(name, "chol_rows")) ctx->opt_chol_rows = value;
-    else if (!strcmp(name, "eig_topk")) ctx->opt_eig_topk = value;
-    else if (!strcmp(name, "topk_one_row")) ctx->opt_topk_one_row = value;
-    else if (!strcmp(name, "topk_cluster")) ctx->opt_topk_cluster = value;
-    else if (!strcmp(name, "tc_waves")) ctx->opt_tc_waves = value;
-    else if (!strcmp(name, "topk_mid")) ctx->opt_topk_mid = value;
-    else if (!strcmp(name, "topk_bt_pairs")) ctx->opt_topk_bt_pairs = value;
-    else if (!strcmp(name, "topk_big_ctas")) ctx->opt_topk_big_ctas = value;
-    else if (!strcmp(name, "topk_passes")) ctx->opt_topk_passes = value;
-    else if (!strcmp(name, "topk_iters")) ctx->opt_topk_iters = value;
-    else if (!strcmp(name, "topk_rr_skip")) ctx->opt_topk_rr_skip = value;
-    else if (!strcmp(name, "blocking_sync")) ctx->opt_blocking_sync = value;
-    else if (!strcmp(name, "readback")) ctx->opt_readback = value;
-    else if (!strcmp(name, "verbose")) ctx->opt_verbose = value;
-    else if (!strcmp(name, "tc")) ctx->opt_tc = value;
-    else if (!strcmp(name, "ssim_exact")) ctx->opt_ssim_exact = value;
-    else if (!strcmp(name, "tc_chunk")) ctx->opt_tc_chunk = value;
     else if (!strcmp(name, "gemm_out_t")) ctx->opt_gemm_out_t = value;
+    else if (!strcmp(name, "tc")) ctx->opt_tc = value;
+    else if (!strcmp(name, "tc_waves")) ctx->opt_tc_waves = value;
+    else if (!strcmp(name, "permute_path")) {
+        NDMPS_REQUIRE(value >= 0 && value <= 2, "ndmps_ctx_set_option: permute_path must be 0, 1 or 2 (got %lld)", (long long)value);
+        ctx->opt_permute_path = value;
+    }
+    else if (!strcmp(name, "eig_topk")) ctx->opt_eig_topk = value;
+    else if (!strcmp(name, "topk_cluster")) ctx->opt_topk_cluster = value;
+    else if (!strcmp(name, "ssim_exact")) ctx->opt_ssim_exact = value;
+    else if (!strcmp(name, "blocking_sync")) {
+        NDMPS_REQUIRE(value == 0 || value == 3, "ndmps_ctx_set_option: blocking_sync must be 0 or 3 (got %lld)", (long long)value);
+        ctx->opt_blocking_sync = value;
+    }
+    else if (!strcmp(name, "verbose")) ctx->opt_verbose = value;
     else {
         set_error("ndmps_ctx_set_option: unknown option '%s'", name);
         return NDMPS_ERR_INVALID;

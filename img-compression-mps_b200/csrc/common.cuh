@@ -36,19 +36,12 @@ struct TilePlan {
     std::vector<int64_t> hi_src;         // tile/pb source offsets of the source runs (read order)
     std::vector<int64_t> hi_dst;         // tile/pa destination offsets of the destination runs (write order)
     std::vector<uint16_t> pos;           // read index -> (skewed) shared-memory slot
-    // bulk-copy (TMA-class) variant: source runs land in shared memory as they are (run r at
-    // r * (pb + run_pad)), threads gather them into destination order, destination runs leave
-    // by bulk store.  rslot[w] = shared-memory slot (in the padded source image) of write index w.
-    std::vector<uint16_t> rslot;
-    int run_pad = 0;
-    int gather_conflict = 0;
     // device copies, uploaded on first use PER DEVICE (a plan is shared by host threads that may drive different GPUs)
     struct DevTables {
         int device = -1;
         int64_t* hi_src = nullptr;
         int64_t* hi_dst = nullptr;
         uint16_t* pos = nullptr;
-        uint16_t* rslot = nullptr;
     };
     std::vector<DevTables> dev;          // guarded by the upload mutex in permute.cu; read through upload_tile_plan only
 };
@@ -154,11 +147,10 @@ struct ndmps_ctx {
     // pinned host scratch for small D2H readbacks (eigenvalues, flags, scalars)
     double* pinned = nullptr;
     size_t pinned_doubles = 0;
-    // options
-    int64_t opt_gram_path = 0;      // 0: auto (FP64 tensor pipe when the shape allows), 2: force the SIMT kernel, 3: force tcgen05 (tc_gemm.cu)
-    int64_t opt_tc = 1;             // tcgen05 contractions on bf16x3 split planes for float32 payloads of a capped sweep / the reconstruction (0: off)
-    int64_t opt_tc_chunk = 0;       // k-tiles (64 columns each) between drains of the tcgen05 Gram accumulator into float64 (0: 4)
-    int64_t opt_gemm_out_t = 0;     // test hook: ndmps_gemm writes C transposed (n x m) through the tcgen05 epilogue
+    // options: ndmps_ctx_set_option in ndmps.h lists names, defaults and values
+    int64_t opt_gram_path = 0;      // 0 auto, 2 SIMT, 3 tcgen05
+    int64_t opt_tc = 1;             // tcgen05 contractions for float32 payloads
+    int64_t opt_gemm_out_t = 0;     // test hook: ndmps_gemm writes C transposed
     // int8 digit planes of the unfolding the tcgen05 Gram sliced last (workspace memory: valid until the next ws.reset);
     // the projection of the same sweep step multiplies the same digits.  exact_host: the device-side "use the FP64 pipe"
     // flag once it has been copied to the host beside the eigenvalues (-1: not yet known)
@@ -167,36 +159,15 @@ struct ndmps_ctx {
         const int* sc = nullptr; const int* use_exact = nullptr; uint64_t gen = 0; int exact_host = -1;
     } tc_digits;
     bool tc_sweep = false;          // set by the sweep while the tcgen05 Gram / projection are admissible (float32, bond cap)
-    int64_t opt_jacobi_block = 0;   // 0: auto
-    int64_t opt_gemm_path = 0;      // 0: FP64 tensor pipe for large row-major products, 2: SIMT only
-    int64_t opt_permute_path = 0;   // 0: register bit-permutation when the shape allows, else ld/st tiles through shared
-                                    // memory; 1: tiles always; 3: bulk-copy (TMA-class) tiles; 2: gather kernel
-    int64_t opt_permute_ctas = 0;   // grid cap of the tiled kernel in CTAs per SM (0: 64)
-    int64_t opt_merge_cap = 512;    // max rows of a merged front group in the sweep
-    int64_t opt_jacobi_max_sweeps = 40;
-    int64_t opt_chol_blocked = 1;         // 8 pivots per pair of grid barriers
-    int64_t opt_chol_cluster = 0;         // pivoted Cholesky inside one thread-block cluster (measured slower: DSMEM row broadcast)
-    int64_t opt_chol_rows = 0;            // rows per CTA of the pivoted Cholesky (0: auto)
-    int64_t opt_eig_small = 1;            // n <= 128: single-CTA all-in-one solver
-    int64_t opt_eig_cholesky = 1;         // pivoted-Cholesky preconditioning of the Jacobi solve
-    int64_t opt_eig_topk = 1;             // bond cap set: leading-eigenpair solver (eig_topk.cu) instead of the full one
-    int64_t opt_topk_cluster = 1;         // 1: n <= 512 tridiagonalisation as one thread-block cluster (exchange through distributed shared memory)
+    int64_t opt_gemm_path = 0;      // 0 auto, 2 SIMT
+    int64_t opt_permute_path = 0;   // 0 auto, 1 tiles, 2 gather
+    int64_t opt_eig_topk = 1;             // leading-eigenpair solver for capped bonds
+    int64_t opt_topk_cluster = 1;         // cluster tridiagonalisation for n <= 512
     int64_t cluster_launches = 0;
-    int64_t opt_tc_waves = 1;             // waves of gram_i8 CTAs (split-K factor = waves x SMs / tiles)
-    int64_t opt_topk_mid = 1;             // 1: 1024 < n <= 1536 tridiagonalisation stays in the register files (140 CTAs x 11 warps)
-    int64_t opt_topk_bt_pairs = 1;        // 1: back-transformation applies the reflectors in pairs (one reduction per pair)
-    int64_t opt_topk_one_row = 0;         // 1: one matrix row per warp in the register-resident reduction (default: two up to n = 512)
-    int64_t opt_topk_big_ctas = 0;        // CTAs per SM of the L2-streamed tridiagonalisation (0: occupancy, at most 3)
-    int64_t opt_topk_passes = 0;          // bisection passes (0: 8, each divides the bracket by 129)
-    int64_t opt_topk_iters = 0;           // inverse-iteration steps (0: 3)
-    int64_t opt_topk_rr_skip = 1;         // pass an already diagonal Rayleigh-Ritz block through without the Jacobi solve
-    int64_t opt_ssim_exact = 0;           // 1: float64 SSIM arithmetic for float32 inputs too (default: shifted / normalised float32)
-    int64_t opt_blocking_sync = 0;        // host waits: 0 spin (cudaStreamSynchronize), 1 sleep on a blocking event, 2 poll the
-                                          // event + yield, 3 watch a pinned word the stream writes (no driver calls) + yield
+    int64_t opt_tc_waves = 1;             // waves of gram_i8 CTAs
+    int64_t opt_ssim_exact = 0;           // float64 SSIM for float32 inputs
+    int64_t opt_blocking_sync = 0;        // host waits: 0 spin, 3 watch a pinned word
     int64_t opt_verbose = 0;
-    cudaEvent_t sync_event = nullptr;     // created on first blocking wait
-    int64_t opt_readback = 0;                 // small device -> host read-backs: 0 stores from the SMs into mapped pinned
-                                              // memory, 1 cudaMemcpyAsync (copy engine)
     volatile unsigned* wait_flag = nullptr;   // pinned word the stream writes its sequence numbers into (wait mode 3)
     unsigned wait_seq = 0;
     // stats of the last eigensolve / sweep (for tests and profiling)
@@ -221,7 +192,7 @@ int copy_small(ndmps_ctx* ctx, void* dev_dst, const void* dev_src, size_t bytes)
 // cudaFuncAttributeMaxDynamicSharedMemorySize is a per-DEVICE attribute of a kernel: raise it to `bytes` once per
 // (kernel, device), from any host thread (the largest value set so far is remembered under a mutex).
 int raise_dynamic_smem(const void* kernel, int device, int bytes);
-// wait for everything enqueued on the context's stream (spinning cudaStreamSynchronize, or a blocking event)
+// wait for everything enqueued on the context's stream (spinning cudaStreamSynchronize, or watching a pinned word)
 cudaError_t stream_wait(ndmps_ctx* ctx);
 
 // RAII stage marker: records an event pair around a leaf stage when profiling is on

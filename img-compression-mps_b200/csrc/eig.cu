@@ -15,7 +15,7 @@
 // pairs); later rounds only rotate cross pairs.  The whole solve is ONE persistent
 // cooperative launch: CTAs exchange column blocks through L2 (ld.cg / st.cg) and meet
 // at a counter barrier after every round; convergence is a per-sweep flag.  Matrices
-// that fit one CTA's shared memory are swept to convergence by a single CTA.
+// with n <= 64 are solved whole by one CTA (eigh_small_kernel).
 //
 // Per rotation the latency chain is what matters (the FP64 work is tiny), so:
 //   * the three reductions of a pair (|x|^2, |y|^2, x.y) run as interleaved butterflies;
@@ -26,18 +26,14 @@
 //     accuracy) instead of the IEEE division / square-root instruction sequences;
 // (de Rijk's dynamic column swaps were tried and dropped: in a parallel tournament they break
 // the once-per-sweep pair coverage and the sweep count explodes.)
-#include <cooperative_groups.h>
-
-#include <atomic>
-
 #include "common.cuh"
-
-namespace cg = cooperative_groups;
 
 namespace ndmps {
 
 // rotation threshold |x.y| <= tol |x||y| with tol = sqrt(n) * 2 eps (LAPACK dgesvj uses sqrt(n) eps)
 static inline double jacobi_tol(int n) { return sqrt((double)n) * 4.4408920985006262e-16; }
+
+constexpr int JACOBI_MAX_SWEEPS = 40;
 
 __device__ __forceinline__ double rsqrt_refined(double x) {   // x in the normal range
     double r;
@@ -461,42 +457,6 @@ jacobi_round_kernel(double* A, int n, int ncols, int b, int nb, int round, unsig
     if (any && (threadIdx.x & 31) == 0) atomicOr(flag, 1u);
 }
 
-// Whole matrix in one CTA (n <= 32; larger ones are faster on the block path): sweep until no rotation happens.  Eight lanes per column
-// pair, four pairs per warp; block = 32*W threads, dynamic smem = n*n doubles.
-// ctrl[1] = sweeps used (negative: not converged).
-template <int NR>
-__global__ void __launch_bounds__(512)
-jacobi_single_kernel(double* A, int n, int max_sweeps, unsigned* ctrl, double tol2, const double* floor2_ptr) {
-    extern __shared__ double S[];
-    const double floor2 = *floor2_ptr;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, W = blockDim.x >> 5;
-    const int grp = lane >> 3, li = lane & 7;
-    for (int i = threadIdx.x; i < n * n; i += blockDim.x) S[i] = A[i];
-    __syncthreads();
-    const int P = (n + 1) & ~1;          // pad to an even number of players; player n (if any) is a bye
-    const int matches = P / 2;
-    int sweep = 0;
-    int done = n < 2 ? 1 : 0;
-    float relmax = 0.f;
-    while (!done && sweep < max_sweeps) {
-        bool any = false;
-        for (int lr = 0; lr < P - 1; lr++) {
-            for (int m0 = warp * 4; m0 < matches; m0 += W * 4) {     // warp-uniform trip count
-                const int m = m0 + grp;
-                int s1 = 0, s2 = 0;
-                if (m < matches) tournament_pair(P, lr, m, s1, s2);
-                const bool valid = m < matches && s1 < n && s2 < n;
-                any |= rotate_group<NR, 8>(S + (size_t)s1 * n, S + (size_t)s2 * n, n, li, valid, tol2, floor2, relmax);
-            }
-            __syncthreads();
-        }
-        sweep++;
-        done = !__syncthreads_or(any ? 1 : 0);
-    }
-    for (int i = threadIdx.x; i < n * n; i += blockDim.x) A[i] = S[i];
-    if (threadIdx.x == 0) ((int*)ctrl)[1] = done ? sweep : -sweep;
-}
-
 // |column j| for j < ncols (columns of length n), one warp per column
 __global__ void __launch_bounds__(256)
 column_norms_kernel(const double* __restrict__ A, int n, int ncols, double* __restrict__ norms) {
@@ -520,24 +480,6 @@ null_floor_kernel(const double* __restrict__ norms, int n, int ncols, double* __
         double f = (double)n * 2.220446049250313e-16 * m;
         floor2[0] = f * f;
     }
-}
-
-// copy column j of A to column rank(j) of B, rank = descending order of the column norms
-__global__ void __launch_bounds__(256)
-sort_columns_kernel(const double* __restrict__ A, const double* __restrict__ norms, int n, double* __restrict__ B) {
-    int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-    if (warp >= n) return;
-    double mine = norms[warp];
-    int cnt = 0;
-    for (int k = lane; k < n; k += 32) {
-        double o = norms[k];
-        cnt += (o > mine || (o == mine && k < warp)) ? 1 : 0;
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
-    const double* src = A + (size_t)warp * n;
-    double* dst = B + (size_t)cnt * n;
-    for (int i = lane; i < n; i += 32) dst[i] = src[i];
 }
 
 // descending rank of every column by counting (ties broken by index), then write
@@ -575,122 +517,13 @@ sort_extract_kernel(const double* __restrict__ A, const double* __restrict__ nor
 // bond Gram matrices of real volumes this halves the sweep count (profiles/r01_jacobi_sweeps.md).
 //
 // Persistent cooperative kernel, rows distributed over CTAs (each keeps its rows of the running
-// Schur complement in shared memory).  Per step: every CTA publishes its best remaining diagonal
-// entry TOGETHER with that row (so one grid barrier per step is enough), all CTAs pick the same
-// winner, scale it into column k of L and update their own rows.  L is produced column-major in
-// the ORIGINAL row order (no permutation to undo: G = sum_k l_k l_k^T).
-// ---------------------------------------------------------------------------------------------
-struct CholCand { double val; int row; int pad; };
-
-__global__ void __launch_bounds__(256)
-pivoted_cholesky_kernel(const double* __restrict__ G, int n, int rows_per, double* __restrict__ Lcol,
-                        double* cand_rows, CholCand* cand, unsigned* ctrl, double stop_rel) {
-    extern __shared__ double sm[];
-    double* slab = sm;                                   // rows_per x n : this CTA's rows of the Schur complement
-    double* piv = slab + (size_t)rows_per * n;           // n : winner row, already divided by sqrt(pivot)
-    double* lrow = piv + n;                              // rows_per : this step's column of L for our rows
-    int* chosen = reinterpret_cast<int*>(lrow + rows_per);   // rows_per
-    __shared__ int s_bi;          // local candidate row (slab index) or -1
-    __shared__ int s_w;           // winning CTA or -1
-    __shared__ int s_prow;        // winning row (global index)
-    __shared__ double s_pval;     // winning pivot
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, cta = blockIdx.x, ncta = gridDim.x;
-    const int row0 = cta * rows_per;
-    int nrows = n - row0;
-    nrows = nrows < 0 ? 0 : (nrows > rows_per ? rows_per : nrows);
-    for (int idx = tid; idx < nrows * n; idx += blockDim.x) slab[idx] = G[(size_t)row0 * n + idx];
-    if (tid < rows_per) chosen[tid] = tid < nrows ? 0 : 1;
-    __syncthreads();
-    double p0 = 0.0;
-    int rank = n;
-    for (int k = 0; k < n; k++) {
-        // ---- [A] local candidate: largest remaining diagonal entry of our rows (warp 0) ----
-        if (warp == 0) {
-            double best = -1.0;
-            int bi = -1;
-            for (int r = lane; r < nrows; r += 32) {
-                double d = slab[(size_t)r * n + row0 + r];
-                if (!chosen[r] && d > best) { best = d; bi = r; }
-            }
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) {
-                double ob = __shfl_xor_sync(0xffffffffu, best, o);
-                int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-                if (ob > best || (ob == best && oi >= 0 && (bi < 0 || oi < bi))) { best = ob; bi = oi; }
-            }
-            if (lane == 0) {
-                s_bi = bi;
-                CholCand c;
-                c.val = best;
-                c.row = bi >= 0 ? row0 + bi : -1;
-                c.pad = 0;
-                cand[(size_t)(k & 1) * ncta + cta] = c;
-            }
-        }
-        __syncthreads();
-        // ---- [B] publish the candidate row itself, then meet ----
-        const int bi = s_bi;
-        if (bi >= 0) {
-            double* dst = cand_rows + ((size_t)(k & 1) * ncta + cta) * n;
-            for (int c = tid; c < n; c += blockDim.x) __stcg(dst + c, slab[(size_t)bi * n + c]);
-        }
-        grid_barrier(ctrl, (unsigned)(k + 1) * ncta);
-        // ---- [C] every CTA picks the same winner (warp 0) ----
-        if (warp == 0) {
-            double best = -1.0;
-            int brow = -1, bw = -1;
-            for (int t = lane; t < ncta; t += 32) {
-                const CholCand* cp = cand + (size_t)(k & 1) * ncta + t;
-                double v = __ldcg(&cp->val);
-                int r = __ldcg(&cp->row);
-                if (r >= 0 && (v > best || (v == best && (brow < 0 || r < brow)))) { best = v; brow = r; bw = t; }
-            }
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) {
-                double ob = __shfl_xor_sync(0xffffffffu, best, o);
-                int orow = __shfl_xor_sync(0xffffffffu, brow, o);
-                int ow = __shfl_xor_sync(0xffffffffu, bw, o);
-                if (orow >= 0 && (ob > best || (ob == best && (brow < 0 || orow < brow)))) { best = ob; brow = orow; bw = ow; }
-            }
-            if (lane == 0) { s_w = bw; s_prow = brow; s_pval = best; }
-        }
-        __syncthreads();
-        const int w = s_w, prow = s_prow;
-        const double pval = s_pval;
-        if (k == 0) p0 = pval;
-        if (w < 0 || !(pval > stop_rel * p0) || !(pval > 0.0)) { rank = k; break; }   // uniform across the grid
-        // ---- [D] winner row (scaled), our entries of column k of L ----
-        const double root = sqrt(pval), inv = 1.0 / root;
-        const double* src = cand_rows + ((size_t)(k & 1) * ncta + w) * n;
-        for (int c = tid; c < n; c += blockDim.x) piv[c] = __ldcg(src + c) * inv;
-        if (tid < nrows) {
-            double l;
-            if (row0 + tid == prow) { l = root; chosen[tid] = 1; }
-            else if (!chosen[tid]) l = slab[(size_t)tid * n + prow] * inv;
-            else l = 0.0;
-            lrow[tid] = chosen[tid] ? 0.0 : l;            // rows already eliminated take no update
-            __stcg(Lcol + (size_t)k * n + row0 + tid, l);
-        }
-        __syncthreads();
-        // ---- [E] Schur complement update of our remaining rows ----
-        for (int idx = tid; idx < nrows * n; idx += blockDim.x) {
-            const int r = idx / n, c = idx - r * n;
-            const double l = lrow[r];
-            if (l != 0.0) slab[idx] = fma(-l, piv[c], slab[idx]);
-        }
-        __syncthreads();
-    }
-    if (cta == 0 && tid == 0) ((int*)ctrl)[1] = rank;
-}
-
-// ---------------------------------------------------------------------------------------------
-// Blocked pivoted Cholesky: CHB pivots per pair of grid barriers instead of one pivot per
-// barrier.  Per block step every CTA (1) publishes the diagonal of its live rows, (2) picks
-// the same CHB largest candidates, whose owners publish those rows, (3) factors the block
-// redundantly with pivoting INSIDE the block (a candidate that turns out to depend on the
-// ones already taken is left for a later step), (4) writes its rows of the new L columns and
-// applies the rank-CHB update to its slab.  Same factor quality as the one-pivot kernel for
-// preconditioning purposes, ~4x fewer microseconds.
+// Schur complement in shared memory), CHB pivots per pair of grid barriers.  Per block step every
+// CTA (1) publishes the diagonal of its live rows, (2) picks the same CHB largest candidates, whose
+// owners publish those rows, (3) factors the block redundantly with pivoting INSIDE the block (a
+// candidate that turns out to depend on the ones already taken is left for a later step), (4)
+// writes its rows of the new L columns and applies the rank-CHB update to its slab.  L is produced
+// column-major in the ORIGINAL row order (no permutation to undo: G = sum_k l_k l_k^T).  A
+// one-pivot-per-barrier kernel gave the same factor quality for preconditioning at ~4x the time.
 // ---------------------------------------------------------------------------------------------
 constexpr int CHB = 8;
 
@@ -838,100 +671,6 @@ pivoted_cholesky_blocked_kernel(const double* __restrict__ G, int n, int rows_pe
         __syncthreads();
     }
     if (cta == 0 && tid == 0) ((int*)ctrl)[1] = rank < k ? rank : k;
-}
-
-// ---------------------------------------------------------------------------------------------
-// Cluster variant of the pivoted Cholesky (n <= ~640): the whole Schur complement lives in the
-// shared memory of ONE thread-block cluster of up to 16 CTAs.  Candidates are exchanged by
-// remote shared-memory stores, the winning row is read from its owner through distributed
-// shared memory, and the per-step synchronisation is the hardware cluster barrier instead of
-// a global-memory counter: ~1 us per step instead of ~5 us.
-// ---------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256)
-pivoted_cholesky_cluster_kernel(const double* __restrict__ G, int n, int rows_per, double* __restrict__ Lcol,
-                                int* __restrict__ rank_out, double stop_rel) {
-    cg::cluster_group cluster = cg::this_cluster();
-    extern __shared__ double sm[];
-    double* slab = sm;                                   // rows_per x n
-    double* piv = slab + (size_t)rows_per * n;           // n
-    double* lrow = piv + n;                              // rows_per
-    int* chosen = reinterpret_cast<int*>(lrow + rows_per);   // rows_per
-    __shared__ double cand_val[2][16];
-    __shared__ int cand_row[2][16];
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int cta = (int)cluster.block_rank(), ncta = (int)cluster.num_blocks();
-    const int row0 = cta * rows_per;
-    int nrows = n - row0;
-    nrows = nrows < 0 ? 0 : (nrows > rows_per ? rows_per : nrows);
-    for (int idx = tid; idx < nrows * n; idx += blockDim.x) slab[idx] = G[(size_t)row0 * n + idx];
-    if (tid < rows_per) chosen[tid] = tid < nrows ? 0 : 1;
-    __syncthreads();
-    double p0 = 0.0;
-    int rank = n;
-    for (int k = 0; k < n; k++) {
-        const int par = k & 1;
-        // ---- [A] local candidate, stored into every CTA's candidate table ----
-        if (warp == 0) {
-            double best = -1.0;
-            int bi = -1;
-            for (int r = lane; r < nrows; r += 32) {
-                double d = slab[(size_t)r * n + row0 + r];
-                if (!chosen[r] && d > best) { best = d; bi = r; }
-            }
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) {
-                double ob = __shfl_xor_sync(0xffffffffu, best, o);
-                int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-                if (oi >= 0 && (ob > best || (ob == best && (bi < 0 || oi < bi)))) { best = ob; bi = oi; }
-            }
-            if (lane < ncta) {
-                double* rv = cluster.map_shared_rank(&cand_val[par][cta], lane);
-                int* rr = cluster.map_shared_rank(&cand_row[par][cta], lane);
-                *rv = best;
-                *rr = bi >= 0 ? row0 + bi : -1;
-            }
-        }
-        cluster.sync();
-        // ---- [C] every warp picks the same winner from its CTA's table ----
-        double wv = -1.0;
-        int wrow = -1;
-        if (lane < ncta) { wv = cand_val[par][lane]; wrow = cand_row[par][lane]; }
-#pragma unroll
-        for (int o = 8; o > 0; o >>= 1) {
-            double ob = __shfl_xor_sync(0xffffffffu, wv, o);
-            int orow = __shfl_xor_sync(0xffffffffu, wrow, o);
-            if (orow >= 0 && (wrow < 0 || ob > wv || (ob == wv && orow < wrow))) { wv = ob; wrow = orow; }
-        }
-        wv = __shfl_sync(0xffffffffu, wv, 0);
-        wrow = __shfl_sync(0xffffffffu, wrow, 0);
-        if (k == 0) p0 = wv;
-        if (wrow < 0 || !(wv > stop_rel * p0) || !(wv > 0.0)) { rank = k; break; }   // uniform across the cluster
-        // ---- [D] winner row through distributed shared memory, our entries of L's column k ----
-        const int wcta = wrow / rows_per;
-        const double root = sqrt(wv), inv = 1.0 / root;
-        const double* wslab = cluster.map_shared_rank(slab, wcta);
-        const double* wr = wslab + (size_t)(wrow - wcta * rows_per) * n;
-        for (int c = tid; c < n; c += blockDim.x) piv[c] = wr[c] * inv;
-        if (tid < nrows) {
-            double l;
-            const bool was = chosen[tid] != 0;
-            if (row0 + tid == wrow) { l = root; chosen[tid] = 1; }
-            else if (!was) l = slab[(size_t)tid * n + wrow] * inv;
-            else l = 0.0;
-            lrow[tid] = (was || row0 + tid == wrow) ? 0.0 : l;      // eliminated rows take no update
-            __stcg(Lcol + (size_t)k * n + row0 + tid, l);
-        }
-        __syncthreads();
-        // ---- [E] Schur complement update of our remaining rows ----
-        for (int idx = tid; idx < nrows * n; idx += blockDim.x) {
-            const int r = idx / n, c = idx - r * n;
-            const double l = lrow[r];
-            if (l != 0.0) slab[idx] = fma(-l, piv[c], slab[idx]);
-        }
-        __syncthreads();
-    }
-    cluster.sync();                                      // nobody may exit while a peer can still read its rows
-    if (cta == 0 && tid == 0) rank_out[0] = rank;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1148,30 +887,19 @@ static int run_round(ndmps_ctx* ctx, double* A, int n, int ncols, int b, int nb,
     return NDMPS_OK;
 }
 
-template <int NR>
-static int run_single(ndmps_ctx* ctx, double* A, int n, int warps, int max_sweeps, unsigned* ctrl, double tol2,
-                      const double* floor2, size_t smem) {
-    NDMPS_TRY(raise_smem(jacobi_single_kernel<NR>, ctx));
-    jacobi_single_kernel<NR><<<1, 32 * warps, smem, ctx->stream>>>(A, n, max_sweeps, ctrl, tol2, floor2);
-    NDMPS_LAUNCH_CHECK(ctx);
-    return NDMPS_OK;
-}
-
 // Jacobi sweeps over the ncols columns (length n) stored at A + j*n, block path.
 static int jacobi_columns(ndmps_ctx* ctx, double* A, int n, int ncols, double tol2, const double* floor2, int* sweeps_used,
                           float quad_stop2) {
-    const int max_sweeps = (int)ctx->opt_jacobi_max_sweeps;
+    const int max_sweeps = JACOBI_MAX_SWEEPS;
     const size_t smem_cap = ctx->smem_optin > 4096 ? ctx->smem_optin - 2048 : 0;
     unsigned* ctrl = nullptr;   // [0] barrier counter, [1] sweeps used, [2..] per-sweep rotation flags
     NDMPS_TRY(ctx->ws.get<unsigned>((size_t)max_sweeps + 4, &ctrl));
     NDMPS_CUDA_TRY(cudaMemsetAsync(ctrl, 0, ((size_t)max_sweeps + 4) * sizeof(unsigned), ctx->stream));
     int* host_flag = reinterpret_cast<int*>(ctx->pinned);
     const int nr = n <= 256 ? 8 : n <= 512 ? 16 : 0;      // rows per lane of the block kernels
-    // block size: as many columns as shared memory allows, at most 16 warps, tunable
+    // block size: as many columns as shared memory allows, at most 8 (measured best: more CTAs, cheaper rounds)
     int b = (int)((smem_cap - 512) / (16 * (size_t)n));
-    if (b > 16) b = 16;
-    if (ctx->opt_jacobi_block > 0) { if (ctx->opt_jacobi_block < b) b = (int)ctx->opt_jacobi_block; }
-    else if (b > 8) b = 8;                                // measured best: more CTAs, cheaper rounds
+    if (b > 8) b = 8;
     NDMPS_REQUIRE(b >= 1, "eigh: n = %d does not fit a column pair in shared memory", n);
     while (b > 1 && (ncols + b - 1) / b < 2) b /= 2;      // at least two blocks
     int nb = (ncols + b - 1) / b;
@@ -1213,61 +941,13 @@ static int jacobi_columns(ndmps_ctx* ctx, double* A, int n, int ncols, double to
 }
 
 // G = L L^T with diagonal pivoting; returns the numerical rank (host) and L column-major.
-static int pivoted_cholesky_cluster(ndmps_ctx* ctx, const double* G, int n, double* Lcol, int* rank_out, bool* done) {
-    *done = false;
-    if (ctx->opt_chol_cluster == 0) return NDMPS_OK;
-    int rows_per = (n + 15) / 16;
-    int ncta = (n + rows_per - 1) / rows_per;
-    const size_t smem = ((size_t)rows_per * n + n + rows_per) * sizeof(double) + (size_t)rows_per * sizeof(int) + 16;
-    if (ncta > 16 || smem > ctx->smem_optin - 4096) return NDMPS_OK;
-    static std::atomic<int> usable{-1};      // -1 unknown, 0 a device refused the cluster launch once, 1 fine
-    if (usable.load() == 0) return NDMPS_OK;
-    {
-        int rc = raise_smem_minus(pivoted_cholesky_cluster_kernel, ctx, 4096);
-        cudaError_t e = rc == NDMPS_OK ? cudaFuncSetAttribute(pivoted_cholesky_cluster_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1)
-                                       : cudaErrorUnknown;
-        if (e != cudaSuccess) { cudaGetLastError(); usable.store(0); return NDMPS_OK; }
-    }
-    int* rank_dev = nullptr;
-    NDMPS_TRY(ctx->ws.get<int>(4, &rank_dev));
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(ncta);
-    cfg.blockDim = dim3(256);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = ctx->stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = ncta;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    double stop_rel = 2.220446049250313e-16;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, pivoted_cholesky_cluster_kernel, G, n, rows_per, Lcol, rank_dev, stop_rel);
-    if (e != cudaSuccess) {      // e.g. no GPC with ncta free SMs: fall back to the global-barrier kernel
-        cudaGetLastError();
-        if (usable.load() < 0) usable.store(0);
-        return NDMPS_OK;
-    }
-    usable.store(1);
-    ctx->launches++;
-    int* host_flag = reinterpret_cast<int*>(ctx->pinned);
-    NDMPS_TRY(readback(ctx, host_flag, rank_dev, sizeof(int)));
-    NDMPS_CUDA_TRY(stream_wait(ctx));
-    *rank_out = host_flag[0];
-    *done = true;
-    return NDMPS_OK;
-}
-
-static int pivoted_cholesky_blocked(ndmps_ctx* ctx, const double* G, int n, double* Lcol, int* rank_out, bool* done) {
-    *done = false;
-    if (ctx->opt_chol_blocked == 0) return NDMPS_OK;
-    int rows_per = (n + 127) / 128;
-    if (ctx->opt_chol_rows > 0) rows_per = (int)ctx->opt_chol_rows;
+static int pivoted_cholesky(ndmps_ctx* ctx, const double* G, int n, double* Lcol, int* rank_out) {
+    int rows_per = (n + 127) / 128;                          // many small slabs: the per-step update is the critical path
     int ncta = (n + rows_per - 1) / rows_per;
     while (ncta > ctx->sm_count) { rows_per++; ncta = (n + rows_per - 1) / rows_per; }
     const size_t smem = ((size_t)rows_per * n + (size_t)n * CHB + (size_t)CHB * n + n) * sizeof(double) + (size_t)n * sizeof(int) + 16;
-    if (smem > ctx->smem_optin - 4096) return NDMPS_OK;
+    NDMPS_REQUIRE(smem <= ctx->smem_optin - 4096, "pivoted_cholesky: n = %d does not fit shared memory", n);
+    // the kernel also has static shared memory: static + dynamic must stay within the opt-in limit
     NDMPS_TRY(raise_smem_minus(pivoted_cholesky_blocked_kernel, ctx, 4096));
     double *diag_g = nullptr, *rows_g = nullptr;
     unsigned* ctrl = nullptr;
@@ -1282,40 +962,6 @@ static int pivoted_cholesky_blocked(ndmps_ctx* ctx, const double* G, int n, doub
     NDMPS_TRY(readback(ctx, host_flag, ctrl + 1, sizeof(int)));
     NDMPS_CUDA_TRY(stream_wait(ctx));
     *rank_out = host_flag[0];
-    *done = true;
-    return NDMPS_OK;
-}
-
-static int pivoted_cholesky(ndmps_ctx* ctx, const double* G, int n, double* Lcol, int* rank_out) {
-    {
-        bool done = false;
-        NDMPS_TRY(pivoted_cholesky_blocked(ctx, G, n, Lcol, rank_out, &done));
-        if (done) return NDMPS_OK;
-        NDMPS_TRY(pivoted_cholesky_cluster(ctx, G, n, Lcol, rank_out, &done));
-        if (done) return NDMPS_OK;
-    }
-    int rows_per = (n + 127) / 128;                          // many small slabs: the per-step update is the critical path
-    if (ctx->opt_chol_rows > 0) rows_per = (int)ctx->opt_chol_rows;
-    int ncta = (n + rows_per - 1) / rows_per;
-    while (ncta > ctx->sm_count) { rows_per++; ncta = (n + rows_per - 1) / rows_per; }
-    const size_t smem = ((size_t)rows_per * n + n + rows_per) * sizeof(double) + (size_t)rows_per * sizeof(int) + 16;
-    NDMPS_REQUIRE(smem <= ctx->smem_optin - 4096, "pivoted_cholesky: n = %d does not fit shared memory", n);
-    // the kernel also has ~3 KB of static shared memory: static + dynamic must stay within the opt-in limit
-    NDMPS_TRY(raise_smem_minus(pivoted_cholesky_kernel, ctx, 4096));
-    double* cand_rows = nullptr;
-    CholCand* cand = nullptr;
-    unsigned* ctrl = nullptr;
-    NDMPS_TRY(ctx->ws.get<double>((size_t)2 * ncta * n, &cand_rows));
-    NDMPS_TRY(ctx->ws.get<CholCand>((size_t)2 * ncta, &cand));
-    NDMPS_TRY(ctx->ws.get<unsigned>(4, &ctrl));
-    NDMPS_CUDA_TRY(cudaMemsetAsync(ctrl, 0, 4 * sizeof(unsigned), ctx->stream));
-    double stop_rel = 2.220446049250313e-16;
-    void* args[] = {&G, &n, &rows_per, &Lcol, &cand_rows, &cand, &ctrl, &stop_rel};
-    NDMPS_TRY(coop_launch(ctx, (const void*)pivoted_cholesky_kernel, dim3(ncta), dim3(256), args, smem));
-    int* host_flag = reinterpret_cast<int*>(ctx->pinned);
-    NDMPS_TRY(readback(ctx, host_flag, ctrl + 1, sizeof(int)));
-    NDMPS_CUDA_TRY(stream_wait(ctx));
-    *rank_out = host_flag[0];
     return NDMPS_OK;
 }
 
@@ -1325,7 +971,7 @@ static int pivoted_cholesky(ndmps_ctx* ctx, const double* G, int n, double* Lcol
 int eigh_small_async(ndmps_ctx* ctx, double* a_in, int n, double* evals_dev, double* evecs_dev, float quad_stop2, int** info_dev,
                      double diag_tol) {
     NDMPS_REQUIRE(n >= 2 && n <= 64, "eigh_small_async: n = %d outside 2..64", n);
-    const int max_sweeps = (int)ctx->opt_jacobi_max_sweeps;
+    const int max_sweeps = JACOBI_MAX_SWEEPS;
     const double tol = jacobi_tol(n);
     const double tol2 = tol * tol;
     int* info = nullptr;
@@ -1348,8 +994,6 @@ int eigh_small_async(ndmps_ctx* ctx, double* a_in, int n, double* evals_dev, dou
 int eigh(ndmps_ctx* ctx, double* a_in, int64_t n64, double* evals_dev, double* evecs_dev, double tol_override) {
     NDMPS_REQUIRE(n64 >= 1 && n64 <= 16384, "eigh: n = %lld outside 1..16384", (long long)n64);
     const int n = (int)n64;
-    const int max_sweeps = (int)ctx->opt_jacobi_max_sweeps;
-    const size_t smem_cap = ctx->smem_optin > 4096 ? ctx->smem_optin - 2048 : 0;
     NDMPS_TRY(ensure_pinned(ctx, 64));
     int sweeps_used = 0;
     double* norms = nullptr;
@@ -1361,7 +1005,7 @@ int eigh(ndmps_ctx* ctx, double* a_in, int64_t n64, double* evals_dev, double* e
     if (tol_override > tol) tol = tol_override;
     const double tol2 = tol * tol;
 
-    if (ctx->opt_eig_small && n >= 2 && n <= 64) {
+    if (n >= 2 && n <= 64) {
         // one launch; the convergence code is read back here because the eigenvalues are needed on the host next
         int* info = nullptr;
         NDMPS_TRY(eigh_small_async(ctx, a_in, n, evals_dev, evecs_dev, tol_override > 0.0 ? 1e-14f : 0.f, &info));
@@ -1369,7 +1013,7 @@ int eigh(ndmps_ctx* ctx, double* a_in, int64_t n64, double* evals_dev, double* e
         NDMPS_TRY(readback(ctx, host_flag, info, 2 * sizeof(int)));
         NDMPS_CUDA_TRY(stream_wait(ctx));
         if (host_flag[0] < 0) {
-            set_error("eigh: Jacobi did not converge in %d sweeps (n = %d, single-CTA solver)", max_sweeps, n);
+            set_error("eigh: Jacobi did not converge in %d sweeps (n = %d, single-CTA solver)", JACOBI_MAX_SWEEPS, n);
             return NDMPS_ERR_NOCONV;
         }
         ctx->last_eig_sweeps = host_flag[0];
@@ -1381,7 +1025,7 @@ int eigh(ndmps_ctx* ctx, double* a_in, int64_t n64, double* evals_dev, double* e
     double* cols = a_in;      // the column set Jacobi works on
     int ncols = n;
     int square = 0;           // eigenvalue = column norm (Jacobi on G) or its square (Jacobi on L)
-    const bool use_chol = ctx->opt_eig_cholesky && n > 32 && n <= 1024;
+    const bool use_chol = n > 64 && n <= 1024;      // n = 1 takes neither the Cholesky nor a sweep
     if (use_chol) {
         double* Lcol = nullptr;
         NDMPS_TRY(ctx->ws.get<double>((size_t)n * n, &Lcol));
@@ -1397,22 +1041,7 @@ int eigh(ndmps_ctx* ctx, double* a_in, int64_t n64, double* evals_dev, double* e
         null_floor_kernel<<<1, 256, 0, ctx->stream>>>(norms, n, ncols, floor2);
         NDMPS_LAUNCH_CHECK(ctx);
     }
-    if (!use_chol && n >= 2 && n <= 32 && (size_t)n * n * sizeof(double) <= smem_cap) {
-        unsigned* ctrl = nullptr;
-        NDMPS_TRY(ctx->ws.get<unsigned>(4, &ctrl));
-        NDMPS_CUDA_TRY(cudaMemsetAsync(ctrl, 0, 4 * sizeof(unsigned), ctx->stream));
-        int matches = (n + 1) / 2;
-        int warps = (matches + 3) / 4;                        // four pairs per warp
-        NDMPS_TRY(run_single<4>(ctx, cols, n, warps, max_sweeps, ctrl, tol2, floor2, (size_t)n * n * sizeof(double)));
-        int* host_flag = reinterpret_cast<int*>(ctx->pinned);
-        NDMPS_TRY(readback(ctx, host_flag, ctrl + 1, sizeof(int)));
-        NDMPS_CUDA_TRY(stream_wait(ctx));
-        if (host_flag[0] <= 0) {
-            set_error("eigh: Jacobi did not converge in %d sweeps (n = %d)", max_sweeps, n);
-            return NDMPS_ERR_NOCONV;
-        }
-        sweeps_used = host_flag[0];
-    } else if (ncols >= 2) {
+    if (ncols >= 2) {
         // float32 payloads (loosened tolerance): a sweep whose largest rotated off-diagonal was below
         // 1e-7 relative leaves less than the tolerance behind (quadratic convergence), so it is the last
         const float quad_stop2 = tol_override > 0.0 ? 1e-14f : 0.f;

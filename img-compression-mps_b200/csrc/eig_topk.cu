@@ -950,10 +950,10 @@ __global__ void __launch_bounds__(256) symmetrise_kernel(double* H, int m) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// 5a. Back-transformation, n <= 1024: one warp (one CTA) per Ritz vector, TWO reflectors per dependent
+// 5. Back-transformation, n <= 1024: one warp (one CTA) per Ritz vector, TWO reflectors per dependent
 // reduction.  With d = v_j.z, e = v_{j-1}.z and g = v_{j-1}.v_j (three dot products of one pass, reduced by
 // interleaved butterflies),  H_{j-1} H_j z = z - tau_j d v_j - tau_{j-1} (e - tau_j d g) v_{j-1}:
-// (n - 2) / 2 reduction latencies instead of n - 2.  The reflector rows arrive through a cp.async ring of
+// (n - 2) / 2 reduction latencies instead of n - 2 (the one-reflector form took about twice as long).  The reflector rows arrive through a cp.async ring of
 // PAIRS_AHEAD pairs in shared memory (only the 16-byte chunks right of the zero part), so the L2 latency of a row
 // is paid PAIRS_AHEAD pairs before it is used.  U[i * ldu + t] = z_i.
 // ---------------------------------------------------------------------------------------------
@@ -1029,66 +1029,6 @@ backtransform_pair_kernel(const double* __restrict__ V, int ldv, const double* _
 #pragma unroll
         for (int q = 0; q < NE; q++) z[q] = fma(-cb, b[q], fma(-ca, a[q], z[q]));
         __syncwarp();                                    // the slot is refilled PAIRS_AHEAD - 1 pairs from now
-    }
-#pragma unroll
-    for (int q = 0; q < NE; q++) {
-        const int k = lane + 32 * q;
-        if (k < n) U[(size_t)k * ldu + t] = z[q];
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
-// 5b. The previous form (kept for the option topk_bt_pairs = 0): one warp per Ritz vector (four per CTA, sharing the reflector rows
-// through L1), z <- H_0 H_1 ... H_{n-3} z.  The next reflector is loaded into registers while the
-// current one is applied; 32-column chunks that lie entirely in the zero part of a reflector
-// are skipped.  U[i * ldu + t] = z_i.
-// (Staging the rows through a shared-memory cp.async ring was measured slower.)
-// ---------------------------------------------------------------------------------------------
-template <int NE>
-__global__ void __launch_bounds__(128)
-backtransform_kernel(const double* __restrict__ V, int ldv, const double* __restrict__ tau_g, int n, const double* __restrict__ Zt,
-                     int m, double* __restrict__ U, int64_t ldu) {
-    const int lane = threadIdx.x & 31, t = blockIdx.x * 4 + (threadIdx.x >> 5);
-    if (t >= m) return;
-    double z[NE], va[NE], vb[NE];
-#pragma unroll
-    for (int q = 0; q < NE; q++) {
-        const int k = lane + 32 * q;
-        z[q] = k < n ? Zt[(size_t)t * n + k] : 0.0;
-    }
-    auto load = [&](double* dst, int j) {
-        const double* v = V + (size_t)j * ldv;
-        const int q0 = (j + 1) >> 5;
-#pragma unroll
-        for (int q = 0; q < NE; q++) {
-            const int k = lane + 32 * q;
-            dst[q] = (q >= q0 && k > j && k < n) ? __ldg(v + k) : 0.0;
-        }
-    };
-    auto apply = [&](const double* v, int j) {
-        const double tau = __ldg(tau_g + j);
-        const int q0 = (j + 1) >> 5;
-        double d0 = 0.0, d1 = 0.0;
-#pragma unroll
-        for (int q = 0; q < NE; q += 2) {
-            if (q >= q0) d0 = fma(v[q], z[q], d0);
-            if (q + 1 >= q0) d1 = fma(v[q + 1], z[q + 1], d1);
-        }
-        const double dot = warp_sum(d0 + d1) * tau;
-#pragma unroll
-        for (int q = 0; q < NE; q++)
-            if (q >= q0) z[q] = fma(-dot, v[q], z[q]);
-    };
-    int j = n - 3;
-    if (j >= 0) load(va, j);
-    while (j >= 0) {
-        if (j >= 1) load(vb, j - 1);
-        apply(va, j);
-        if (j >= 1) {
-            if (j >= 2) load(va, j - 2);
-            apply(vb, j - 1);
-        }
-        j -= 2;
     }
 #pragma unroll
     for (int q = 0; q < NE; q++) {
@@ -1199,11 +1139,11 @@ int eigh_topk(ndmps_ctx* ctx, const double* G, int64_t n64, int64_t k64, double*
     if (n64 < 96 || n64 > NMAX || k64 < 1 || k64 > 128 || 2 * k64 > n64) return NDMPS_OK;
     const int n = (int)n64, m = (int)k64;
     // 1024 < n <= 1536: still register-resident, 11 warps x one row per CTA, if that many CTAs fit the device
-    const bool mid = n > 1024 && n <= 1536 && (n + MID_NT / 32 - 1) / (MID_NT / 32) <= ctx->sm_count && ctx->opt_topk_mid;
+    const bool mid = n > 1024 && n <= 1536 && (n + MID_NT / 32 - 1) / (MID_NT / 32) <= ctx->sm_count;
     const bool big = n > 1024 && !mid;
     // register route: RPW rows per warp.  Two rows per warp up to n = 512 (the row pair still fits the register
     // file) halve the SMs a reduction sits on, which is what the other volumes in flight need
-    const int rpw = (n <= 512 && !ctx->opt_topk_one_row) ? 2 : 1;
+    const int rpw = n <= 512 ? 2 : 1;
     const int C = big ? ctx->sm_count : (mid ? (n + MID_NT / 32 - 1) / (MID_NT / 32) : (n + rpw * (TDT / 32) - 1) / (rpw * (TDT / 32)));
     const size_t smem_iv = (size_t)6 * n * sizeof(double) + (size_t)n + 16;
     const size_t smem_ch = (size_t)(chol_two_buffers(ctx, m) ? 2 : 1) * m * (m + 1) * sizeof(double);
@@ -1254,7 +1194,6 @@ int eigh_topk(ndmps_ctx* ctx, const double* G, int64_t n64, int64_t k64, double*
         int per_sm = 1;
         NDMPS_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, tridiag_big_kernel, TDT, smem_big));
         per_sm = per_sm < 1 ? 1 : (per_sm > 3 ? 3 : per_sm);
-        if (ctx->opt_topk_big_ctas > 0) per_sm = (int)ctx->opt_topk_big_ctas;
         void* args[] = {&Awork, &n_arg, &ldv_arg, &V, &tau, &d, &e, &pbuf, &rowbuf, &ctrl};
         NDMPS_TRY(coop_launch(ctx, (const void*)tridiag_big_kernel, dim3(C * per_sm), dim3(TDT), args, smem_big));
     } else {
@@ -1289,8 +1228,7 @@ int eigh_topk(ndmps_ctx* ctx, const double* G, int64_t n64, int64_t k64, double*
             if (n > 1024) {
                 NDMPS_TRY(coop_launch(ctx, (const void*)tridiag_kernel<48, 1, false, MID_NT>, dim3(C), dim3(MID_NT), args, 0));
             } else {
-                void* fn = n <= 512 ? (rpw == 2 ? (void*)tridiag_kernel<16, 2, false, TDT> : (void*)tridiag_kernel<16, 1, false, TDT>)
-                                    : (void*)tridiag_kernel<32, 1, false, TDT>;
+                void* fn = n <= 512 ? (void*)tridiag_kernel<16, 2, false, TDT> : (void*)tridiag_kernel<32, 1, false, TDT>;
                 NDMPS_TRY(coop_launch(ctx, fn, dim3(C), dim3(TDT), args, 0));
             }
         }
@@ -1307,12 +1245,12 @@ int eigh_topk(ndmps_ctx* ctx, const double* G, int64_t n64, int64_t k64, double*
 #endif
     }
     // 2. shifts
-    const int passes = ctx->opt_topk_passes > 0 ? (int)ctx->opt_topk_passes : 8;
+    const int passes = 8;
     bisect_kernel<<<m, BIS, (size_t)2 * n * sizeof(double), ctx->stream>>>(d, e, n, passes, lam, bounds);
     NDMPS_LAUNCH_CHECK(ctx);
     // 3. inverse iteration (the LU factors of step 1 are reused), re-orthonormalised between steps;
     //    the last basis is orthonormalised twice
-    const int iters = ctx->opt_topk_iters > 0 ? (int)ctx->opt_topk_iters : 2;   // the Ritz residuals are checked below
+    const int iters = 2;                                 // the Ritz residuals are checked below
     const double* rhs = nullptr;
     for (int it = 0; it < iters; it++) {
         invit_kernel<<<m, 32, smem_iv, ctx->stream>>>(d, e, n, lam, bounds, rhs, Xa, factors, it > 0 ? 1 : 0);
@@ -1332,19 +1270,15 @@ int eigh_topk(ndmps_ctx* ctx, const double* G, int64_t n64, int64_t k64, double*
     // no host round trip.  Converged Ritz vectors of separated eigenvalues give a diagonal H (off-diagonals at the
     // residual level): then the block is passed through; clusters keep the Jacobi rotation.  Either way the residual
     // check below decides whether the result is used.
-    if (m >= 2 && m <= 64) NDMPS_TRY(eigh_small_async(ctx, H, m, hev, W, 1e-16f, &rr_info, ctx->opt_topk_rr_skip ? 1e-13 : 0.0));
-    else {
-        bool passed = false;
-        if (ctx->opt_topk_rr_skip) {                     // one short host round trip against 1.6 ms of the general solver
-            int* flag = info + 2;
-            rr_passthrough_kernel<<<1, 512, 0, ctx->stream>>>(H, m, 1e-13, hev, W, flag);
-            NDMPS_LAUNCH_CHECK(ctx);
-            NDMPS_TRY(ensure_pinned(ctx, 64));
-            NDMPS_TRY(readback(ctx, ctx->pinned, flag, sizeof(int)));
-            NDMPS_CUDA_TRY(stream_wait(ctx));
-            passed = *reinterpret_cast<const int*>(ctx->pinned) == 1;
-        }
-        if (!passed) NDMPS_TRY(eigh(ctx, H, m, hev, W, 0.0));
+    if (m >= 2 && m <= 64) NDMPS_TRY(eigh_small_async(ctx, H, m, hev, W, 1e-16f, &rr_info, 1e-13));
+    else {                                               // one short host round trip against 1.6 ms of the general solver
+        int* flag = info + 2;
+        rr_passthrough_kernel<<<1, 512, 0, ctx->stream>>>(H, m, 1e-13, hev, W, flag);
+        NDMPS_LAUNCH_CHECK(ctx);
+        NDMPS_TRY(ensure_pinned(ctx, 64));
+        NDMPS_TRY(readback(ctx, ctx->pinned, flag, sizeof(int)));
+        NDMPS_CUDA_TRY(stream_wait(ctx));
+        if (*reinterpret_cast<const int*>(ctx->pinned) != 1) NDMPS_TRY(eigh(ctx, H, m, hev, W, 0.0));
     }
     // Zt[c] = sum_r W[r][c] Q[r]
     combine_rows_kernel<<<dim3((unsigned)((n + 127) / 128), (unsigned)((m + 7) / 8)), 128, 0, ctx->stream>>>(W, 1, m, Xa, m, n, Xb);
@@ -1354,7 +1288,7 @@ int eigh_topk(ndmps_ctx* ctx, const double* G, int64_t n64, int64_t k64, double*
     ritz_residual_kernel<<<m, 128, 0, ctx->stream>>>(d, e, Xb, hev, n, res);
     NDMPS_LAUNCH_CHECK(ctx);
     // 5. back-transform
-    if (n <= 1024 && ctx->opt_topk_bt_pairs) {
+    if (n <= 1024) {
         const size_t ring = (size_t)(PAIRS_AHEAD * 2 + 1) * (n <= 512 ? 512 : 1024) * sizeof(double);
         if (n <= 512) {
             NDMPS_TRY(raise_dynamic_smem((const void*)backtransform_pair_kernel<16>, ctx->device, (int)ring));
@@ -1363,9 +1297,7 @@ int eigh_topk(ndmps_ctx* ctx, const double* G, int64_t n64, int64_t k64, double*
             NDMPS_TRY(raise_dynamic_smem((const void*)backtransform_pair_kernel<32>, ctx->device, (int)ring));
             backtransform_pair_kernel<32><<<(unsigned)m, 32, ring, ctx->stream>>>(V, ldv, tau, n, Xb, U, ldu);
         }
-    } else if (n <= 512) backtransform_kernel<16><<<(unsigned)((m + 3) / 4), 128, 0, ctx->stream>>>(V, ldv, tau, n, Xb, m, U, ldu);
-    else if (n <= 1024) backtransform_kernel<32><<<(unsigned)((m + 3) / 4), 128, 0, ctx->stream>>>(V, ldv, tau, n, Xb, m, U, ldu);
-    else backtransform_big_kernel<<<m, TDT, 0, ctx->stream>>>(V, ldv, tau, n, Xb, U, ldu);
+    } else backtransform_big_kernel<<<m, TDT, 0, ctx->stream>>>(V, ldv, tau, n, Xb, U, ldu);
     NDMPS_LAUNCH_CHECK(ctx);
     finish_kernel<<<1, 256, 0, ctx->stream>>>(G, n, hev, m, info, rr_info, res, bounds, out_dev);
     NDMPS_LAUNCH_CHECK(ctx);

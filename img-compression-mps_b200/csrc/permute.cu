@@ -182,119 +182,6 @@ permute_tiled_kernel(const T* __restrict__ src, T* __restrict__ dst, const TileA
 }
 
 // ---------------------------------------------------------------------------------------------
-// Bulk-copy variant: the global traffic is issued by the TMA engine, not by the threads.
-//   cp.async.bulk.shared.global  : one copy per contiguous SOURCE run, completion on an mbarrier
-//   threads                      : gather shared -> shared into destination order (slot table)
-//   cp.async.bulk.global.shared  : one copy per contiguous DESTINATION run (bulk async-group)
-// Two-stage ring: the loads of tile t+1 are in flight while tile t is gathered and stored.
-// ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, unsigned count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, unsigned parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_LOOP:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra DONE;\n"
-        "bra WAIT_LOOP;\n"
-        "DONE:\n"
-        "}\n" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void bulk_load(void* smem_dst, const void* gsrc, unsigned bytes, uint64_t* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(smem_dst)),
-                 "l"(gsrc), "r"(bytes), "r"(smem_u32(bar))
-                 : "memory");
-}
-__device__ __forceinline__ void bulk_store(void* gdst, const void* smem_src, unsigned bytes) {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst), "r"(smem_u32(smem_src)), "r"(bytes)
-                 : "memory");
-}
-
-struct BulkArgs {
-    int tile, pa, pb, n_outer, run_pad;
-    int64_t n_tiles;
-    uint32_t outer_extent[NDMPS_MAX_DIGITS];
-    int64_t outer_dst[NDMPS_MAX_DIGITS];
-    int64_t outer_src[NDMPS_MAX_DIGITS];
-    const int64_t* hi_src;
-    const int64_t* hi_dst;
-    const uint16_t* rslot;
-};
-
-template <class T>
-__global__ void __launch_bounds__(PERM_THREADS)
-permute_bulk_kernel(const T* __restrict__ src, T* __restrict__ dst, const BulkArgs ba, double scale, bool do_scale) {
-    extern __shared__ __align__(128) unsigned char perm_smem[];
-    const int nruns_in = ba.tile / ba.pb, nruns_out = ba.tile / ba.pa;
-    const int in_elems = nruns_in * (ba.pb + ba.run_pad);
-    T* inbuf = reinterpret_cast<T*>(perm_smem);                       // 2 x in_elems
-    T* outbuf = inbuf + 2 * (size_t)in_elems;                         // 2 x tile
-    __shared__ __align__(8) uint64_t bars[2];
-    const int tid = threadIdx.x;
-    if (tid == 0) { mbar_init(&bars[0], 1); mbar_init(&bars[1], 1); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    __syncthreads();
-
-    auto tile_bases = [&](int64_t tile, int64_t& base_dst, int64_t& base_src) {
-        int64_t rem = tile;
-        base_dst = 0; base_src = 0;
-        for (int j = ba.n_outer - 1; j >= 0; j--) {
-            int64_t q = rem / ba.outer_extent[j];
-            int64_t d = rem - q * ba.outer_extent[j];
-            base_dst += d * ba.outer_dst[j];
-            base_src += d * ba.outer_src[j];
-            rem = q;
-        }
-    };
-    auto issue_loads = [&](int64_t tile, int stage) {
-        int64_t bd, bs;
-        tile_bases(tile, bd, bs);
-        if (tid == 0) mbar_expect_tx(&bars[stage], (unsigned)(ba.tile * sizeof(T)));
-        __syncwarp();
-        for (int r = tid; r < nruns_in; r += PERM_THREADS)
-            bulk_load(inbuf + (size_t)stage * in_elems + (size_t)r * (ba.pb + ba.run_pad), src + bs + ba.hi_src[r],
-                      (unsigned)(ba.pb * sizeof(T)), &bars[stage]);
-    };
-
-    int64_t tile = blockIdx.x;
-    int it = 0;
-    if (tile < ba.n_tiles) issue_loads(tile, 0);
-    for (; tile < ba.n_tiles; tile += gridDim.x, it++) {
-        const int stage = it & 1;
-        const int64_t next = tile + gridDim.x;
-        // the other input stage was fully gathered in the previous iteration (barrier at its end)
-        if (next < ba.n_tiles) issue_loads(next, stage ^ 1);
-        mbar_wait(&bars[stage], (unsigned)((it >> 1) & 1));
-        // outbuf[stage] was handed to bulk stores two iterations ago: they must have read it
-        if (tid < 32) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
-        __syncthreads();
-        const T* in = inbuf + (size_t)stage * in_elems;
-        T* out = outbuf + (size_t)stage * ba.tile;
-        for (int w = tid; w < ba.tile; w += PERM_THREADS) {
-            T v = in[ba.rslot[w]];
-            if (do_scale) v = (T)((double)v * scale);
-            out[w] = v;
-        }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy writes -> visible to the bulk engine
-        __syncthreads();
-        int64_t bd, bs;
-        tile_bases(tile, bd, bs);
-        if (tid < 32) {
-            for (int r = tid; r < nruns_out; r += 32)
-                bulk_store(dst + bd + ba.hi_dst[r], out + (size_t)r * ba.pa, (unsigned)(ba.pa * sizeof(T)));
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-        }
-    }
-    if (tid < 32) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
-}
-
-// ---------------------------------------------------------------------------------------------
 // Register-only permutation for power-of-two shapes (256^3, 512^3, 2^k images): every factor is a power of two, so
 // the voxel -> site map permutes the BITS of the element offset (a Morton-style interleave).  No shared memory, no
 // tables, no barrier.  In both directions destination bit 0 is source bit 0 (the last axis' lowest digit); a thread
@@ -526,38 +413,6 @@ static void build_tile_plan(const DigitList& dl, TilePlan& tp) {
         for (int k = 0; k < 32; k++) worst = cnt[k] > worst ? cnt[k] : worst;
     }
     tp.conflict = worst;
-    // gather table of the bulk-copy variant: try paddings of 0..28 words between source runs
-    // (multiples of 4 keep the 16-byte alignment bulk copies need) and keep the least conflicting
-    {
-        std::vector<int> read_of_write((size_t)tile, 0);
-        for (int64_t r = 0; r < tile; r++) {
-            int w = tp.pos[(size_t)r];
-            w -= (w / 33);                                   // undo skew_slot: s = w + w/32  =>  w = s - s/33
-            read_of_write[(size_t)w] = (int)r;
-        }
-        int best_pad = 0, best_conf = 1 << 30;
-        for (int pad = 0; pad <= 28; pad += 4) {
-            if ((tile / pb) * (pb + pad) > 65535) break;
-            int conf = 1;
-            for (int64_t w0 = 0; w0 + 32 <= tile; w0 += 32) {
-                int cnt[32] = {0};
-                for (int k = 0; k < 32; k++) {
-                    int r = read_of_write[(size_t)(w0 + k)];
-                    int slot = (r / (int)pb) * ((int)pb + pad) + r % (int)pb;
-                    cnt[slot & 31]++;
-                }
-                for (int k = 0; k < 32; k++) conf = cnt[k] > conf ? cnt[k] : conf;
-            }
-            if (conf < best_conf) { best_conf = conf; best_pad = pad; }
-        }
-        tp.run_pad = best_pad;
-        tp.gather_conflict = best_conf;
-        tp.rslot.assign((size_t)tile, 0);
-        for (int64_t w = 0; w < tile; w++) {
-            int r = read_of_write[(size_t)w];
-            tp.rslot[(size_t)w] = (uint16_t)((r / (int)pb) * ((int)pb + best_pad) + r % (int)pb);
-        }
-    }
     tp.ok = true;
 }
 
@@ -574,8 +429,6 @@ static int upload_tile_plan(TilePlan& tp, int device, TilePlan::DevTables* out) 
     NDMPS_CUDA_TRY(cudaMalloc(&d.hi_src, tp.hi_src.size() * sizeof(int64_t)));
     NDMPS_CUDA_TRY(cudaMalloc(&d.hi_dst, tp.hi_dst.size() * sizeof(int64_t)));
     NDMPS_CUDA_TRY(cudaMalloc(&d.pos, tp.pos.size() * sizeof(uint16_t)));
-    NDMPS_CUDA_TRY(cudaMalloc(&d.rslot, tp.rslot.size() * sizeof(uint16_t)));
-    NDMPS_CUDA_TRY(cudaMemcpy(d.rslot, tp.rslot.data(), tp.rslot.size() * sizeof(uint16_t), cudaMemcpyHostToDevice));
     NDMPS_CUDA_TRY(cudaMemcpy(d.hi_src, tp.hi_src.data(), tp.hi_src.size() * sizeof(int64_t), cudaMemcpyHostToDevice));
     NDMPS_CUDA_TRY(cudaMemcpy(d.hi_dst, tp.hi_dst.data(), tp.hi_dst.size() * sizeof(int64_t), cudaMemcpyHostToDevice));
     NDMPS_CUDA_TRY(cudaMemcpy(d.pos, tp.pos.data(), tp.pos.size() * sizeof(uint16_t), cudaMemcpyHostToDevice));
@@ -596,36 +449,6 @@ static int permute_tiled(ndmps_ctx* ctx, TilePlan& tp, const T* src, T* dst, dou
         ta.outer_src[j] = tp.outer_src[j];
     }
     ta.hi_src = dt.hi_src; ta.hi_dst = dt.hi_dst; ta.pos = dt.pos;
-    // ---- bulk-copy (TMA-class) variant: every run and offset must be a multiple of 16 bytes ----
-    {
-        const int q = 16 / (int)sizeof(T);
-        bool aligned = ctx->opt_permute_path == 3 && tp.pa % q == 0 && tp.pb % q == 0 &&
-                       reinterpret_cast<uintptr_t>(src) % 16 == 0 && reinterpret_cast<uintptr_t>(dst) % 16 == 0;
-        for (size_t k = 0; k < tp.hi_src.size() && aligned; k++) aligned = tp.hi_src[k] % q == 0;
-        for (size_t k = 0; k < tp.hi_dst.size() && aligned; k++) aligned = tp.hi_dst[k] % q == 0;
-        for (int j = 0; j < tp.n_outer && aligned; j++) aligned = tp.outer_dst[j] % q == 0 && tp.outer_src[j] % q == 0;
-        const size_t in_elems = (size_t)(tp.tile / tp.pb) * (tp.pb + tp.run_pad);
-        const size_t bsmem = (2 * in_elems + 2 * (size_t)tp.tile) * sizeof(T) + 128;
-        if (aligned && bsmem <= ctx->smem_optin - 2048 && (tp.pb + tp.run_pad) * sizeof(T) % 16 == 0) {
-            BulkArgs ba;
-            ba.tile = tp.tile; ba.pa = tp.pa; ba.pb = tp.pb; ba.n_outer = tp.n_outer; ba.run_pad = tp.run_pad; ba.n_tiles = tp.n_tiles;
-            for (int j = 0; j < tp.n_outer; j++) {
-                ba.outer_extent[j] = tp.outer_extent[j];
-                ba.outer_dst[j] = tp.outer_dst[j];
-                ba.outer_src[j] = tp.outer_src[j];
-            }
-            ba.hi_src = dt.hi_src; ba.hi_dst = dt.hi_dst; ba.rslot = dt.rslot;
-            NDMPS_TRY(raise_dynamic_smem((const void*)permute_bulk_kernel<T>, ctx->device, (int)ctx->smem_optin - 2048));
-            int per_sm = (int)((ctx->smem_optin - 2048) / (bsmem + 1024));
-            if (per_sm < 1) per_sm = 1;
-            if (per_sm > 4) per_sm = 4;
-            int64_t bgrid = (int64_t)ctx->sm_count * per_sm;
-            if (bgrid > tp.n_tiles) bgrid = tp.n_tiles;
-            permute_bulk_kernel<T><<<(unsigned)bgrid, PERM_THREADS, bsmem, ctx->stream>>>(src, dst, ba, scale, do_scale);
-            NDMPS_LAUNCH_CHECK(ctx);
-            return NDMPS_OK;
-        }
-    }
     const size_t smem = (size_t)(skew_slot(tp.tile) + 8) * sizeof(T);
     {
         // float64 tiles exceed the 48 KB default
@@ -635,7 +458,7 @@ static int permute_tiled(ndmps_ctx* ctx, TilePlan& tp, const T* src, T* dst, dou
     int64_t grid = tp.n_tiles;
     // measured: the fewer tiles a CTA walks the better (the hardware scheduler balances the tail); 64 CTAs
     // per SM in the grid means one tile per CTA up to 512^3 and a grid-stride loop beyond
-    int64_t cap = (int64_t)ctx->sm_count * (ctx->opt_permute_ctas > 0 ? ctx->opt_permute_ctas : 64);
+    int64_t cap = (int64_t)ctx->sm_count * 64;
     if (grid > cap) grid = cap;
     // 16-byte accesses when every run and every run offset is a multiple of 4 elements (float32 only)
     bool vec4 = sizeof(T) == 4 && (tp.pa % 4 == 0) && (tp.pb % 4 == 0) &&
@@ -773,7 +596,6 @@ int ndmps_plan_destroy(ndmps_plan_t* plan) {
                 cudaFree(d.hi_src);
                 cudaFree(d.hi_dst);
                 cudaFree(d.pos);
-                cudaFree(d.rslot);
                 if (d.device != cur) cudaSetDevice(cur);
             }
             tp->dev.clear();

@@ -7,7 +7,7 @@
 //   * left factor from the Gram matrix G = M M^T (float64 accumulation) and a
 //     float64 Jacobi eigensolve: U = eigenvectors, s = sqrt(lambda); the remainder
 //     is T = U_r^T M (= diag(s) V^T, weight absorbed right as quimb does).
-//   * FRONT MERGING: consecutive sites whose fused row count stays <= merge_cap
+//   * FRONT MERGING: consecutive sites whose fused row count stays <= MERGE_CAP (512)
 //     share ONE Gram pass and ONE projection pass over the big unfolding.  With
 //     rows (a, s_i, .., s_{i+k-1}) fused, the Gram of sub-step j is
 //         G_j = (P_j (x) I)^T  Tr_rest(G)  (P_j (x) I)
@@ -22,6 +22,8 @@
 #include "common.cuh"
 
 namespace ndmps {
+
+constexpr int64_t MERGE_CAP = 512;   // largest fused row count of a front-merged group of sites
 
 // ---------------------------------------------------------------------------------
 // small float64 glue kernels
@@ -320,7 +322,7 @@ static int ttsvd(ndmps_ctx* ctx, const void* dense, int dtype, int L, const int6
         int k = 1;
         while (site + k < L - 1) {
             int64_t Dn = D * dims[site + k], Cn = C / dims[site + k];
-            if (Dn <= ctx->opt_merge_cap && Dn <= Cn) { D = Dn; C = Cn; k++; } else break;
+            if (Dn <= MERGE_CAP && Dn <= Cn) { D = Dn; C = Cn; k++; } else break;
         }
         if (sh) {
             // sharded phase ends when the global remainder is small or the local block gets wider than long

@@ -84,13 +84,15 @@ class VolumePipeline:
             # a spinning waiter per worker of every rank of the node, plus the ranks' main threads, must each find a core
             blocking_sync = (self.workers + 1) * ranks_here > max(1, usable - 1)
         self.blocking_sync = bool(blocking_sync)
-        # how a worker's native context waits inside the sweep (ndmps option blocking_sync): 0 spin, 1 sleep, 2 poll the event + yield,
-        # 3 watch a pinned word the stream writes + yield (no driver calls while waiting).
-        # Oversubscribed nodes poll and yield: the sweep's waits are short, a driver sleep costs a wake-up per wait
+        # how a worker's native context waits inside the sweep (ndmps option blocking_sync): 0 spin, 3 watch a pinned word the
+        # stream writes + yield (no driver calls while waiting).  Oversubscribed nodes watch and yield: the sweep's waits are
+        # short, and a sleep in the driver costs a wake-up per wait
         env_mode = os.environ.get("NDMPS_WAIT_MODE")
         if wait_mode is None and env_mode is not None:
             wait_mode = int(env_mode)
         self.wait_mode = int(wait_mode) if wait_mode is not None else (3 if self.blocking_sync else 0)
+        if self.wait_mode not in (0, 3):                # checked here: a worker thread that failed to start would hang the barrier
+            raise ValueError(f"wait_mode must be 0 (spin) or 3 (pinned word), got {self.wait_mode}")
         self._ctx_lock = threading.Lock()
         self._contexts = []                             # the workers' native contexts (for launch counts / options)
         self._queues = [queue.SimpleQueue() for _ in range(self.workers)]

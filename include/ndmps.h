@@ -74,15 +74,23 @@ int ndmps_ctx_stage_times(ndmps_ctx_t* ctx, double* ms_out, int64_t* calls_out, 
 /* counters: "eig_flops" (rotation + factorisation flops of the bond eigensolves), "eig_calls",
  * "workspace_bytes" (arena high-water mark). */
 int ndmps_ctx_get_stat(ndmps_ctx_t* ctx, const char* name, double* value_out, int reset);
-/* knobs (defaults in parentheses):
- *   "eig_topk" (1)       bond cap set: leading-eigenpair solver instead of the full one when the cap provably binds
- *   "topk_iters" (2), "topk_passes" (8), "topk_big_ctas" (occupancy)   inverse-iteration steps, bisection passes, CTAs/SM of the n > 1024 reduction
- *   "topk_one_row" (0)   one matrix row per warp in the register-resident reduction (faster alone, worse beside other volumes)
- *   "merge_cap" (512)    largest fused row count of a front-merged group of sites
- *   "eig_cholesky" (1), "eig_small" (1), "chol_blocked" (1), "chol_cluster" (0), "chol_rows", "jacobi_block", "jacobi_max_sweeps" (40)
- *   "gram_path", "gemm_path" (0 = FP64 tensor pipe when the shape allows, 2 = SIMT only), "permute_path" (0 tiles, 3 bulk copies, 2 gather), "permute_ctas" (64)
- *   "blocking_sync" (0)  host waits sleep on a blocking event instead of spinning (more waiting host threads than cores)
- *   "verbose" (0)
+/* options: name (default) values - what the option is for.  An unknown name, or a value outside the listed set of
+ * permute_path / blocking_sync, returns NDMPS_ERR_INVALID.
+ *   "gram_path" (0)      0 auto (tcgen05 in a capped float32 sweep, else the FP64 tensor pipe when the shape allows),
+ *                        2 SIMT kernel, 3 tcgen05 - lets tests compare the Gram routes
+ *   "gemm_path" (0)      0 FP64 tensor pipe when the shape allows, 2 SIMT only, 3 tcgen05 - lets tests compare the routes
+ *   "gemm_out_t" (0)     1: ndmps_gemm writes C transposed through the tcgen05 epilogue - test hook
+ *   "tc" (1)             0/1: tcgen05 contractions on bf16x3 planes for float32 payloads of a capped sweep / reconstruction
+ *   "tc_waves" (1)       waves of integer-Gram CTAs (split-K factor = waves x SMs / tiles) - tests check it is the same bound
+ *   "permute_path" (0)   0 register bit-permutation when the shape allows, else shared-memory tiles; 1 tiles always;
+ *                        2 gather kernel - 1 and 2 are the references of the permutation tests
+ *   "eig_topk" (1)       0/1: leading-eigenpair solver when a bond cap provably binds - 0, the full solver, is its reference
+ *   "topk_cluster" (1)   0/1: n <= 512 tridiagonalisation as one thread-block cluster - 0 forces the grid-barrier kernel
+ *                        that runs when the cluster does not fit the device
+ *   "ssim_exact" (0)     0/1: float64 SSIM arithmetic for float32 inputs too - the reference of the SSIM tests
+ *   "blocking_sync" (0)  host waits: 0 spin in cudaStreamSynchronize, 3 watch a pinned word the stream writes and yield
+ *                        (more waiting host threads than cores: batch.VolumePipeline picks)
+ *   "verbose" (0)        0/1: one line per eigensolve / sweep step on stderr - diagnostics
  * A context belongs to one host thread; several contexts (one per thread, each with its own stream) may run concurrently. */
 int ndmps_ctx_set_option(ndmps_ctx_t* ctx, const char* name, int64_t value);
 

@@ -248,29 +248,52 @@ def test_roundtrip_host_entry():
     assert np.linalg.norm(rec - ro) / np.linalg.norm(ro) < 1e-5
 
 
-def test_readback_routes_agree():
-    """Small device -> host read-backs (eigenvalues, flags, scalars) leave through SM stores into mapped pinned memory
-    by default and through cudaMemcpyAsync with readback = 1: same bytes either way, under every host wait mode."""
+def test_wait_modes_agree():
+    """The host waits of a sweep spin in cudaStreamSynchronize (blocking_sync = 0) or watch a pinned word the stream
+    writes (blocking_sync = 3): same bytes either way."""
     from imgcompressionmps import _native, _ops
     from imgcompressionmps.utils.metrics import compute_psnr, compute_ssim_by_dim
     x = phantom((64, 64, 64), seed=6, background=0.01).astype(np.float32)
     ctx = _native.context()
     results = []
     try:
-        for readback, wait in ((1, 0), (0, 0), (0, 3), (0, 2), (0, 1)):
-            ctx.set_option("readback", readback)
+        for wait in (0, 3):
             ctx.set_option("blocking_sync", wait)
             extras = {}
             rec, ranks = _ops.roundtrip_host(x, max_bond=16, extras=extras)
             results.append((rec, ranks, extras["norm"], extras["boundary_list"], compute_ssim_by_dim(rec, x), compute_psnr(rec, x)))
     finally:
-        ctx.set_option("readback", 0)
         ctx.set_option("blocking_sync", 0)
     for r in results[1:]:
         assert r[1] == results[0][1]
         assert np.array_equal(r[0], results[0][0])
         assert r[2] == results[0][2] and np.array_equal(r[3], results[0][3])
         assert r[4] == results[0][4] and r[5] == results[0][5]
+
+
+REMOVED_OPTIONS = ["permute_ctas", "merge_cap", "jacobi_max_sweeps", "jacobi_block", "eig_cholesky", "eig_small", "chol_blocked",
+                   "chol_cluster", "chol_rows", "topk_one_row", "topk_mid", "topk_bt_pairs", "topk_big_ctas", "topk_passes",
+                   "topk_iters", "topk_rr_skip", "readback", "tc_chunk"]
+
+
+def test_set_option_rejects_removed_names_and_values():
+    """Options whose paths were removed, and values of permute_path / blocking_sync that no longer select a path, raise
+    instead of silently running another path (a stale NDMPS_OPT_* or NDMPS_WAIT_MODE setting fails loudly)."""
+    from imgcompressionmps import _native
+    from imgcompressionmps.batch import VolumePipeline
+    ctx = _native.context()
+    for name in REMOVED_OPTIONS:
+        with pytest.raises(ValueError, match="unknown option"):
+            ctx.set_option(name, 1)
+    for name, value in (("permute_path", 3), ("permute_path", -1), ("blocking_sync", 1), ("blocking_sync", 2)):
+        with pytest.raises(ValueError, match=name):
+            ctx.set_option(name, value)
+    for wait in (1, 2):
+        with pytest.raises(ValueError, match="wait_mode"):
+            VolumePipeline(workers=1, wait_mode=wait)
+    for name, value in (("permute_path", 0), ("permute_path", 1), ("permute_path", 2), ("blocking_sync", 3), ("blocking_sync", 0)):
+        ctx.set_option(name, value)
+    ctx.set_option("permute_path", 0)
 
 
 # ---- capped bonds: leading-eigenpair solver vs the full solver ---------------------------------------

@@ -32,18 +32,15 @@ def main(which):
     ctx = _native.context()
     g = torch.Generator(device="cuda").manual_seed(0)
     if "eigh" in which:
-        for chol in (1, 0):
-            ctx.set_option("eig_cholesky", chol)
-            for n in (8, 64, 128, 256, 512, 1024):
-                a = torch.randn(n, 4 * n, dtype=torch.float64, device="cuda", generator=g)
-                gm = a @ a.T
-                try:
-                    ms = timeit(lambda: _ops.eigh(gm), reps=3, warm=1)
-                    _, _, sw = _ops.eigh(gm)
-                    print(f"eigh n={n} cholesky={chol}: {ms:.3f} ms, {sw} sweeps", flush=True)
-                except Exception as exc:
-                    print(f"eigh n={n} cholesky={chol}: FAILED {exc}", flush=True)
-        ctx.set_option("eig_cholesky", 1)
+        for n in (8, 64, 128, 256, 512, 1024):
+            a = torch.randn(n, 4 * n, dtype=torch.float64, device="cuda", generator=g)
+            gm = a @ a.T
+            try:
+                ms = timeit(lambda: _ops.eigh(gm), reps=3, warm=1)
+                _, _, sw = _ops.eigh(gm)
+                print(f"eigh n={n}: {ms:.3f} ms, {sw} sweeps", flush=True)
+            except Exception as exc:
+                print(f"eigh n={n}: FAILED {exc}", flush=True)
     if "topk" in which:
         from bench import synthetic_volume
         vol = torch.from_numpy(synthetic_volume((128, 128, 128), 7)).cuda().double()

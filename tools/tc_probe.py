@@ -3,7 +3,7 @@
 
     python tools/tc_probe.py [gram] [gemm] [sweep]
 
-gram : G = M M^T on bf16x3 planes for several drain chunks vs the FP64-tensor-pipe Gram (exact
+gram : G = M M^T on bf16x3 planes vs the FP64-tensor-pipe Gram (exact
        float64 accumulation of the same float32 data), on a random and a phantom unfolding.
 gemm : the four operand-major combinations and both output orders of gemm_tc vs torch float64.
 sweep: one 256^3 / 512^3 volume through NDMPS.from_tensor / to_tensor with the tcgen05 paths on and
@@ -45,25 +45,22 @@ def gram_case(name, m):
     exact = _ops.gram(m)
     t_dmma = timed(lambda: _ops.gram(m))
     lam = torch.linalg.eigvalsh(exact).flip(0)
-    for chunk in (0,):
-        ctx.set_option("gram_path", 3)
-        ctx.set_option("tc_chunk", chunk)
-        g = _ops.gram(m)
-        t_tc = timed(lambda: _ops.gram(m))
-        err = (g - exact)
-        rel_max = float(err.abs().max() / exact.abs().max())
-        nz = exact.diagonal() > 0
-        rel_diag = float((err.diagonal()[nz].abs() / exact.diagonal()[nz]).max())
-        mean_rel_diag = float((err.diagonal()[nz] / exact.diagonal()[nz]).mean())
-        lam_tc = torch.linalg.eigvalsh(g).flip(0)
-        k = min(64, lam.numel())
-        sv_err = float(((lam_tc[:k].clamp_min(0).sqrt() - lam[:k].clamp_min(0).sqrt()).abs() / lam[0].sqrt()).max())
-        sym = float((g - g.T).abs().max())
-        print(f"  gram {name} {tuple(m.shape)} chunk {chunk:3d}: tc {t_tc:.3f} ms (dmma {t_dmma:.3f} ms)  max|dG|/max|G| {rel_max:.2e}  "
-              f"diag rel max {rel_diag:.2e} mean {mean_rel_diag:+.2e}  top-{k} sigma err / sigma_1 {sv_err:.2e}  asym {sym:.1e}", flush=True)
+    ctx.set_option("gram_path", 3)
+    g = _ops.gram(m)
+    t_tc = timed(lambda: _ops.gram(m))
+    err = (g - exact)
+    rel_max = float(err.abs().max() / exact.abs().max())
+    nz = exact.diagonal() > 0
+    rel_diag = float((err.diagonal()[nz].abs() / exact.diagonal()[nz]).max())
+    mean_rel_diag = float((err.diagonal()[nz] / exact.diagonal()[nz]).mean())
+    lam_tc = torch.linalg.eigvalsh(g).flip(0)
+    k = min(64, lam.numel())
+    sv_err = float(((lam_tc[:k].clamp_min(0).sqrt() - lam[:k].clamp_min(0).sqrt()).abs() / lam[0].sqrt()).max())
+    sym = float((g - g.T).abs().max())
+    print(f"  gram {name} {tuple(m.shape)}: tc {t_tc:.3f} ms (dmma {t_dmma:.3f} ms)  max|dG|/max|G| {rel_max:.2e}  "
+          f"diag rel max {rel_diag:.2e} mean {mean_rel_diag:+.2e}  top-{k} sigma err / sigma_1 {sv_err:.2e}  asym {sym:.1e}", flush=True)
     ctx.set_option("gram_path", 0)
     ctx.set_option("tc", 1)
-    ctx.set_option("tc_chunk", 0)
 
 
 def run_gram():
