@@ -15,6 +15,7 @@ pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
 
 from conftest import phantom                              # noqa: E402
+from test_gpu_truncation import SHARDED_CUTOFF_CASE      # noqa: E402
 
 ROOT = Path(__file__).resolve().parents[1]
 
@@ -37,14 +38,20 @@ def _compare(sh, ref_obj, ref_rec, vol, factors, rank, world, tol):
     return rel
 
 
-@pytest.mark.parametrize("shape,chi", [((64, 64, 64), 16), ((32, 48, 40), 12)])
-def test_sharded_world1_equals_plain_sweep(shape, chi):
+@pytest.mark.parametrize("shape,chi,cutoff", [
+    pytest.param((64, 64, 64), 16, 1e-10, id="shape0-16"),
+    pytest.param((32, 48, 40), 12, 1e-10, id="shape1-12"),
+    # an rsum2 cutoff that binds below chi (test_gpu_truncation.py::test_sharded_cutoff_case_is_decidable checks
+    # that no threshold sits within rounding of a compared value)
+    pytest.param(*SHARDED_CUTOFF_CASE, id="shape0-16-cutoff4e-3"),
+])
+def test_sharded_world1_equals_plain_sweep(shape, chi, cutoff):
     from imgcompressionmps.core.ndmps import NDMPS
     from imgcompressionmps.distributed import ShardedNDMPS
     from imgcompressionmps.utils.core import get_factorlist
     x = torch.from_numpy(phantom(shape, seed=3, background=0.01).astype(np.float32)).cuda()
-    ref = NDMPS.from_tensor(x, max_bond=chi)
-    sh = ShardedNDMPS.from_local(x, shape, rank=0, world=1, max_bond=chi, stop_bytes=1 << 16)
+    ref = NDMPS.from_tensor(x, max_bond=chi, cutoff=cutoff)
+    sh = ShardedNDMPS.from_local(x, shape, rank=0, world=1, max_bond=chi, cutoff=cutoff, stop_bytes=1 << 16)
     factors, _ = get_factorlist(shape)
     _compare(sh, ref, ref.to_tensor_device(), x, factors, 0, 1, 1e-6)
     for a, b in zip(sh.cores, ref.mps.cores):
