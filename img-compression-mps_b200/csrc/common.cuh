@@ -246,6 +246,26 @@ int coop_launch(ndmps_ctx* ctx, const void* fn, dim3 grid, dim3 block, void** ar
 int minmax_device(ndmps_ctx* ctx, const void* x, int64_t n, int dtype, double* out_dev2);
 int permute(ndmps_ctx* ctx, const ndmps_plan* plan, bool inverse, const void* src, void* dst, int dtype, double scale);
 
+// Gather by per-axis offset tables (region.cu): for every multi-index (i_0, .., i_{n-1}) in C order over ext,
+//   dst[(multi-index) * row + t] = src[(tab_0[i_0] + .. + tab_{n-1}[i_{n-1}]) * row + t],   t < row.
+// row > 1 moves whole rows (bond vectors), row = 1 single elements.  Tables are device memory.
+#define NDMPS_GATHER_AXES 9            // ndim (<= 8) + the bond axis of a right-chain level
+struct GatherArgs {
+    int n = 0;
+    int64_t ext[NDMPS_GATHER_AXES] = {0};
+    const int64_t* tab[NDMPS_GATHER_AXES] = {nullptr};
+    int64_t row = 1;
+};
+int gather_sum(ndmps_ctx* ctx, const void* src, void* dst, int dtype, const GatherArgs& g);
+// MPS -> dense in two chains and one product (ttsvd.cu), shared by contract_dense and the region / point paths.
+// gathers == nullptr builds the full chains; otherwise gathers[k] keeps the rows (left) / columns (right) of level k.
+int split_site(int L, const int64_t* dims);
+int left_chain(ndmps_ctx* ctx, const void* const* cores, int dtype, int s, const int64_t* dims, const int64_t* ranks,
+               const GatherArgs* gathers, const void** X_out, int64_t* rows_out);
+int right_chain(ndmps_ctx* ctx, const void* const* cores, int dtype, int L, int s, const int64_t* dims, const int64_t* ranks,
+                const GatherArgs* gathers, const void** W_out, int64_t* cols_out);
+int chain_product(ndmps_ctx* ctx, int64_t rows, int64_t cols, int64_t r, const void* X, const void* W, int dtype, void* out);
+
 #ifdef __CUDACC__
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll

@@ -549,54 +549,121 @@ static int compress_bond(ndmps_ctx* ctx, const void* t1, const void* t2, int dty
 // ---------------------------------------------------------------------------------
 // MPS -> dense (cumulative left -> right, Appendix A.3)
 // ---------------------------------------------------------------------------------
-static int contract_dense(ndmps_ctx* ctx, const void* const* cores, int dtype, int L, const int64_t* dims,
-                          const int64_t* ranks, void* dense_out) {
-    // Meet in the middle: X = product of the cores left of a split site s (P_s x r), W = product of
-    // the cores from s on (r x Q_s), dense = X W in ONE large product that writes every voxel once.
-    // Left and right chains are small; total flops ~ 2 N r instead of sum_k 2 P_k r d r.
-    const size_t esz = dtype_size(dtype);
-    if (L == 1) {
-        NDMPS_CUDA_TRY(cudaMemcpyAsync(dense_out, cores[0], (size_t)dims[0] * esz, cudaMemcpyDeviceToDevice, ctx->stream));
-        return NDMPS_OK;
-    }
-    StageScope sc(ctx, ST_CONTRACT);
-    // split site: first s with P_s = prod_{k<s} d_k >= sqrt(N) (balanced), 1 <= s <= L-1
+// Meet in the middle: X = product of the cores left of a split site s (P_s x r), W = product of
+// the cores from s on (r x Q_s), dense = X W in ONE large product that writes every voxel once.
+// Left and right chains are small; total flops ~ 2 N r instead of sum_k 2 P_k r d r.
+// The chains and the product are shared with the region and point paths (region.cu), which pass
+// per-level gathers that keep only the rows / columns a box or a set of points needs.
+
+// split site: first s with P_s = prod_{k<s} d_k >= sqrt(N) (balanced), 1 <= s <= L-1 (L >= 2)
+int split_site(int L, const int64_t* dims) {
     double logn = 0.0;
     for (int k = 0; k < L; k++) logn += log((double)dims[k]);
     int s = 1;
-    {
-        double acc = log((double)dims[0]);
-        while (s < L - 1 && acc < 0.5 * logn) { acc += log((double)dims[s]); s++; }
-    }
-    // left chain: X (rows x ranks[s-1])
+    double acc = log((double)dims[0]);
+    while (s < L - 1 && acc < 0.5 * logn) { acc += log((double)dims[s]); s++; }
+    return s;
+}
+
+static int64_t gather_count(const GatherArgs& g) {
+    int64_t n = 1;
+    for (int a = 0; a < g.n; a++) n *= g.ext[a];
+    return n;
+}
+
+// left chain: X (rows x ranks[s-1]).  gathers[k] (optional): rows of level k kept, in units of ranks[k] elements
+int left_chain(ndmps_ctx* ctx, const void* const* cores, int dtype, int s, const int64_t* dims, const int64_t* ranks,
+               const GatherArgs* gathers, const void** X_out, int64_t* rows_out) {
+    const size_t esz = dtype_size(dtype);
     const void* X = cores[0];
     int64_t rows = dims[0];
+    if (gathers) {
+        void* kept = nullptr;
+        rows = gather_count(gathers[0]);
+        NDMPS_TRY(ctx->ws.alloc((size_t)(rows * ranks[0]) * esz, &kept));
+        NDMPS_TRY(gather_sum(ctx, X, kept, dtype, gathers[0]));
+        X = kept;
+    }
     for (int k = 1; k < s; k++) {
         int64_t rin = ranks[k - 1], rout = ranks[k], ncols = dims[k] * rout;
         void* out = nullptr;
         NDMPS_TRY(ctx->ws.alloc((size_t)(rows * ncols) * esz, &out));
         NDMPS_TRY(gemm(ctx, rows, ncols, rin, 1.0, X, dtype, rin, 1, cores[k], dtype, ncols, 1, out, dtype, ncols));
         X = out;
-        rows *= dims[k];
+        if (gathers) {   // out read as (rows * d_k) x rout: row (parent, digit)
+            void* kept = nullptr;
+            rows = gather_count(gathers[k]);
+            NDMPS_TRY(ctx->ws.alloc((size_t)(rows * rout) * esz, &kept));
+            NDMPS_TRY(gather_sum(ctx, out, kept, dtype, gathers[k]));
+            X = kept;
+        } else {
+            rows *= dims[k];
+        }
     }
-    // right chain: W (ranks[s-1] x cols), built from the last core backwards
+    *X_out = X;
+    *rows_out = rows;
+    return NDMPS_OK;
+}
+
+// right chain: W (ranks[s-1] x cols), built from the last core backwards.  gathers[k] (optional): element gather of
+// level k whose first axis is the left bond ranks[k-1]; the columns kept are its other axes
+int right_chain(ndmps_ctx* ctx, const void* const* cores, int dtype, int L, int s, const int64_t* dims, const int64_t* ranks,
+                const GatherArgs* gathers, const void** W_out, int64_t* cols_out) {
+    const size_t esz = dtype_size(dtype);
     const void* W = cores[L - 1];                 // (r_{L-2} x d_{L-1})
     int64_t cols = dims[L - 1];
+    if (gathers) {
+        void* kept = nullptr;
+        cols = gather_count(gathers[L - 1]) / ranks[L - 2];
+        NDMPS_TRY(ctx->ws.alloc((size_t)(ranks[L - 2] * cols) * esz, &kept));
+        NDMPS_TRY(gather_sum(ctx, W, kept, dtype, gathers[L - 1]));
+        W = kept;
+    }
     for (int k = L - 2; k >= s; k--) {
         int64_t rl = ranks[k - 1], rr = ranks[k];  // core k: (rl, d_k, rr) = (rl*d_k) x rr
         void* out = nullptr;
         NDMPS_TRY(ctx->ws.alloc((size_t)(rl * dims[k] * cols) * esz, &out));
         NDMPS_TRY(gemm(ctx, rl * dims[k], cols, rr, 1.0, cores[k], dtype, rr, 1, W, dtype, cols, 1, out, dtype, cols));
         W = out;
-        cols *= dims[k];
+        if (gathers) {   // out read as rl x (d_k * cols): column (digit, child)
+            void* kept = nullptr;
+            cols = gather_count(gathers[k]) / rl;
+            NDMPS_TRY(ctx->ws.alloc((size_t)(rl * cols) * esz, &kept));
+            NDMPS_TRY(gather_sum(ctx, out, kept, dtype, gathers[k]));
+            W = kept;
+        } else {
+            cols *= dims[k];
+        }
     }
-    const int64_t r = ranks[s - 1];
+    *W_out = W;
+    *cols_out = cols;
+    return NDMPS_OK;
+}
+
+// out (rows x cols) = X (rows x r) W (r x cols)
+int chain_product(ndmps_ctx* ctx, int64_t rows, int64_t cols, int64_t r, const void* X, const void* W, int dtype, void* out) {
     if (ctx->opt_tc && dtype == NDMPS_F32 && rows * cols >= (int64_t(1) << 20)) {   // float32 payload: the one big product on tcgen05
         bool on_tc = false;
-        NDMPS_TRY(gemm_tc(ctx, rows, cols, r, 1.0, X, dtype, r, 1, W, dtype, cols, 1, dense_out, dtype, cols, false, &on_tc));
+        NDMPS_TRY(gemm_tc(ctx, rows, cols, r, 1.0, X, dtype, r, 1, W, dtype, cols, 1, out, dtype, cols, false, &on_tc));
         if (on_tc) return NDMPS_OK;
     }
-    return gemm(ctx, rows, cols, r, 1.0, X, dtype, r, 1, W, dtype, cols, 1, dense_out, dtype, cols);
+    return gemm(ctx, rows, cols, r, 1.0, X, dtype, r, 1, W, dtype, cols, 1, out, dtype, cols);
+}
+
+static int contract_dense(ndmps_ctx* ctx, const void* const* cores, int dtype, int L, const int64_t* dims,
+                          const int64_t* ranks, void* dense_out) {
+    const size_t esz = dtype_size(dtype);
+    if (L == 1) {
+        NDMPS_CUDA_TRY(cudaMemcpyAsync(dense_out, cores[0], (size_t)dims[0] * esz, cudaMemcpyDeviceToDevice, ctx->stream));
+        return NDMPS_OK;
+    }
+    StageScope sc(ctx, ST_CONTRACT);
+    const int s = split_site(L, dims);
+    const void *X = nullptr, *W = nullptr;
+    int64_t rows = 0, cols = 0;
+    NDMPS_TRY(left_chain(ctx, cores, dtype, s, dims, ranks, nullptr, &X, &rows));
+    NDMPS_TRY(right_chain(ctx, cores, dtype, L, s, dims, ranks, nullptr, &W, &cols));
+    return chain_product(ctx, rows, cols, ranks[s - 1], X, W, dtype, dense_out);
 }
 
 // ---------------------------------------------------------------------------------

@@ -67,6 +67,9 @@ PROTOTYPES = {
     "ndmps_ttsvd": (ci, [vp, vp, ci, ci, p_i64, f64, ci, i64, ci, p_vp, p_i64, p_i64, p_f64, i64]),
     "ndmps_compress_bond": (ci, [vp, vp, vp, ci, i64, i64, i64, f64, ci, i64, ci, vp, vp, p_i64, p_f64]),
     "ndmps_contract_dense": (ci, [vp, p_vp, ci, ci, p_i64, p_i64, vp]),
+    "ndmps_contract_region": (ci, [vp, vp, p_vp, ci, p_i64, p_i64, p_i64, vp]),
+    "ndmps_evaluate_points": (ci, [vp, vp, p_vp, ci, p_i64, vp, i64, ci, vp]),
+    "ndmps_region_debug_offsets": (ci, [vp, p_i64, p_i64, p_i64, p_i64]),
     "ndmps_overlap": (ci, [vp, p_vp, p_i64, ci, p_vp, p_i64, ci, ci, p_i64, p_f64]),
     "ndmps_quantize": (ci, [vp, vp, i64, ci, f64, f64, ci, vp]),
     "ndmps_dequantize": (ci, [vp, vp, i64, ci, f64, f64, ci, vp]),
@@ -231,6 +234,15 @@ class Plan:
         check(self.lib.ndmps_plan_debug_offsets(self.handle, int(bool(inverse)), int(first), int(count),
                                                 out.ctypes.data_as(p_i64)), "ndmps_plan_debug_offsets")
         return out
+
+    def region_debug(self, lo, hi):
+        """(dict(s, rows, cols), flat site-order index per voxel of the box [lo, hi)) as the region path computes it."""
+        count = int(np.prod([int(h) - int(l) for l, h in zip(lo, hi)], dtype=np.int64)) if len(lo) else 0
+        out = np.empty(max(count, 0), dtype=np.int64)
+        info = (C.c_int64 * 3)()
+        check(self.lib.ndmps_region_debug_offsets(self.handle, i64_array(lo), i64_array(hi), info,
+                                                  out.ctypes.data_as(p_i64)), "ndmps_region_debug_offsets")
+        return dict(zip(("s", "rows", "cols"), (int(v) for v in info))), out
 
     def tile_info(self, inverse: bool) -> dict:
         out = (C.c_int64 * 6)()

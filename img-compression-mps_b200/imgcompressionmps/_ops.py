@@ -333,6 +333,81 @@ def contract_dense(cores):
     return out
 
 
+def region_box(shape, index):
+    """numpy basic indexing with step 1 -> (lo, hi, result shape) of the box it selects in a volume of ``shape``.
+
+    ``index``: an int, a slice, ``Ellipsis`` or a tuple of them, with at most one ``Ellipsis`` and at most ``ndim``
+    entries (missing trailing entries select whole axes).  Ints drop their axis and may be negative; slice bounds
+    are clipped as numpy clips them.  Errors have numpy's types: ``IndexError`` for an int out of range, too many
+    indices, a second ``Ellipsis`` or an index of another type, ``TypeError`` for a slice bound that is not an
+    integer.  A slice step other than 1 (or None), ``None`` (new axis), booleans and arrays are not supported here
+    and raise ``ValueError``."""
+    import operator
+    shape = tuple(int(s) for s in shape)
+    ndim = len(shape)
+    items = index if isinstance(index, tuple) else (index,)
+    for it in items:
+        if it is None or isinstance(it, (bool, np.bool_, np.ndarray, list)):
+            raise ValueError(f"region index: {it!r} is not supported (ints, step-1 slices and Ellipsis only)")
+        if not (it is Ellipsis or isinstance(it, slice) or hasattr(it, "__index__")):
+            raise IndexError("only integers, slices (`:`) and ellipsis (`...`) are valid region indices")
+    n_ell = sum(1 for it in items if it is Ellipsis)
+    if n_ell > 1:
+        raise IndexError("an index can only have a single ellipsis ('...')")
+    if len(items) - n_ell > ndim:
+        raise IndexError(f"too many indices: the volume is {ndim}-dimensional, but {len(items) - n_ell} were indexed")
+    if n_ell:
+        at = items.index(Ellipsis)
+        items = items[:at] + (slice(None),) * (ndim - len(items) + 1) + items[at + 1:]
+    items = items + (slice(None),) * (ndim - len(items))
+    lo, hi, out_shape = [], [], []
+    for axis, (it, n) in enumerate(zip(items, shape)):
+        if isinstance(it, slice):
+            if it.step is not None and operator.index(it.step) != 1:
+                raise ValueError(f"region index: slice step {it.step} on axis {axis} (only step 1 is supported)")
+            start, stop, _ = slice(it.start, it.stop).indices(n)
+            stop = max(stop, start)
+            lo.append(start)
+            hi.append(stop)
+            out_shape.append(stop - start)
+        else:
+            i = operator.index(it)
+            if not -n <= i < n:
+                raise IndexError(f"index {i} is out of bounds for axis {axis} with size {n}")
+            i += n if i < 0 else 0
+            lo.append(i)
+            hi.append(i + 1)
+    return lo, hi, tuple(out_shape)
+
+
+def contract_region(cores, shape, lo, hi):
+    """Box [lo, hi) of the volume of ``shape`` that the cores encode, as a device tensor of shape hi - lo."""
+    torch = _torch()
+    cores = [_dev(c, "core") for c in cores]
+    plan = plan_for(tuple(shape))
+    out = torch.empty([int(h) - int(l) for l, h in zip(lo, hi)], dtype=cores[0].dtype, device=cores[0].device)
+    N.check(N.load_library().ndmps_contract_region(N.handle(), plan.handle, N.ptr_array(cores), N.dtype_code(cores[0].dtype),
+                                                   N.i64_array(_ranks_of(cores)), N.i64_array(lo), N.i64_array(hi),
+                                                   N.ptr(out)), "ndmps_contract_region")
+    return out
+
+
+def evaluate_points(cores, shape, coords, idct_last_axis: bool = False):
+    """Values of the volume of ``shape`` at ``coords`` (int64 device tensor, K x ndim), as a device tensor of K values."""
+    torch = _torch()
+    cores = [_dev(c, "core") for c in cores]
+    _dev(coords, "coords")
+    if coords.dtype != torch.int64 or coords.ndim != 2 or coords.shape[1] != len(shape):
+        raise ValueError("evaluate_points: coords must be an int64 (K, ndim) tensor")
+    plan = plan_for(tuple(shape))
+    count = int(coords.shape[0])
+    out = torch.empty(count, dtype=cores[0].dtype, device=cores[0].device)
+    N.check(N.load_library().ndmps_evaluate_points(N.handle(), plan.handle, N.ptr_array(cores), N.dtype_code(cores[0].dtype),
+                                                   N.i64_array(_ranks_of(cores)), N.ptr(coords), count,
+                                                   int(bool(idct_last_axis)), N.ptr(out)), "ndmps_evaluate_points")
+    return out
+
+
 def overlap(cores_a, cores_b) -> float:
     cores_a = [_dev(c, "core") for c in cores_a]
     cores_b = [_dev(c, "core") for c in cores_b]

@@ -175,6 +175,74 @@ class NDMPS:
         rec = self.to_tensor_device()
         return None if rec is None else rec.cpu().numpy()
 
+    # ------------------------------------------------------------------ partial reconstruction (extension)
+    def to_tensor_region_device(self, index):
+        """``to_tensor_device()[index]`` for basic indexing with step 1 (ints, slices, ``...``; see
+        ``_ops.region_box`` for the rules and errors), computed without the whole tensor: only the core slices the
+        box touches are contracted, and the workspace is a small multiple of the box.  In "DCT" mode the inverse DCT
+        runs along the whole last axis, so the box is decoded over the full last axis first and cropped after: that
+        costs (last extent / box's last extent) times the memory and work of the box itself.  Any other mode returns
+        None, as ``to_tensor`` does."""
+        torch = _torch()
+        lo, hi, out_shape = _ops.region_box(self._shape, index)
+        if self.mode not in ("Std", "DCT"):
+            return None
+        cores = self.mps.cores
+        if any(h == l for l, h in zip(lo, hi)):
+            return torch.empty(out_shape, dtype=cores[0].dtype, device=cores[0].device)
+        if self.mode == "Std":
+            return _ops.contract_region(cores, self._shape, lo, hi).view(out_shape)
+        n = self._shape[-1]
+        wide = _ops.contract_region(cores, self._shape, lo[:-1] + [0], hi[:-1] + [n])
+        rec = _ops.dct_last_axis(wide, inverse=True)
+        del wide
+        return rec[..., lo[-1]:hi[-1]].contiguous().view(out_shape)
+
+    def to_tensor_region(self, index):
+        """``to_tensor()[index]`` as a numpy array, without reconstructing the whole tensor (see
+        ``to_tensor_region_device``); None for a mode other than "Std" / "DCT"."""
+        rec = self.to_tensor_region_device(index)
+        return None if rec is None else rec.cpu().numpy()
+
+    def values_at(self, coords):
+        """``to_tensor()[tuple(coords.T)]``: the values at K points, without reconstructing the whole tensor.
+
+        ``coords``: integer array of shape (K, ndim), numpy (result: numpy array) or a CUDA tensor (result: CUDA
+        tensor); negative coordinates count from the end, duplicates and K = 0 are allowed.  A coordinate outside
+        [-extent, extent) raises ``IndexError``, a wrong shape ``ValueError``, a non-integer array ``IndexError``
+        (numpy's errors for the same indexing).  Each point costs one bond-length dot product on the device; in "DCT"
+        mode it costs one per element of its last-axis line (the inverse DCT of that line evaluated at the point).
+        Any other mode returns None."""
+        torch = _torch()
+        ndim = len(self._shape)
+        on_device = isinstance(coords, torch.Tensor)
+        if on_device and not coords.is_cuda:
+            raise ValueError("values_at: coords must be a numpy array or a CUDA tensor")
+        if not on_device:
+            coords = np.asarray(coords)
+        if coords.ndim != 2 or int(coords.shape[1]) != ndim:
+            raise ValueError(f"values_at: coords must have shape (K, {ndim}), got {tuple(coords.shape)}")
+        integer = (not coords.dtype.is_floating_point and not coords.dtype.is_complex and coords.dtype != torch.bool
+                   if on_device else np.issubdtype(coords.dtype, np.integer))
+        if not integer:
+            raise IndexError(f"values_at: coordinates must be integers, got {coords.dtype}")
+        if on_device:
+            coords = coords.to(torch.int64).contiguous()
+            extent = torch.tensor(self._shape, dtype=torch.int64, device=coords.device)
+            outside = bool(((coords < -extent) | (coords >= extent)).any().item()) if coords.numel() else False
+        else:
+            coords = np.ascontiguousarray(coords, dtype=np.int64)
+            extent = np.array(self._shape, dtype=np.int64)
+            outside = bool(((coords < -extent) | (coords >= extent)).any())
+        if outside:
+            raise IndexError(f"values_at: a coordinate is out of bounds for shape {self._shape}")
+        if self.mode not in ("Std", "DCT"):
+            return None
+        cores = self.mps.cores
+        dev = coords if on_device else torch.from_numpy(coords).to(cores[0].device)
+        out = _ops.evaluate_points(cores, self._shape, dev, idct_last_axis=self.mode == "DCT")
+        return out if on_device else out.cpu().numpy()
+
     # ------------------------------------------------------------------ core access
     def replace_tensordata(self, tensorlist):
         """Shape-asserting in-place overwrite of every core (``core/ndmps.py:163-175``)."""

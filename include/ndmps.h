@@ -213,6 +213,31 @@ int ndmps_compress_bond(ndmps_ctx_t* ctx, const void* t1, const void* t2, int dt
 int ndmps_contract_dense(ndmps_ctx_t* ctx, const void* const* cores, int dtype, int levels,
                          const int64_t* dims, const int64_t* ranks, void* dense_out);
 
+/* ---- K7b: part of the MPS -> volume, without the whole tensor ----------------
+ * An extension beyond the reference: to_tensor()[box] and to_tensor()[points] at core/ndmps.py:131-153 without
+ * the N-element reconstruction.  `plan` is the volume's (ndmps_plan_create); cores / ranks as for
+ * ndmps_contract_dense with levels = the plan's levels.
+ * ndmps_contract_region: out = the box [lo, hi) (ndim values each) of the volume, in volume axis order,
+ * C-contiguous, written on the context's stream without a host synchronisation.  The workspace is bounded by a
+ * small multiple of the box (at most 3^ndim times it) plus the two chains restricted to the digits the box
+ * touches.  A box outside the volume returns NDMPS_ERR_INVALID; an empty box is a no-op (out may then be NULL). */
+int ndmps_contract_region(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void* const* cores, int dtype,
+                          const int64_t* ranks, const int64_t* lo, const int64_t* hi, void* out);
+/* out_dev[i] = volume[coords_dev[i, :]] for `count` points; coords_dev: int64 device array (count x ndim),
+ * negative coordinates count from the end as in numpy.  idct_last_axis = 1: the cores hold the DCT-II of the
+ * volume along its last axis (mode "DCT"), the value is the orthonormal inverse DCT of that line evaluated at
+ * the point (n = last extent dot products per point instead of 1).  A coordinate outside [-extent, extent) gives NaN;
+ * no core is ever read outside its bounds.  No host synchronisation. */
+int ndmps_evaluate_points(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void* const* cores, int dtype,
+                          const int64_t* ranks, const int64_t* coords_dev, int64_t count, int idct_last_axis,
+                          void* out_dev);
+/* host-only index check of ndmps_contract_region (no device work): info_out[3] = {split site s, |H| kept rows,
+ * |C| kept columns}; site_offsets_out_host (one value per box voxel, C order) = the flat site-order index
+ * (row * Q_s + column) the region path reads for the voxel, mapped back from its compact row and column sets.
+ * An empty box writes {s, 0, 0} and no offsets. */
+int ndmps_region_debug_offsets(const ndmps_plan_t* plan, const int64_t* lo, const int64_t* hi, int64_t* info_out,
+                               int64_t* site_offsets_out_host);
+
 /* ---- K8: <a|b> --------------------------------------------------------------
  * `mps @ mps` at core/ndmps.py:76,86 and utils/metrics.py:160 (no conjugation). */
 int ndmps_overlap(ndmps_ctx_t* ctx, const void* const* cores_a, const int64_t* ranks_a, int dtype_a,
