@@ -23,6 +23,19 @@ __global__ void __launch_bounds__(256) dct_matrix_kernel(double* __restrict__ C,
     }
 }
 
+// B[k][j] = (1/block) sum_{t in block j} C[k][t] (n x n/block): the DCT-III matrix averaged over column blocks, so that
+// y B is the block mean of the inverse transform y C
+__global__ void __launch_bounds__(256) dct_block_mean_matrix_kernel(double* __restrict__ B, int64_t n, int64_t block) {
+    const int64_t m = n / block, total = n * m, stride = (int64_t)gridDim.x * blockDim.x;
+    const double scale = sqrt(2.0 / (double)n) / (double)block;
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += stride) {
+        const int64_t k = e / m, j = e - k * m;
+        double s = 0.0;
+        for (int64_t t = j * block; t < (j + 1) * block; t++) s += cospi((double)(((2 * t + 1) * k) % (4 * n)) / (double)(2 * n));
+        B[e] = (k == 0 ? 0.70710678118654752440 : 1.0) * scale * s;
+    }
+}
+
 }  // namespace ndmps
 
 using namespace ndmps;
@@ -52,6 +65,29 @@ int ndmps_dct_last_axis(ndmps_ctx_t* ctx, const void* src, void* dst, int64_t li
         return gemm(ctx, lines, n, n, 1.0, src, dtype, n, 1, C, NDMPS_F64, n, 1, dst, dtype, n);
     // x[l, i] = sum_k y[l, k] C[k, i]
     return gemm(ctx, lines, n, n, 1.0, src, dtype, n, 1, C, NDMPS_F64, n, 1, dst, dtype, n);
+}
+
+int ndmps_idct_block_mean_last_axis(ndmps_ctx_t* ctx, const void* src, void* dst, int64_t lines, int64_t n, int64_t block, int dtype) {
+    NDMPS_REQUIRE(ctx && src && dst, "ndmps_idct_block_mean_last_axis: NULL argument");
+    NDMPS_REQUIRE(dtype_ok(dtype) && lines >= 0 && n >= 1, "ndmps_idct_block_mean_last_axis: bad shape or dtype");
+    NDMPS_REQUIRE(block >= 1 && n % block == 0, "ndmps_idct_block_mean_last_axis: block %lld does not divide n = %lld",
+                  (long long)block, (long long)n);
+    NDMPS_REQUIRE(src != dst, "ndmps_idct_block_mean_last_axis: in-place transform is not supported");
+    if (lines == 0) return NDMPS_OK;
+    NDMPS_TRY(ctx->ws.reset(ctx->stream));
+    StageScope sc(ctx, ST_DCT);
+    const int64_t m = n / block;
+    double* B = nullptr;
+    NDMPS_TRY(ctx->ws.get<double>((size_t)(n * m), &B));
+    int64_t want = (n * m + 255) / 256, cap = (int64_t)ctx->sm_count * 8;
+    dct_block_mean_matrix_kernel<<<(int)(want < cap ? want : cap), 256, 0, ctx->stream>>>(B, n, block);
+    NDMPS_LAUNCH_CHECK(ctx);
+    if (ctx->opt_tc && dtype == NDMPS_F32 && lines * n >= (int64_t(1) << 20)) {   // same rule as ndmps_dct_last_axis
+        bool on_tc = false;
+        NDMPS_TRY(gemm_tc(ctx, lines, m, n, 1.0, src, dtype, n, 1, B, NDMPS_F64, m, 1, dst, dtype, m, false, &on_tc));
+        if (on_tc) return NDMPS_OK;
+    }
+    return gemm(ctx, lines, m, n, 1.0, src, dtype, n, 1, B, NDMPS_F64, m, 1, dst, dtype, m);
 }
 
 }  // extern "C"

@@ -46,6 +46,8 @@ PROTOTYPES = {
     "ndmps_plan_create": (ci, [ci, p_i64, ci, p_i64, p_vp]),
     "ndmps_plan_destroy": (ci, [vp]),
     "ndmps_plan_site_dims": (ci, [vp, p_i64]),
+    "ndmps_plan_layout": (ci, [vp, C.POINTER(ci), C.POINTER(ci), p_i64, p_i64]),
+    "ndmps_plan_coarse": (ci, [vp, p_i64, p_vp]),
     "ndmps_plan_debug_offsets": (ci, [vp, ci, i64, i64, p_i64]),
     "ndmps_plan_debug_tile_info": (ci, [vp, ci, p_i64]),
     "ndmps_plan_debug_apply_tiled": (ci, [vp, ci, vp, vp]),
@@ -57,6 +59,7 @@ PROTOTYPES = {
     "ndmps_minmax": (ci, [vp, p_vp, p_i64, ci, ci, p_f64]),
     "ndmps_psnr_terms": (ci, [vp, vp, vp, i64, ci, p_f64]),
     "ndmps_dct_last_axis": (ci, [vp, vp, vp, i64, i64, ci, ci]),
+    "ndmps_idct_block_mean_last_axis": (ci, [vp, vp, vp, i64, i64, i64, ci]),
     "ndmps_gram": (ci, [vp, vp, i64, i64, i64, ci, ci, vp]),
     "ndmps_eigh": (ci, [vp, vp, i64, vp, vp, C.POINTER(ci)]),
     "ndmps_eigh_topk": (ci, [vp, vp, i64, i64, vp, vp]),
@@ -70,6 +73,7 @@ PROTOTYPES = {
     "ndmps_contract_region": (ci, [vp, vp, p_vp, ci, p_i64, p_i64, p_i64, vp]),
     "ndmps_evaluate_points": (ci, [vp, vp, p_vp, ci, p_i64, vp, i64, ci, vp]),
     "ndmps_region_debug_offsets": (ci, [vp, p_i64, p_i64, p_i64, p_i64]),
+    "ndmps_marginalize": (ci, [vp, vp, p_vp, ci, p_i64, p_i64, p_vp, p_i64]),
     "ndmps_overlap": (ci, [vp, p_vp, p_i64, ci, p_vp, p_i64, ci, ci, p_i64, p_f64]),
     "ndmps_quantize": (ci, [vp, vp, i64, ci, f64, f64, ci, vp]),
     "ndmps_dequantize": (ci, [vp, vp, i64, ci, f64, f64, ci, vp]),
@@ -223,11 +227,34 @@ class Plan:
         h = vp()
         check(self.lib.ndmps_plan_create(ndim, i64_array(self.shape), int(self.levels),
                                          factors.ctypes.data_as(p_i64), C.byref(h)), "ndmps_plan_create")
+        self._adopt(h, factors)
+
+    def _adopt(self, h, factors):
         self.handle = h
+        self.factors = factors
         dims = (C.c_int64 * self.levels)()
         check(self.lib.ndmps_plan_site_dims(h, dims), "ndmps_plan_site_dims")
         self.site_dims = [int(d) for d in dims]
         self.total = int(np.prod(self.shape, dtype=np.int64)) if len(self.shape) else 0
+
+    def coarse(self, drop_levels) -> "Plan":
+        """Plan of the block-mean tensor that averages the finest ``drop_levels[a]`` digits of axis a
+        (``ndmps_plan_coarse`` decides its shape and factor table; this only reads them back)."""
+        h = vp()
+        check(self.lib.ndmps_plan_coarse(self.handle, i64_array(drop_levels), C.byref(h)), "ndmps_plan_coarse")
+        out = Plan.__new__(Plan)
+        out.lib = self.lib
+        out.handle = h                                   # freed by __del__ even if a read below fails
+        ndim, levels = C.c_int(), C.c_int()
+        check(self.lib.ndmps_plan_layout(h, C.byref(ndim), C.byref(levels), None, None), "ndmps_plan_layout")
+        shape = np.empty(ndim.value, dtype=np.int64)
+        factors = np.empty((levels.value, ndim.value), dtype=np.int64)
+        check(self.lib.ndmps_plan_layout(h, C.byref(ndim), C.byref(levels), shape.ctypes.data_as(p_i64),
+                                         factors.ctypes.data_as(p_i64)), "ndmps_plan_layout")
+        out.shape = tuple(int(s) for s in shape)
+        out.levels = levels.value
+        out._adopt(h, factors)
+        return out
 
     def debug_offsets(self, inverse: bool, first: int, count: int) -> np.ndarray:
         out = np.empty(count, dtype=np.int64)

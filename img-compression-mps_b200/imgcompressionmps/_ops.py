@@ -34,6 +34,42 @@ def plan_for(shape) -> N.Plan:
     return N.Plan(shape, factors)
 
 
+def coarse_levels(shape, levels) -> tuple:
+    """Validated per-axis digit counts of a block mean: ``levels`` is an int (every axis) or a sequence of ``ndim``
+    ints, each in ``0 ..= L`` (L = the levels of ``get_factorlist(shape)``); numpy integers are accepted.  A bool or a
+    non-integer raises ``TypeError``, a wrong length or a value out of range ``ValueError``."""
+    import operator
+    shape = tuple(int(s) for s in shape)
+    L = int(get_factorlist(shape)[0].shape[0])
+
+    def one(v):
+        if isinstance(v, (bool, np.bool_)) or not hasattr(v, "__index__"):
+            raise TypeError(f"levels: {v!r} is not an integer")
+        return operator.index(v)
+
+    if isinstance(levels, (list, tuple, np.ndarray)):
+        ks = tuple(one(v) for v in levels)
+        if len(ks) != len(shape):
+            raise ValueError(f"levels: {len(ks)} values for a {len(shape)}-dimensional volume")
+    else:
+        ks = (one(levels),) * len(shape)
+    if any(not 0 <= k <= L for k in ks):
+        raise ValueError(f"levels: {ks} outside 0..{L} (the volume has {L} levels)")
+    return ks
+
+
+@lru_cache(maxsize=64)
+def _coarse_plan(shape, ks) -> N.Plan:
+    return plan_for(shape).coarse(ks)
+
+
+def coarse_plan(shape, levels) -> N.Plan:
+    """Plan of the block mean of a volume of ``shape`` over the finest ``levels`` digits of each axis
+    (``ndmps_plan_coarse``; its ``shape`` is the coarse shape)."""
+    shape = tuple(int(s) for s in shape)
+    return _coarse_plan(shape, coarse_levels(shape, levels))
+
+
 # ---- K1 ---------------------------------------------------------------------------
 def encode(volume, scale: float = 1.0, plan=None):
     """volume (original shape, device) -> dense array shaped by the site dims."""
@@ -96,6 +132,18 @@ def dct_last_axis(x, inverse: bool = False):
     out = torch.empty_like(x)
     N.check(N.load_library().ndmps_dct_last_axis(N.handle(), N.ptr(x), N.ptr(out), x.numel() // n, n,
                                                  int(bool(inverse)), N.dtype_code(x.dtype)), "ndmps_dct_last_axis")
+    return out
+
+
+def idct_block_mean_last_axis(x, block: int):
+    """Block mean (``block`` elements) of the orthonormal inverse DCT along the last axis, without the full lines."""
+    torch = _torch()
+    _dev(x)
+    n = int(x.shape[-1])
+    block = int(block)
+    out = torch.empty(tuple(x.shape[:-1]) + (n // block if block >= 1 else 0,), dtype=x.dtype, device=x.device)
+    N.check(N.load_library().ndmps_idct_block_mean_last_axis(N.handle(), N.ptr(x), N.ptr(out), x.numel() // n, n, block,
+                                                             N.dtype_code(x.dtype)), "ndmps_idct_block_mean_last_axis")
     return out
 
 
@@ -380,15 +428,33 @@ def region_box(shape, index):
     return lo, hi, tuple(out_shape)
 
 
-def contract_region(cores, shape, lo, hi):
+def contract_region(cores, shape, lo, hi, plan=None):
     """Box [lo, hi) of the volume of ``shape`` that the cores encode, as a device tensor of shape hi - lo."""
     torch = _torch()
     cores = [_dev(c, "core") for c in cores]
-    plan = plan_for(tuple(shape))
+    plan = plan or plan_for(tuple(shape))
     out = torch.empty([int(h) - int(l) for l, h in zip(lo, hi)], dtype=cores[0].dtype, device=cores[0].device)
     N.check(N.load_library().ndmps_contract_region(N.handle(), plan.handle, N.ptr_array(cores), N.dtype_code(cores[0].dtype),
                                                    N.i64_array(_ranks_of(cores)), N.i64_array(lo), N.i64_array(hi),
                                                    N.ptr(out)), "ndmps_contract_region")
+    return out
+
+
+def marginalize(cores, shape, levels):
+    """Cores of the block mean of the volume of ``shape`` that ``cores`` encode, averaged over the finest ``levels``
+    digits of each axis, in the layout of ``coarse_plan(shape, levels)``."""
+    torch = _torch()
+    cores = [_dev(c, "core") for c in cores]
+    shape = tuple(int(s) for s in shape)
+    ks = coarse_levels(shape, levels)
+    cplan = coarse_plan(shape, ks)
+    ranks = _ranks_of(cores)[:cplan.levels - 1]
+    shapes = [core_shape(i, cplan.levels, cplan.site_dims, ranks) for i in range(cplan.levels)]
+    out = [torch.empty(s, dtype=cores[0].dtype, device=cores[0].device) for s in shapes]
+    N.check(N.load_library().ndmps_marginalize(N.handle(), plan_for(shape).handle, N.ptr_array(cores),
+                                               N.dtype_code(cores[0].dtype), N.i64_array(_ranks_of(cores)),
+                                               N.i64_array(ks), N.ptr_array(out), N.i64_array([o.numel() for o in out])),
+            "ndmps_marginalize")
     return out
 
 

@@ -243,6 +243,55 @@ class NDMPS:
         out = _ops.evaluate_points(cores, self._shape, dev, idct_last_axis=self.mode == "DCT")
         return out if on_device else out.cpu().numpy()
 
+    # ------------------------------------------------------------------ block-mean reconstruction (extension)
+    def coarse_shape(self, levels) -> tuple:
+        """Shape of ``to_tensor_coarse(levels)`` with no index: axis a averaged over its finest ``k_a`` digits, i.e.
+        over blocks of ``b_a`` = the product of the axis' factors (``get_factorlist``) at the finest ``k_a`` levels.
+        ``levels``: an int (every axis) or ``ndim`` ints, each in ``0 ..= L``; see ``_ops.coarse_levels`` for the
+        errors.  Host only."""
+        return _ops.coarse_plan(self._shape, levels).shape
+
+    def to_tensor_coarse_device(self, levels, index=None):
+        """``block_mean(to_tensor_device(), b)[index]``, the mean over non-overlapping blocks of ``b_a`` voxels along
+        each axis (``coarse_shape`` gives the result's shape with no index), computed from the cores without the
+        full-resolution tensor: each finest core is averaged over its digits and the trailing fully averaged sites
+        fold into a boundary vector, then the reduced MPS is decoded like ``to_tensor`` (or like
+        ``to_tensor_region`` for an ``index``, whose rules are ``_ops.region_box``'s, on the coarse shape).  In "DCT"
+        mode every axis but the last is averaged in the cores and the last one through a block-averaged inverse DCT
+        of its full lines.  Any other mode returns None after the arguments are checked."""
+        torch = _torch()
+        ks = _ops.coarse_levels(self._shape, levels)
+        cplan = _ops.coarse_plan(self._shape, ks)
+        cshape = cplan.shape
+        lo, hi, out_shape = _ops.region_box(cshape, () if index is None else index)
+        if self.mode not in ("Std", "DCT"):
+            return None
+        cores = self.mps.cores
+        if any(h == l for l, h in zip(lo, hi)):
+            return torch.empty(out_shape, dtype=cores[0].dtype, device=cores[0].device)
+        if self.mode == "Std":
+            red = _ops.marginalize(cores, self._shape, ks)
+            if lo == [0] * len(cshape) and hi == list(cshape):
+                return _ops.decode(_ops.contract_dense(red), cshape, plan=cplan).view(out_shape)
+            return _ops.contract_region(red, cshape, lo, hi, plan=cplan).view(out_shape)
+        dks = ks[:-1] + (0,)                     # the last axis holds DCT coefficients: averaged after the inverse
+        dplan = _ops.coarse_plan(self._shape, dks)
+        red = _ops.marginalize(cores, self._shape, dks)
+        n = self._shape[-1]
+        if lo[:-1] == [0] * (len(cshape) - 1) and hi[:-1] == list(cshape[:-1]):
+            wide = _ops.decode(_ops.contract_dense(red), dplan.shape, plan=dplan)
+        else:
+            wide = _ops.contract_region(red, dplan.shape, lo[:-1] + [0], hi[:-1] + [n], plan=dplan)
+        del red
+        rec = _ops.idct_block_mean_last_axis(wide, n // cshape[-1])
+        del wide
+        return rec[..., lo[-1]:hi[-1]].contiguous().view(out_shape)
+
+    def to_tensor_coarse(self, levels, index=None):
+        """``to_tensor_coarse_device(levels, index)`` as a numpy array; None for a mode other than "Std" / "DCT"."""
+        rec = self.to_tensor_coarse_device(levels, index)
+        return None if rec is None else rec.cpu().numpy()
+
     # ------------------------------------------------------------------ core access
     def replace_tensordata(self, tensorlist):
         """Shape-asserting in-place overwrite of every core (``core/ndmps.py:163-175``)."""

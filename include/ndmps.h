@@ -104,6 +104,9 @@ int ndmps_plan_create(int ndim, const int64_t* shape, int levels, const int64_t*
                       ndmps_plan_t** out);
 int ndmps_plan_destroy(ndmps_plan_t* plan);
 int ndmps_plan_site_dims(const ndmps_plan_t* plan, int64_t* dims_out);
+/* ndim, levels, shape (ndim values) and factor table (levels x ndim, row-major) of a plan; shape_out and factors_out
+ * may be NULL, so a caller can read ndim and levels first (plans from ndmps_plan_coarse). */
+int ndmps_plan_layout(const ndmps_plan_t* plan, int* ndim_out, int* levels_out, int64_t* shape_out, int64_t* factors_out);
 /* host-only index check (no device work): source offsets the kernels read for
  * destination elements [first, first+count); inverse=0 encode, 1 decode. */
 int ndmps_plan_debug_offsets(const ndmps_plan_t* plan, int inverse, int64_t first, int64_t count, int64_t* out_host);
@@ -135,6 +138,12 @@ int ndmps_psnr_terms(ndmps_ctx_t* ctx, const void* a, const void* b, int64_t n, 
 /* ---- K11: orthonormal DCT-II / DCT-III along the last axis ----------------
  * scipy.fftpack.dct(x, norm="ortho") / idct at core/ndmps.py:63,153. */
 int ndmps_dct_last_axis(ndmps_ctx_t* ctx, const void* src, void* dst, int64_t lines, int64_t n, int inverse, int dtype);
+/* Block mean of the inverse transform, without the n-element lines: dst (lines x n/block) = src (lines x n) . B with
+ * B[k, j] = (1/block) sum_{t in block j} C[k, t], C the orthonormal DCT-III matrix (built on the device in float64).
+ * tcgen05 (bf16x3) for float32 when lines * n >= 2^20, as ndmps_dct_last_axis.  block must be >= 1 and divide n,
+ * otherwise NDMPS_ERR_INVALID.  block = 1 is ndmps_dct_last_axis(inverse = 1). */
+int ndmps_idct_block_mean_last_axis(ndmps_ctx_t* ctx, const void* src, void* dst, int64_t lines, int64_t n, int64_t block,
+                                    int dtype);
 
 /* ---- building blocks of the sweep (exported for tests and profiling) ------ */
 /* G (float64, device) = M M^T (side 0, rows x rows) or M^T M (side 1, cols x cols);
@@ -237,6 +246,25 @@ int ndmps_evaluate_points(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void
  * An empty box writes {s, 0, 0} and no offsets. */
 int ndmps_region_debug_offsets(const ndmps_plan_t* plan, const int64_t* lo, const int64_t* hi, int64_t* info_out,
                                int64_t* site_offsets_out_host);
+
+/* ---- K7c: block-mean (coarse) MPS, without the whole tensor -------------------
+ * An extension beyond the reference: the mean of to_tensor() over non-overlapping blocks, from the cores.
+ * drop_levels (ndim values, 0 <= k_a <= levels): axis a is averaged over its finest k_a digits, i.e. over blocks of
+ * b_a = prod_{l >= levels - k_a} factors[l, a] voxels.
+ * ndmps_plan_coarse (host only): *out = the plan of the block-mean tensor, shape[a] / b_a, with factors[l, a] = 1
+ * wherever the digit is averaged and the trailing levels averaged on every axis removed (at least one level stays).
+ * The result is an ordinary plan (ndmps_plan_layout reads it, ndmps_plan_destroy frees it).  This is the one place
+ * that decides the coarse site layout. */
+int ndmps_plan_coarse(const ndmps_plan_t* plan, const int64_t* drop_levels, ndmps_plan_t** out);
+/* cores_out[i] (i < the coarse plan's levels, core_cap[i] elements each): the cores of the block-mean tensor in the
+ * layout of ndmps_plan_coarse; cores / ranks as for ndmps_contract_region.  A partly averaged site maps (r, d, r') to
+ * (r, d', r'), the mean over the averaged digits of the fused site index (float64 sums, stored in the payload dtype);
+ * the removed sites fold, in float64, into one right boundary vector that the last kept core absorbs.  Output ranks:
+ * the kept bonds (ranks[0 .. levels'-2]); the last kept core has no right bond.  On the context's stream, no host
+ * synchronisation.  Bad drop_levels: NDMPS_ERR_INVALID; a core_cap below a core's size: NDMPS_ERR_CAPACITY, before
+ * anything is enqueued. */
+int ndmps_marginalize(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void* const* cores, int dtype, const int64_t* ranks,
+                      const int64_t* drop_levels, void* const* cores_out, const int64_t* core_cap);
 
 /* ---- K8: <a|b> --------------------------------------------------------------
  * `mps @ mps` at core/ndmps.py:76,86 and utils/metrics.py:160 (no conjugation). */
