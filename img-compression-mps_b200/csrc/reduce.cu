@@ -133,7 +133,10 @@ __global__ void __launch_bounds__(256) quantize_kernel(const T* __restrict__ x, 
         // every step rounded separately (no FMA contraction) so the bytes match numpy's
         double u = __ddiv_rn(__dsub_rn((double)x[i], lo), span);
         double v = __dmul_rn(u, qmax);
-        q[i] = (Q)v;
+        // NaN (0 / 0: a constant array, lo == hi) gives 0 for every type; the conversion alone gives 0x80...0 for the
+        // 32- and 64-bit ones.  Values past the type's range (the top code of the 64-bit types, 2^64 or 2^63 in
+        // float64) saturate in the conversion
+        q[i] = isnan(v) ? (Q)0 : (Q)v;
     }
 }
 
@@ -189,7 +192,7 @@ static void launch_dequantize(ndmps_ctx* ctx, int grid, const void* q, int64_t n
 extern "C" {
 
 int ndmps_sumsq(ndmps_ctx_t* ctx, const void* x, int64_t n, int dtype, double* out_host) {
-    NDMPS_REQUIRE(ctx && x && out_host, "ndmps_sumsq: NULL argument");
+    NDMPS_REQUIRE(ctx && (x || n == 0) && out_host, "ndmps_sumsq: NULL argument");   // an empty tensor may have no storage
     NDMPS_REQUIRE(dtype_ok(dtype) && n >= 0, "ndmps_sumsq: bad dtype or size");
     NDMPS_TRY(ctx->ws.reset(ctx->stream));
     NDMPS_TRY(ensure_pinned(ctx, 2));

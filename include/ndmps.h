@@ -127,7 +127,7 @@ int ndmps_encode(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void* src, vo
 int ndmps_decode(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void* src, void* dst, int dtype);
 
 /* ---- reductions ---------------------------------------------------------- */
-/* sum of squares (np.linalg.norm at core/ndmps.py:61 is its square root) */
+/* sum of squares (np.linalg.norm at core/ndmps.py:61 is its square root); n = 0 gives 0 and x may then be NULL */
 int ndmps_sumsq(ndmps_ctx_t* ctx, const void* x, int64_t n, int dtype, double* out_host);
 /* K12: [min, max] of each of `count` arrays (boundary_list, core/ndmps.py:75,82) */
 int ndmps_minmax(ndmps_ctx_t* ctx, const void* const* arrays, const int64_t* sizes, int count, int dtype,
@@ -275,7 +275,9 @@ int ndmps_overlap(ndmps_ctx_t* ctx, const void* const* cores_a, const int64_t* r
 /* ---- K12: min-max quantisation ----------------------------------------------
  * utils/filetools.py:20-26 (scale_to_dtype, truncating cast) and :29-39
  * (scale_back), used by core/ndmps.py:200-204.  `bits` names the integer type like numpy's iinfo
- * dtypes: 8 / 16 / 32 / 64 unsigned, -8 / -16 / -32 / -64 signed; iinfo(dtype).max is the scale. */
+ * dtypes: 8 / 16 / 32 / 64 unsigned, -8 / -16 / -32 / -64 signed; iinfo(dtype).max is the scale.
+ * Where numpy's cast is undefined the result is defined here: NaN (every element of a constant array,
+ * lo == hi) gives 0, and values past the type's range (the top code of the 64-bit types) saturate. */
 int ndmps_quantize(ndmps_ctx_t* ctx, const void* x, int64_t n, int dtype, double lo, double hi, int bits, void* q_out);
 int ndmps_dequantize(ndmps_ctx_t* ctx, const void* q, int64_t n, int bits, double lo, double hi, int dtype, void* x_out);
 
