@@ -21,6 +21,10 @@
 // Point path (ndmps_evaluate_points): the full chains X (P_s x r) and W (r x Q_s) of contract_dense, W transposed so
 // that the column of a point is one contiguous bond vector; a warp works out the indices of 32 points (one per lane)
 // and then runs their 32 length-r dot products.
+//
+// Sampling (ndmps_sample_points, ndmps_sample_grid): multilinear interpolation at real coordinates on the same chains
+// and tables.  Each axis is clamped to [0, n - 1] and contributes its floor and floor + 1 (clamped) digits, so a sample
+// is the weighted sum of the dot products of its 2^ndim corners; corners of weight 0 are skipped.
 #include <math.h>
 
 #include "common.cuh"
@@ -81,6 +85,14 @@ __device__ __forceinline__ double bond_dot(const T* __restrict__ x, const T* __r
     return s;
 }
 
+// C[k, t] of the orthonormal inverse DCT-II of length n: x[t] = sum_k y[k] C[k, t],
+// C[k, t] = sqrt(2/n) cos(pi (2t+1) k / (2n)), row k = 0 scaled by 1/sqrt(2); q = (2t+1) k mod 4n
+__device__ __forceinline__ double idct_basis(int64_t q, int64_t k, int64_t n) {
+    double c = sqrt(2.0 / (double)n) * cospi((double)q / (double)(2 * n));
+    if (k == 0) c *= 0.70710678118654752440;
+    return c;
+}
+
 // out[p] = X[row(x_p), :] . Wt[col(x_p), :]; NaN for a coordinate outside [-shape, shape) (the host checks first).
 // A warp takes 32 points: each lane works out the row and column of its own point (the integer divisions are most of
 // a point's instructions), then the warp walks the 32 points with the indices shuffled to every lane, one length-r
@@ -123,12 +135,8 @@ evaluate_points_kernel(const T* __restrict__ X, const T* __restrict__ Wt, const 
             if (okj && !pa.idct) {
                 acc = bond_dot(X + rj * pa.r, Wt ? Wt + cj * pa.r : nullptr, pa.r, lane);
             } else if (okj) {
-                // x[t] = sum_k y[k] C[k, t],  C[k, t] = sqrt(2/n) cos(pi (2t+1) k / (2n)), row k = 0 scaled by 1/sqrt(2)
-                const double scale = sqrt(2.0 / (double)nl);
                 for (int64_t k = 0; k < nl; k++) {
-                    const int64_t q = ((2 * xj + 1) * k) % (4 * nl);
-                    double c = scale * cospi((double)q / (double)(2 * nl));
-                    if (k == 0) c *= 0.70710678118654752440;
+                    const double c = idct_basis(((2 * xj + 1) * k) % (4 * nl), k, nl);
                     const int64_t rk = rj + rl[k / gl], ck = cj + cl[k % gl];
                     acc = fma(c, bond_dot(X + rk * pa.r, Wt ? Wt + ck * pa.r : nullptr, pa.r, lane), acc);
                 }
@@ -140,8 +148,149 @@ evaluate_points_kernel(const T* __restrict__ X, const T* __restrict__ Wt, const 
     }
 }
 
-static int warp_grid(const ndmps_ctx* ctx, int64_t warps) {
-    int64_t want = (warps + 7) / 8, cap = (int64_t)ctx->sm_count * 16;
+// coordinate sources of sample_points_kernel: at(p, n, x) writes the n coordinates of sample p
+struct CoordList {                     // (count x n) float64, C order
+    const double* c = nullptr;
+    __device__ __forceinline__ void at(int64_t p, int n, double (&x)[8]) const {
+#pragma unroll
+        for (int a = 0; a < 8; a++) x[a] = a < n ? c[p * n + a] : 0.0;
+    }
+};
+
+struct AffineGrid {                    // sample p = C-order index (i_0, .., i_{m-1}) over shape: origin + sum_j i_j steps[j]
+    int m = 0;
+    int64_t shape[8] = {0};
+    double origin[8] = {0};
+    double steps[8][8] = {{0}};
+    __device__ __forceinline__ void at(int64_t p, int n, double (&x)[8]) const {
+#pragma unroll
+        for (int a = 0; a < 8; a++) x[a] = origin[a];
+        int64_t rem = p;
+#pragma unroll
+        for (int j = 7; j >= 0; j--)
+            if (j < m) {
+                const int64_t q = rem / shape[j];
+                const double i = (double)(rem - q * shape[j]);
+                rem = q;
+#pragma unroll
+                for (int a = 0; a < 8; a++)
+                    if (a < n) x[a] = fma(i, steps[j][a], x[a]);
+            }
+    }
+};
+
+struct SampleCorners {                 // one sample as its warp reads it
+    int64_t row, col;                  // the corner at the floor of every axis
+    int64_t drow[8], dcol[8];          // change of row / column when axis a moves to its upper neighbour
+    double f[8];                       // weight of the upper neighbour (1 - f of the floor)
+    int64_t t0, t1;                    // DCT mode: the two positions on the last axis
+    int ok;
+};
+
+// SampleCorners of 32 samples per warp: 30 KB of shared memory a block.  The kernel asks for 4 resident blocks (up to
+// 128 registers a thread): left to the shared-memory occupancy of 7 blocks, ptxas caps it at 72 registers and spills.
+#define NDMPS_SAMPLE_WARPS 4
+
+// out[p] = multilinear interpolation of the volume at src.at(p), each coordinate clamped to [0, n - 1] first; NaN for a
+// non-finite coordinate, for which no core is read (the host refuses such input first).  Layout of
+// evaluate_points_kernel: a lane works out the corners of its own sample into shared memory, then the warp walks the
+// 32 samples, accumulating w_c * (its lanes' share of the dot product of corner c) over the corners, so one warp sum per
+// sample; the 32 results leave in one coalesced store.  In DCT mode the last axis holds coefficients: the basis row
+// c(k) = (1 - f) C[k, t0] + f C[k, t1] is interpolated instead, and every coefficient k is summed over the corners of the
+// other axes.
+template <class T, class Src>
+__global__ void __launch_bounds__(NDMPS_SAMPLE_WARPS * 32, 4)
+sample_points_kernel(const T* __restrict__ X, const T* __restrict__ Wt, Src src, int64_t count, PointArgs pa,
+                     T* __restrict__ out) {
+    __shared__ SampleCorners smem[NDMPS_SAMPLE_WARPS][32];
+    const int lane = threadIdx.x & 31;
+    SampleCorners* sc = smem[threadIdx.x >> 5];
+    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    const int nc = pa.n - pa.idct;     // axes interpolated through corners
+    int64_t nl = 1, gl = 1;
+    const int64_t *rl = nullptr, *cl = nullptr;
+#pragma unroll
+    for (int a = 0; a < 8; a++)
+        if (a == pa.n - 1) { nl = pa.shape[a]; gl = pa.gran[a]; rl = pa.rtab[a]; cl = pa.ctab[a]; }
+    for (int64_t first = (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5) * 32; first < count; first += nwarps * 32) {
+        const int64_t p = first + lane;
+        SampleCorners& s = sc[lane];
+        int ok = p < count;
+        if (ok) {
+            double x[8];
+            src.at(p, pa.n, x);
+            int64_t row = 0, col = 0;
+#pragma unroll
+            for (int a = 0; a < 8; a++) {
+                if (a >= pa.n) continue;
+                if (!isfinite(x[a])) ok = 0;     // clamped below like any other value, so every table read stays in bounds
+                const double v = fmin(fmax(x[a], 0.0), (double)(pa.shape[a] - 1));
+                const double fl = floor(v);
+                const int64_t i0 = (int64_t)fl, i1 = i0 + 1 < pa.shape[a] ? i0 + 1 : i0;
+                s.f[a] = v - fl;
+                if (a >= nc) {
+                    s.t0 = i0;
+                    s.t1 = i1;
+                } else {
+                    const int64_t r0 = pa.rtab[a][i0 / pa.gran[a]], c0 = pa.ctab[a][i0 % pa.gran[a]];
+                    row += r0;
+                    col += c0;
+                    s.drow[a] = pa.rtab[a][i1 / pa.gran[a]] - r0;
+                    s.dcol[a] = pa.ctab[a][i1 % pa.gran[a]] - c0;
+                }
+            }
+            s.row = row;
+            s.col = col;
+        }
+        s.ok = ok;
+        __syncwarp();
+        const int m = count - first < 32 ? (int)(count - first) : 32;
+        double mine = 0.0;
+        for (int j = 0; j < m; j++) {                 // uniform over the warp
+            const SampleCorners& sj = sc[j];
+            if (!sj.ok) continue;
+            double acc = 0.0;
+            const int64_t kn = pa.idct ? nl : 1;
+            const double ft = pa.idct ? sj.f[pa.n - 1] : 0.0;
+            // DCT mode: (2t+1) k mod 4n of both positions and the digits k / gl, k mod gl, stepped with k
+            int64_t q0 = 0, q1 = 0, kh = 0, kl = 0;
+            for (int64_t k = 0; k < kn; k++) {
+                double ck = 1.0;
+                int64_t rk = sj.row, ckol = sj.col;
+                if (pa.idct) {
+                    ck = idct_basis(q0, k, nl);
+                    if (ft != 0.0) ck = fma(ft, idct_basis(q1, k, nl) - ck, ck);
+                    rk += rl[kh];
+                    ckol += cl[kl];
+                    q0 += 2 * sj.t0 + 1;
+                    q0 -= q0 >= 4 * nl ? 4 * nl : 0;
+                    q1 += 2 * sj.t1 + 1;
+                    q1 -= q1 >= 4 * nl ? 4 * nl : 0;
+                    if (++kl == gl) { kl = 0; kh++; }
+                }
+                for (int c = 0; c < (1 << nc); c++) {
+                    double w = ck;
+                    int64_t rc = rk, cc = ckol;
+#pragma unroll
+                    for (int a = 0; a < 8; a++)
+                        if (a < nc) {
+                            if ((c >> a) & 1) { w *= sj.f[a]; rc += sj.drow[a]; cc += sj.dcol[a]; }
+                            else w *= 1.0 - sj.f[a];
+                        }
+                    if (w == 0.0) continue;
+                    acc = fma(w, bond_dot(X + rc * pa.r, Wt ? Wt + cc * pa.r : nullptr, pa.r, lane), acc);
+                }
+            }
+            acc = warp_sum(acc);
+            if (lane == j) mine = acc;
+        }
+        if (p < count) out[p] = ok ? (T)mine : (T)NAN;
+        __syncwarp();                                 // sc is rewritten by the next round
+    }
+}
+
+static int warp_grid(const ndmps_ctx* ctx, int64_t warps, int warps_per_block = 8) {
+    int64_t want = (warps + warps_per_block - 1) / warps_per_block, cap = (int64_t)ctx->sm_count * 16 * (8 / warps_per_block);
     if (want < 1) want = 1;
     return (int)(want < cap ? want : cap);
 }
@@ -368,8 +517,10 @@ static int contract_region(ndmps_ctx* ctx, const ndmps_plan* p, const void* cons
     return gather_sum(ctx, T, out, dtype, level_args(rp.box, tabs, 1));
 }
 
-static int evaluate_points(ndmps_ctx* ctx, const ndmps_plan* p, const void* const* cores, int dtype, const int64_t* ranks,
-                           const int64_t* coords, int64_t count, int idct, void* out) {
+// Set-up shared by the point and sampling paths: the per-axis row / column tables (uploaded in one copy), the full
+// left chain X (P_s x r) and W^T (Q_s x r), the gather of the full right chain.  L = 1: X is the core and *Wt nullptr.
+static int point_setup(ndmps_ctx* ctx, const ndmps_plan* p, const void* const* cores, int dtype, const int64_t* ranks,
+                       int idct, PointArgs* pa_out, const void** X_out, const void** Wt_out) {
     const int L = p->levels, n = p->ndim;
     const size_t esz = dtype_size(dtype);
     const int s = split_of(p);
@@ -409,7 +560,6 @@ static int evaluate_points(ndmps_ctx* ctx, const ndmps_plan* p, const void* cons
     }
     int64_t* tabs_dev = nullptr;
     NDMPS_TRY(upload_tables(ctx, tabs, &tabs_dev));
-    StageScope sc(ctx, ST_CONTRACT);
     const void* X = cores[0];          // L = 1: the core is the volume and W the scalar 1 (Wt = nullptr)
     void* Wt = nullptr;
     if (L > 1) {
@@ -426,7 +576,7 @@ static int evaluate_points(ndmps_ctx* ctx, const ndmps_plan* p, const void* cons
         g.tab[1] = tabs_dev + toff + Q;
         NDMPS_TRY(gather_sum(ctx, W, Wt, dtype, g));
     }
-    PointArgs pa;
+    PointArgs& pa = *pa_out;
     pa.n = n;
     pa.idct = idct;
     pa.r = r;
@@ -436,12 +586,50 @@ static int evaluate_points(ndmps_ctx* ctx, const ndmps_plan* p, const void* cons
         pa.rtab[a] = tabs_dev + roff[(size_t)a];
         pa.ctab[a] = tabs_dev + coff[(size_t)a];
     }
+    *X_out = X;
+    *Wt_out = Wt;
+    return NDMPS_OK;
+}
+
+static int evaluate_points(ndmps_ctx* ctx, const ndmps_plan* p, const void* const* cores, int dtype, const int64_t* ranks,
+                           const int64_t* coords, int64_t count, int idct, void* out) {
+    StageScope sc(ctx, ST_CONTRACT);
+    PointArgs pa;
+    const void *X = nullptr, *Wt = nullptr;
+    NDMPS_TRY(point_setup(ctx, p, cores, dtype, ranks, idct, &pa, &X, &Wt));
     const int grid = warp_grid(ctx, (count + 31) / 32);   // a warp per 32 points
     if (dtype == NDMPS_F32)
         evaluate_points_kernel<float><<<grid, 256, 0, ctx->stream>>>((const float*)X, (const float*)Wt, coords, count, pa, (float*)out);
     else
         evaluate_points_kernel<double><<<grid, 256, 0, ctx->stream>>>((const double*)X, (const double*)Wt, coords, count, pa, (double*)out);
     NDMPS_LAUNCH_CHECK(ctx);
+    return NDMPS_OK;
+}
+
+template <class Src>
+static int sample_points(ndmps_ctx* ctx, const ndmps_plan* p, const void* const* cores, int dtype, const int64_t* ranks,
+                         const Src& src, int64_t count, int idct, void* out) {
+    StageScope sc(ctx, ST_CONTRACT);
+    PointArgs pa;
+    const void *X = nullptr, *Wt = nullptr;
+    NDMPS_TRY(point_setup(ctx, p, cores, dtype, ranks, idct, &pa, &X, &Wt));
+    const int grid = warp_grid(ctx, (count + 31) / 32, NDMPS_SAMPLE_WARPS);   // a warp per 32 samples
+    if (dtype == NDMPS_F32)
+        sample_points_kernel<float, Src><<<grid, NDMPS_SAMPLE_WARPS * 32, 0, ctx->stream>>>((const float*)X, (const float*)Wt, src,
+                                                                                          count, pa, (float*)out);
+    else
+        sample_points_kernel<double, Src><<<grid, NDMPS_SAMPLE_WARPS * 32, 0, ctx->stream>>>((const double*)X, (const double*)Wt,
+                                                                                           src, count, pa, (double*)out);
+    NDMPS_LAUNCH_CHECK(ctx);
+    return NDMPS_OK;
+}
+
+// the argument checks every point entry point makes on the MPS itself
+static int check_mps(const char* fn, const ndmps_plan* plan, const void* const* cores, int dtype, const int64_t* ranks) {
+    NDMPS_REQUIRE(dtype_ok(dtype), "%s: bad dtype %d", fn, dtype);
+    NDMPS_REQUIRE(plan->levels == 1 || ranks, "%s: ranks is NULL", fn);
+    for (int i = 0; i < plan->levels; i++) NDMPS_REQUIRE(cores[i], "%s: core %d is NULL", fn, i);
+    for (int i = 0; i + 1 < plan->levels; i++) NDMPS_REQUIRE(ranks[i] >= 1, "%s: bond %d is %lld", fn, i, (long long)ranks[i]);
     return NDMPS_OK;
 }
 
@@ -477,6 +665,48 @@ int ndmps_evaluate_points(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void
     if (count == 0) return NDMPS_OK;
     NDMPS_TRY(ctx->ws.reset(ctx->stream));
     return evaluate_points(ctx, plan, cores, dtype, ranks, coords_dev, count, idct_last_axis ? 1 : 0, out_dev);
+}
+
+int ndmps_sample_points(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void* const* cores, int dtype, const int64_t* ranks,
+                        const double* coords_dev, int64_t count, int idct_last_axis, void* out_dev) {
+    NDMPS_REQUIRE(ctx && plan && cores && (count == 0 || (coords_dev && out_dev)), "ndmps_sample_points: NULL argument");
+    NDMPS_REQUIRE(count >= 0, "ndmps_sample_points: count %lld", (long long)count);
+    NDMPS_TRY(check_mps("ndmps_sample_points", plan, cores, dtype, ranks));
+    if (count == 0) return NDMPS_OK;
+    NDMPS_TRY(ctx->ws.reset(ctx->stream));
+    CoordList src;
+    src.c = coords_dev;
+    return sample_points(ctx, plan, cores, dtype, ranks, src, count, idct_last_axis ? 1 : 0, out_dev);
+}
+
+int ndmps_sample_grid(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void* const* cores, int dtype, const int64_t* ranks,
+                      const double* origin, const double* steps, const int64_t* out_shape, int m, int idct_last_axis,
+                      void* out_dev) {
+    NDMPS_REQUIRE(ctx && plan && cores && origin && steps && out_shape, "ndmps_sample_grid: NULL argument");
+    NDMPS_REQUIRE(m >= 1 && m <= 8, "ndmps_sample_grid: m = %d outside 1..8", m);
+    NDMPS_TRY(check_mps("ndmps_sample_grid", plan, cores, dtype, ranks));
+    const int n = plan->ndim;
+    AffineGrid src;
+    src.m = m;
+    int64_t count = 1;
+    for (int j = 0; j < m; j++) {
+        NDMPS_REQUIRE(out_shape[j] >= 0, "ndmps_sample_grid: out_shape[%d] = %lld", j, (long long)out_shape[j]);
+        src.shape[j] = out_shape[j];
+        count *= out_shape[j];
+    }
+    for (int a = 0; a < n; a++) {
+        NDMPS_REQUIRE(std::isfinite(origin[a]), "ndmps_sample_grid: origin[%d] is not finite", a);
+        src.origin[a] = origin[a];
+        for (int j = 0; j < m; j++) {
+            NDMPS_REQUIRE(std::isfinite(steps[j * n + a]), "ndmps_sample_grid: steps[%d][%d] is not finite", j, a);
+            src.steps[j][a] = steps[j * n + a];
+        }
+    }
+    // an empty grid writes nothing, so its output may be NULL
+    if (count == 0) return NDMPS_OK;
+    NDMPS_REQUIRE(out_dev, "ndmps_sample_grid: out_dev is NULL");
+    NDMPS_TRY(ctx->ws.reset(ctx->stream));
+    return sample_points(ctx, plan, cores, dtype, ranks, src, count, idct_last_axis ? 1 : 0, out_dev);
 }
 
 int ndmps_region_debug_offsets(const ndmps_plan_t* plan, const int64_t* lo, const int64_t* hi, int64_t* info_out,

@@ -72,6 +72,8 @@ PROTOTYPES = {
     "ndmps_contract_dense": (ci, [vp, p_vp, ci, ci, p_i64, p_i64, vp]),
     "ndmps_contract_region": (ci, [vp, vp, p_vp, ci, p_i64, p_i64, p_i64, vp]),
     "ndmps_evaluate_points": (ci, [vp, vp, p_vp, ci, p_i64, vp, i64, ci, vp]),
+    "ndmps_sample_points": (ci, [vp, vp, p_vp, ci, p_i64, vp, i64, ci, vp]),
+    "ndmps_sample_grid": (ci, [vp, vp, p_vp, ci, p_i64, p_f64, p_f64, p_i64, ci, ci, vp]),
     "ndmps_region_debug_offsets": (ci, [vp, p_i64, p_i64, p_i64, p_i64]),
     "ndmps_marginalize": (ci, [vp, vp, p_vp, ci, p_i64, p_i64, p_vp, p_i64]),
     "ndmps_overlap": (ci, [vp, p_vp, p_i64, ci, p_vp, p_i64, ci, ci, p_i64, p_f64]),

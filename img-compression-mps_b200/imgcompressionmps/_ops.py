@@ -474,6 +474,78 @@ def evaluate_points(cores, shape, coords, idct_last_axis: bool = False):
     return out
 
 
+def sample_points(cores, shape, coords, idct_last_axis: bool = False):
+    """Multilinear interpolation of the volume of ``shape`` at ``coords`` (float64 device tensor, K x ndim), each
+    coordinate clamped to [0, extent - 1]; a device tensor of K values.  A non-finite coordinate gives NaN."""
+    torch = _torch()
+    cores = [_dev(c, "core") for c in cores]
+    _dev(coords, "coords")
+    if coords.dtype != torch.float64 or coords.ndim != 2 or coords.shape[1] != len(shape):
+        raise ValueError("sample_points: coords must be a float64 (K, ndim) tensor")
+    plan = plan_for(tuple(shape))
+    count = int(coords.shape[0])
+    out = torch.empty(count, dtype=cores[0].dtype, device=cores[0].device)
+    N.check(N.load_library().ndmps_sample_points(N.handle(), plan.handle, N.ptr_array(cores), N.dtype_code(cores[0].dtype),
+                                                 N.i64_array(_ranks_of(cores)), N.ptr(coords), count,
+                                                 int(bool(idct_last_axis)), N.ptr(out)), "ndmps_sample_points")
+    return out
+
+
+def grid_args(ndim, origin, steps, shape):
+    """Validated (origin (ndim,), steps (m, ndim), shape (m,)) of an affine sampling grid, as float64 arrays and a tuple
+    of ints.  ``origin`` and ``steps`` must be real and finite, 1 <= m <= 8, ``shape`` m non-negative ints; every
+    coordinate of the grid must be finite too.  A wrong length, a non-real or non-finite value or a negative extent
+    raises ``ValueError``; a bool or non-integer extent ``TypeError``."""
+    import operator
+
+    def real(a, what):
+        a = np.asarray(a)
+        if a.dtype == np.bool_ or a.dtype.kind not in "iuf":
+            raise ValueError(f"{what} must be real numbers, got {a.dtype}")
+        a = np.ascontiguousarray(a, dtype=np.float64)
+        if not np.isfinite(a).all():
+            raise ValueError(f"{what} must be finite")
+        return a
+
+    origin = real(origin, "origin")
+    steps = real(steps, "steps")
+    if origin.shape != (ndim,):
+        raise ValueError(f"origin must have {ndim} values, got shape {origin.shape}")
+    if steps.ndim != 2 or steps.shape[1] != ndim or not 1 <= steps.shape[0] <= 8:
+        raise ValueError(f"steps must have shape (m, {ndim}) with 1 <= m <= 8, got {steps.shape}")
+    out_shape = []
+    for v in shape:
+        if isinstance(v, (bool, np.bool_)) or not hasattr(v, "__index__"):
+            raise TypeError(f"shape: {v!r} is not an integer")
+        out_shape.append(operator.index(v))
+    if len(out_shape) != steps.shape[0]:
+        raise ValueError(f"shape has {len(out_shape)} extents for {steps.shape[0]} step vectors")
+    if any(v < 0 for v in out_shape):
+        raise ValueError(f"shape {tuple(out_shape)} has a negative extent")
+    # the largest |coordinate| the grid reaches: finite, so is every coordinate
+    with np.errstate(over="ignore"):
+        far = np.abs(origin) + (np.maximum(np.array(out_shape, dtype=np.float64) - 1, 0)[:, None] * np.abs(steps)).sum(axis=0)
+    if not np.isfinite(far).all():
+        raise ValueError("the grid reaches a non-finite coordinate")
+    return origin, steps, tuple(out_shape)
+
+
+def sample_grid(cores, shape, origin, steps, out_shape, idct_last_axis: bool = False):
+    """``sample_points`` at the affine grid origin + sum_j i_j steps[j] over ``out_shape`` (C order), with the
+    coordinates computed in the kernel; a device tensor of ``out_shape``.  Arguments as ``grid_args`` returns them."""
+    torch = _torch()
+    cores = [_dev(c, "core") for c in cores]
+    plan = plan_for(tuple(shape))
+    origin = np.ascontiguousarray(origin, dtype=np.float64)
+    steps = np.ascontiguousarray(steps, dtype=np.float64)
+    out = torch.empty(tuple(int(v) for v in out_shape), dtype=cores[0].dtype, device=cores[0].device)
+    N.check(N.load_library().ndmps_sample_grid(N.handle(), plan.handle, N.ptr_array(cores), N.dtype_code(cores[0].dtype),
+                                               N.i64_array(_ranks_of(cores)), origin.ctypes.data_as(N.p_f64),
+                                               steps.ctypes.data_as(N.p_f64), N.i64_array(out_shape), len(out_shape),
+                                               int(bool(idct_last_axis)), N.ptr(out)), "ndmps_sample_grid")
+    return out
+
+
 def overlap(cores_a, cores_b) -> float:
     cores_a = [_dev(c, "core") for c in cores_a]
     cores_b = [_dev(c, "core") for c in cores_b]

@@ -243,6 +243,80 @@ class NDMPS:
         out = _ops.evaluate_points(cores, self._shape, dev, idct_last_axis=self.mode == "DCT")
         return out if on_device else out.cpu().numpy()
 
+    # ------------------------------------------------------------------ interpolated sampling (extension)
+    def sample(self, coords):
+        """``scipy.ndimage.map_coordinates(to_tensor(), coords.T, order=1, mode="nearest")``: the reconstruction
+        linearly interpolated at K real-valued points, without reconstructing the whole tensor.
+
+        ``coords``: real array of shape (K, ndim), numpy (result: numpy array) or a CUDA tensor (result: CUDA tensor),
+        any real dtype; integer coordinates give ``values_at``'s values.  Each coordinate is clamped to
+        [0, extent - 1] and the 2^ndim voxels around it are weighted multilinearly; duplicates and K = 0 are allowed.
+        A wrong shape, a bool or non-real dtype, or a NaN / infinite coordinate raises ``ValueError``.  A sample costs
+        up to 2^ndim bond-length dot products on the device (fewer where a coordinate is an integer); in "DCT" mode
+        the inverse-DCT basis row is interpolated along the last axis, n * 2^(ndim-1) dot products per sample for a
+        last extent n.  The path is for samples few compared with the voxels: oblique slices, probes along a path,
+        a few in-between frames; the workspace is the decode chains and tables of ``values_at``, nothing of the
+        size of the volume.  Any other mode returns None after the arguments are checked."""
+        torch = _torch()
+        ndim = len(self._shape)
+        on_device = isinstance(coords, torch.Tensor)
+        if on_device and not coords.is_cuda:
+            raise ValueError("sample: coords must be a numpy array or a CUDA tensor")
+        if not on_device:
+            coords = np.asarray(coords)
+        if coords.ndim != 2 or int(coords.shape[1]) != ndim:
+            raise ValueError(f"sample: coords must have shape (K, {ndim}), got {tuple(coords.shape)}")
+        if on_device:
+            real = not coords.dtype.is_complex and coords.dtype != torch.bool
+        else:
+            real = coords.dtype.kind in "iuf"
+        if not real:
+            raise ValueError(f"sample: coordinates must be real numbers, got {coords.dtype}")
+        if on_device:
+            coords = coords.to(torch.float64).contiguous()
+            finite = bool(torch.isfinite(coords).all().item()) if coords.numel() else True
+        else:
+            coords = np.ascontiguousarray(coords, dtype=np.float64)
+            finite = bool(np.isfinite(coords).all())
+        if not finite:
+            raise ValueError("sample: a coordinate is NaN or infinite")
+        if self.mode not in ("Std", "DCT"):
+            return None
+        cores = self.mps.cores
+        dev = coords if on_device else torch.from_numpy(coords).to(cores[0].device)
+        out = _ops.sample_points(cores, self._shape, dev, idct_last_axis=self.mode == "DCT")
+        return out if on_device else out.cpu().numpy()
+
+    def sample_grid_device(self, origin, steps, shape):
+        """``sample`` at an affine grid, as a CUDA tensor of ``shape``: the value at index (i_0, .., i_{m-1}) is the
+        sample at ``origin + sum_j i_j * steps[j]``.  The coordinates are computed on the device, so nothing of the
+        output's size is allocated besides the output.
+
+        ``origin``: ndim real numbers (voxel units, axis order of the volume); ``steps``: (m, ndim), 1 <= m <= 8;
+        ``shape``: m non-negative ints.  Mismatched lengths, non-finite values and negative extents raise
+        ``ValueError``.  For a volume of shape (D, H, W):
+
+        * an oblique 512 x 512 plane through the centre c, spanned by orthonormal directions u and v (voxel units):
+          ``origin = c - 255.5 * (u + v)``, ``steps = [u, v]``, ``shape = (512, 512)``;
+        * a resample to (D', H', W') with the corners kept (``align_corners=True``):
+          ``origin = (0, 0, 0)``, ``steps = diag((D - 1) / (D' - 1), (H - 1) / (H' - 1), (W - 1) / (W' - 1))``,
+          ``shape = (D', H', W')``.
+
+        Costs are ``sample``'s per output value.  Any other mode returns None after the arguments are checked."""
+        torch = _torch()
+        origin, steps, out_shape = _ops.grid_args(len(self._shape), origin, steps, shape)
+        if self.mode not in ("Std", "DCT"):
+            return None
+        cores = self.mps.cores
+        if 0 in out_shape:
+            return torch.empty(out_shape, dtype=cores[0].dtype, device=cores[0].device)
+        return _ops.sample_grid(cores, self._shape, origin, steps, out_shape, idct_last_axis=self.mode == "DCT")
+
+    def sample_grid(self, origin, steps, shape):
+        """``sample_grid_device(origin, steps, shape)`` as a numpy array; None for a mode other than "Std" / "DCT"."""
+        rec = self.sample_grid_device(origin, steps, shape)
+        return None if rec is None else rec.cpu().numpy()
+
     # ------------------------------------------------------------------ block-mean reconstruction (extension)
     def coarse_shape(self, levels) -> tuple:
         """Shape of ``to_tensor_coarse(levels)`` with no index: axis a averaged over its finest ``k_a`` digits, i.e.

@@ -240,6 +240,22 @@ int ndmps_contract_region(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void
 int ndmps_evaluate_points(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void* const* cores, int dtype,
                           const int64_t* ranks, const int64_t* coords_dev, int64_t count, int idct_last_axis,
                           void* out_dev);
+/* Multilinear interpolation of the volume at real-valued coordinates: scipy.ndimage.map_coordinates(volume, coords.T,
+ * order=1, mode="nearest"), i.e. each coordinate clamped to [0, extent - 1], then the 2^ndim corners around it weighted
+ * by prod_a (1 - f_a or f_a) (corners of weight 0 are skipped).  Same chains as ndmps_evaluate_points, float64
+ * accumulation, result in the cores' dtype.  idct_last_axis = 1 (mode "DCT"): the inverse-DCT basis row is interpolated
+ * along the last axis instead, n * 2^(ndim-1) dot products per sample.  A non-finite coordinate gives NaN and reads no
+ * core.  No host synchronisation.
+ * ndmps_sample_points: coords_dev: float64 device array (count x ndim).  count 0 is a no-op (NULLs allowed). */
+int ndmps_sample_points(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void* const* cores, int dtype,
+                        const int64_t* ranks, const double* coords_dev, int64_t count, int idct_last_axis, void* out_dev);
+/* ndmps_sample_grid: the coordinates of an affine grid, computed in the kernel (nothing of the output's size is
+ * uploaded): out_dev (C order over out_shape, m axes, 1 <= m <= 8) at index (i_0, .., i_{m-1}) is the sample at
+ * origin + sum_j i_j steps[j].  origin (ndim), steps (m x ndim, row-major) and out_shape (m) are host arrays; origin
+ * and steps must be finite, out_shape non-negative.  A grid with a zero extent is a no-op (out_dev may be NULL). */
+int ndmps_sample_grid(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void* const* cores, int dtype,
+                      const int64_t* ranks, const double* origin, const double* steps, const int64_t* out_shape, int m,
+                      int idct_last_axis, void* out_dev);
 /* host-only index check of ndmps_contract_region (no device work): info_out[3] = {split site s, |H| kept rows,
  * |C| kept columns}; site_offsets_out_host (one value per box voxel, C order) = the flat site-order index
  * (row * Q_s + column) the region path reads for the voxel, mapped back from its compact row and column sets.
