@@ -123,9 +123,7 @@ static int marginalize(ndmps_ctx* ctx, const ndmps_plan* p, const void* const* c
     }
     NDMPS_TRY(ctx->ws.reset(ctx->stream));
     int64_t* tabs_dev = nullptr;
-    NDMPS_TRY(ctx->ws.get<int64_t>(tabs.size(), &tabs_dev));
-    // pageable source: staged before the call returns, so the host vector may go right after
-    NDMPS_CUDA_TRY(cudaMemcpyAsync(tabs_dev, tabs.data(), tabs.size() * sizeof(int64_t), cudaMemcpyHostToDevice, ctx->stream));
+    NDMPS_TRY(upload_tables(ctx, tabs, &tabs_dev));
     StageScope sc(ctx, ST_CONTRACT);
     auto reduce = [&](int l, void* out, bool to_f64) {
         return reduce_site(ctx, cores[l], out, dtype, to_f64, rl_of(l), p->site_dims[l], dk[(size_t)l], rr_of(l),
@@ -188,11 +186,8 @@ int ndmps_plan_layout(const ndmps_plan_t* plan, int* ndim_out, int* levels_out, 
 int ndmps_marginalize(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void* const* cores, int dtype, const int64_t* ranks,
                       const int64_t* drop_levels, void* const* cores_out, const int64_t* core_cap) {
     NDMPS_REQUIRE(ctx && plan && cores && cores_out && core_cap, "ndmps_marginalize: NULL argument");
-    NDMPS_REQUIRE(dtype_ok(dtype), "ndmps_marginalize: bad dtype %d", dtype);
-    NDMPS_REQUIRE(plan->levels == 1 || ranks, "ndmps_marginalize: ranks is NULL");
+    NDMPS_TRY(check_mps("ndmps_marginalize", plan, cores, dtype, ranks));
     NDMPS_TRY(check_drop(plan, drop_levels, "ndmps_marginalize"));
-    for (int i = 0; i < plan->levels; i++) NDMPS_REQUIRE(cores[i], "ndmps_marginalize: core %d is NULL", i);
-    for (int i = 0; i + 1 < plan->levels; i++) NDMPS_REQUIRE(ranks[i] >= 1, "ndmps_marginalize: bond %d is %lld", i, (long long)ranks[i]);
     int Lk = 1;
     std::vector<int64_t> cf;
     coarse_layout(plan, drop_levels, &Lk, cf);

@@ -257,6 +257,10 @@ struct GatherArgs {
     int64_t row = 1;
 };
 int gather_sum(ndmps_ctx* ctx, const void* src, void* dst, int dtype, const GatherArgs& g);
+// host tables -> workspace in one copy on the context's stream (region.cu); the vector may go when the call returns
+int upload_tables(ndmps_ctx* ctx, const std::vector<int64_t>& tabs, int64_t** out);
+// the argument checks every entry point that reads an MPS makes on it (region.cu); fn prefixes the error text
+int check_mps(const char* fn, const ndmps_plan* plan, const void* const* cores, int dtype, const int64_t* ranks);
 // MPS -> dense in two chains and one product (ttsvd.cu), shared by contract_dense and the region / point paths.
 // gathers == nullptr builds the full chains; otherwise gathers[k] keeps the rows (left) / columns (right) of level k.
 int split_site(int L, const int64_t* dims);

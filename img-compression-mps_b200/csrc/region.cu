@@ -18,14 +18,15 @@
 //   3. out[x] = T[iH(x), iC(x)] in volume order, one more gather_sum.
 // The workspace holds T, the restricted chains and the tables - nothing of the size of the volume.
 //
-// Point path (ndmps_evaluate_points): the full chains X (P_s x r) and W (r x Q_s) of contract_dense, W transposed so
-// that the column of a point is one contiguous bond vector; a warp works out the indices of 32 points (one per lane)
-// and then runs their 32 length-r dot products.
-//
-// Sampling (ndmps_sample_points, ndmps_sample_grid): multilinear interpolation at real coordinates on the same chains
-// and tables.  Each axis is clamped to [0, n - 1] and contributes its floor and floor + 1 (clamped) digits, so a sample
-// is the weighted sum of the dot products of its 2^ndim corners; corners of weight 0 are skipped.
+// Point path (ndmps_evaluate_points, ndmps_sample_points, ndmps_sample_grid): one kernel over three coordinate sources
+// (integer points, a list of real coordinates, an affine grid) on the full chains X (P_s x r) and W (r x Q_s) of
+// contract_dense, W transposed so that the column of a point is one contiguous bond vector; a warp works out the
+// indices of 32 points (one per lane) and then runs their length-r dot products.  A real coordinate is clamped to
+// [0, n - 1] per axis and contributes its floor and floor + 1 (clamped) digits, so a sample is the weighted sum of the
+// dot products of its 2^ndim corners (corners of weight 0 are skipped); an integer point is its one corner, weight 1.
 #include <math.h>
+
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -93,63 +94,25 @@ __device__ __forceinline__ double idct_basis(int64_t q, int64_t k, int64_t n) {
     return c;
 }
 
-// out[p] = X[row(x_p), :] . Wt[col(x_p), :]; NaN for a coordinate outside [-shape, shape) (the host checks first).
-// A warp takes 32 points: each lane works out the row and column of its own point (the integer divisions are most of
-// a point's instructions), then the warp walks the 32 points with the indices shuffled to every lane, one length-r
-// dot product each, and the 32 results leave in one coalesced store.
-template <class T>
-__global__ void __launch_bounds__(256)
-evaluate_points_kernel(const T* __restrict__ X, const T* __restrict__ Wt, const int64_t* __restrict__ coords, int64_t count,
-                       PointArgs pa, T* __restrict__ out) {
-    const int lane = threadIdx.x & 31;
-    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-    // the last axis of a DCT-mode volume is summed over: its tables, extent and block size
-    int64_t nl = 1, gl = 1;
-    const int64_t *rl = nullptr, *cl = nullptr;
-#pragma unroll
-    for (int a = 0; a < 8; a++)
-        if (a == pa.n - 1) { nl = pa.shape[a]; gl = pa.gran[a]; rl = pa.rtab[a]; cl = pa.ctab[a]; }
-    for (int64_t first = (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5) * 32; first < count; first += nwarps * 32) {
-        const int64_t p = first + lane;
-        int64_t row = 0, col = 0, xl = 0;
-        int ok = p < count;
-        if (ok) {
-#pragma unroll
-            for (int a = 0; a < 8; a++) {
-                if (a >= pa.n) break;
-                int64_t x = coords[p * pa.n + a];
-                if (x < 0) x += pa.shape[a];
-                if (x < 0 || x >= pa.shape[a]) { ok = 0; x = 0; }
-                if (pa.idct && a == pa.n - 1) { xl = x; continue; }
-                row += pa.rtab[a][x / pa.gran[a]];
-                col += pa.ctab[a][x % pa.gran[a]];
-            }
-        }
-        const int m = count - first < 32 ? (int)(count - first) : 32;
-        double mine = 0.0;
-        for (int j = 0; j < m; j++) {                 // uniform over the warp
-            const int64_t rj = __shfl_sync(0xffffffffu, row, j), cj = __shfl_sync(0xffffffffu, col, j);
-            const int64_t xj = __shfl_sync(0xffffffffu, xl, j);
-            const int okj = __shfl_sync(0xffffffffu, ok, j);
-            double acc = 0.0;
-            if (okj && !pa.idct) {
-                acc = bond_dot(X + rj * pa.r, Wt ? Wt + cj * pa.r : nullptr, pa.r, lane);
-            } else if (okj) {
-                for (int64_t k = 0; k < nl; k++) {
-                    const double c = idct_basis(((2 * xj + 1) * k) % (4 * nl), k, nl);
-                    const int64_t rk = rj + rl[k / gl], ck = cj + cl[k % gl];
-                    acc = fma(c, bond_dot(X + rk * pa.r, Wt ? Wt + ck * pa.r : nullptr, pa.r, lane), acc);
-                }
-            }
-            acc = warp_sum(acc);
-            if (lane == j) mine = acc;
-        }
-        if (p < count) out[p] = ok ? (T)mine : (T)NAN;
-    }
-}
+// Coordinate sources of sample_points_kernel.  `interpolates` is false for integer points: their one corner is the point
+// itself, so the kernel stages no neighbours for them (PointStage below) and walks no corners.  `warps` (a block) and
+// `min_blocks` (resident blocks asked of ptxas, 0: none) follow the size of the staging record.
+struct IntPoints {                     // (count x n) int64, C order; negatives count from the end
+    // PointStage of 32 points per warp: 8 KB a block; the kernel fits 64 registers without asking
+    static constexpr bool interpolates = false;
+    static constexpr int warps = 8, min_blocks = 0;
+    const int64_t* c = nullptr;
+};
 
-// coordinate sources of sample_points_kernel: at(p, n, x) writes the n coordinates of sample p
-struct CoordList {                     // (count x n) float64, C order
+struct Interpolated {
+    // SampleStage of 32 samples per warp: 30 KB of shared memory a block.  The kernel asks for 4 resident blocks (up to
+    // 128 registers a thread): left to the shared-memory occupancy of 7 blocks, ptxas caps it at 72 registers and spills.
+    static constexpr bool interpolates = true;
+    static constexpr int warps = 4, min_blocks = 4;
+};
+
+// real sources: at(p, n, x) writes the n coordinates of sample p
+struct CoordList : Interpolated {      // (count x n) float64, C order
     const double* c = nullptr;
     __device__ __forceinline__ void at(int64_t p, int n, double (&x)[8]) const {
 #pragma unroll
@@ -157,7 +120,7 @@ struct CoordList {                     // (count x n) float64, C order
     }
 };
 
-struct AffineGrid {                    // sample p = C-order index (i_0, .., i_{m-1}) over shape: origin + sum_j i_j steps[j]
+struct AffineGrid : Interpolated {     // sample p = C-order index (i_0, .., i_{m-1}) over shape: origin + sum_j i_j steps[j]
     int m = 0;
     int64_t shape[8] = {0};
     double origin[8] = {0};
@@ -179,34 +142,36 @@ struct AffineGrid {                    // sample p = C-order index (i_0, .., i_{
     }
 };
 
-struct SampleCorners {                 // one sample as its warp reads it
-    int64_t row, col;                  // the corner at the floor of every axis
-    int64_t drow[8], dcol[8];          // change of row / column when axis a moves to its upper neighbour
-    double f[8];                       // weight of the upper neighbour (1 - f of the floor)
-    int64_t t0, t1;                    // DCT mode: the two positions on the last axis
+struct PointStage {                    // one point as its warp reads it
+    int64_t row, col;                  // the corner at the floor of every axis (an integer point: the point)
+    int64_t t0;                        // DCT mode: the (lower) position on the last axis
     int ok;
 };
 
-// SampleCorners of 32 samples per warp: 30 KB of shared memory a block.  The kernel asks for 4 resident blocks (up to
-// 128 registers a thread): left to the shared-memory occupancy of 7 blocks, ptxas caps it at 72 registers and spills.
-#define NDMPS_SAMPLE_WARPS 4
+struct SampleStage : PointStage {      // an interpolated sample adds its upper neighbours
+    int64_t drow[8], dcol[8];          // change of row / column when axis a moves to its upper neighbour
+    double f[8];                       // weight of the upper neighbour (1 - f of the floor)
+    int64_t t1;                        // DCT mode: the upper position on the last axis
+};
 
-// out[p] = multilinear interpolation of the volume at src.at(p), each coordinate clamped to [0, n - 1] first; NaN for a
-// non-finite coordinate, for which no core is read (the host refuses such input first).  Layout of
-// evaluate_points_kernel: a lane works out the corners of its own sample into shared memory, then the warp walks the
-// 32 samples, accumulating w_c * (its lanes' share of the dot product of corner c) over the corners, so one warp sum per
-// sample; the 32 results leave in one coalesced store.  In DCT mode the last axis holds coefficients: the basis row
-// c(k) = (1 - f) C[k, t0] + f C[k, t1] is interpolated instead, and every coefficient k is summed over the corners of the
-// other axes.
+// out[p] = the volume at src's point p: X[row, :] . Wt[col, :] at an integer point, NaN for one outside
+// [-shape, shape); for a real one the multilinear interpolation, each coordinate clamped to [0, n - 1] first, NaN for a
+// non-finite coordinate.  A NaN point reads no core (the host refuses such input first).  A warp takes 32 points: each
+// lane works out the row and column of its own point (the integer divisions are most of a point's instructions) and,
+// for a real one, those of its upper neighbours into shared memory; then the warp walks the 32 points, accumulating
+// w_c * (its lanes' share of the dot product of corner c) over the corners, so one warp sum per point, and the 32
+// results leave in one coalesced store.  In DCT mode the last axis holds coefficients: every coefficient k is summed
+// with the basis row C[k, t] (for a real t, c(k) = (1 - f) C[k, t0] + f C[k, t1]), over the corners of the other axes.
 template <class T, class Src>
-__global__ void __launch_bounds__(NDMPS_SAMPLE_WARPS * 32, 4)
+__global__ void __launch_bounds__(Src::warps * 32, Src::min_blocks)
 sample_points_kernel(const T* __restrict__ X, const T* __restrict__ Wt, Src src, int64_t count, PointArgs pa,
                      T* __restrict__ out) {
-    __shared__ SampleCorners smem[NDMPS_SAMPLE_WARPS][32];
+    using Stage = std::conditional_t<Src::interpolates, SampleStage, PointStage>;
+    __shared__ Stage smem[Src::warps][32];
     const int lane = threadIdx.x & 31;
-    SampleCorners* sc = smem[threadIdx.x >> 5];
+    Stage* sc = smem[threadIdx.x >> 5];
     const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-    const int nc = pa.n - pa.idct;     // axes interpolated through corners
+    const int nc = pa.n - pa.idct;     // axes that contribute a row and a column (the others: the DCT axis)
     int64_t nl = 1, gl = 1;
     const int64_t *rl = nullptr, *cl = nullptr;
 #pragma unroll
@@ -214,29 +179,42 @@ sample_points_kernel(const T* __restrict__ X, const T* __restrict__ Wt, Src src,
         if (a == pa.n - 1) { nl = pa.shape[a]; gl = pa.gran[a]; rl = pa.rtab[a]; cl = pa.ctab[a]; }
     for (int64_t first = (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5) * 32; first < count; first += nwarps * 32) {
         const int64_t p = first + lane;
-        SampleCorners& s = sc[lane];
+        Stage& s = sc[lane];
         int ok = p < count;
         if (ok) {
-            double x[8];
-            src.at(p, pa.n, x);
             int64_t row = 0, col = 0;
+            if constexpr (Src::interpolates) {
+                double x[8];
+                src.at(p, pa.n, x);
 #pragma unroll
-            for (int a = 0; a < 8; a++) {
-                if (a >= pa.n) continue;
-                if (!isfinite(x[a])) ok = 0;     // clamped below like any other value, so every table read stays in bounds
-                const double v = fmin(fmax(x[a], 0.0), (double)(pa.shape[a] - 1));
-                const double fl = floor(v);
-                const int64_t i0 = (int64_t)fl, i1 = i0 + 1 < pa.shape[a] ? i0 + 1 : i0;
-                s.f[a] = v - fl;
-                if (a >= nc) {
-                    s.t0 = i0;
-                    s.t1 = i1;
-                } else {
-                    const int64_t r0 = pa.rtab[a][i0 / pa.gran[a]], c0 = pa.ctab[a][i0 % pa.gran[a]];
-                    row += r0;
-                    col += c0;
-                    s.drow[a] = pa.rtab[a][i1 / pa.gran[a]] - r0;
-                    s.dcol[a] = pa.ctab[a][i1 % pa.gran[a]] - c0;
+                for (int a = 0; a < 8; a++) {
+                    if (a >= pa.n) continue;
+                    if (!isfinite(x[a])) ok = 0;     // clamped below like any other value, so every table read stays in bounds
+                    const double v = fmin(fmax(x[a], 0.0), (double)(pa.shape[a] - 1));
+                    const double fl = floor(v);
+                    const int64_t i0 = (int64_t)fl, i1 = i0 + 1 < pa.shape[a] ? i0 + 1 : i0;
+                    s.f[a] = v - fl;
+                    if (a >= nc) {
+                        s.t0 = i0;
+                        s.t1 = i1;
+                    } else {
+                        const int64_t r0 = pa.rtab[a][i0 / pa.gran[a]], c0 = pa.ctab[a][i0 % pa.gran[a]];
+                        row += r0;
+                        col += c0;
+                        s.drow[a] = pa.rtab[a][i1 / pa.gran[a]] - r0;
+                        s.dcol[a] = pa.ctab[a][i1 % pa.gran[a]] - c0;
+                    }
+                }
+            } else {
+#pragma unroll
+                for (int a = 0; a < 8; a++) {
+                    if (a >= pa.n) break;
+                    int64_t x = src.c[p * pa.n + a];
+                    if (x < 0) x += pa.shape[a];
+                    if (x < 0 || x >= pa.shape[a]) { ok = 0; x = 0; }   // x = 0 keeps the table reads in bounds
+                    if (a >= nc) { s.t0 = x; continue; }
+                    row += pa.rtab[a][x / pa.gran[a]];
+                    col += pa.ctab[a][x % pa.gran[a]];
                 }
             }
             s.row = row;
@@ -247,11 +225,12 @@ sample_points_kernel(const T* __restrict__ X, const T* __restrict__ Wt, Src src,
         const int m = count - first < 32 ? (int)(count - first) : 32;
         double mine = 0.0;
         for (int j = 0; j < m; j++) {                 // uniform over the warp
-            const SampleCorners& sj = sc[j];
+            const Stage& sj = sc[j];
             if (!sj.ok) continue;
             double acc = 0.0;
             const int64_t kn = pa.idct ? nl : 1;
-            const double ft = pa.idct ? sj.f[pa.n - 1] : 0.0;
+            double ft = 0.0;
+            if constexpr (Src::interpolates) ft = pa.idct ? sj.f[pa.n - 1] : 0.0;
             // DCT mode: (2t+1) k mod 4n of both positions and the digits k / gl, k mod gl, stepped with k
             int64_t q0 = 0, q1 = 0, kh = 0, kl = 0;
             for (int64_t k = 0; k < kn; k++) {
@@ -259,25 +238,29 @@ sample_points_kernel(const T* __restrict__ X, const T* __restrict__ Wt, Src src,
                 int64_t rk = sj.row, ckol = sj.col;
                 if (pa.idct) {
                     ck = idct_basis(q0, k, nl);
-                    if (ft != 0.0) ck = fma(ft, idct_basis(q1, k, nl) - ck, ck);
                     rk += rl[kh];
                     ckol += cl[kl];
                     q0 += 2 * sj.t0 + 1;
                     q0 -= q0 >= 4 * nl ? 4 * nl : 0;
-                    q1 += 2 * sj.t1 + 1;
-                    q1 -= q1 >= 4 * nl ? 4 * nl : 0;
+                    if constexpr (Src::interpolates) {
+                        if (ft != 0.0) ck = fma(ft, idct_basis(q1, k, nl) - ck, ck);
+                        q1 += 2 * sj.t1 + 1;
+                        q1 -= q1 >= 4 * nl ? 4 * nl : 0;
+                    }
                     if (++kl == gl) { kl = 0; kh++; }
                 }
-                for (int c = 0; c < (1 << nc); c++) {
+                for (int c = 0; c < (Src::interpolates ? 1 << nc : 1); c++) {
                     double w = ck;
                     int64_t rc = rk, cc = ckol;
+                    if constexpr (Src::interpolates) {
 #pragma unroll
-                    for (int a = 0; a < 8; a++)
-                        if (a < nc) {
-                            if ((c >> a) & 1) { w *= sj.f[a]; rc += sj.drow[a]; cc += sj.dcol[a]; }
-                            else w *= 1.0 - sj.f[a];
-                        }
-                    if (w == 0.0) continue;
+                        for (int a = 0; a < 8; a++)
+                            if (a < nc) {
+                                if ((c >> a) & 1) { w *= sj.f[a]; rc += sj.drow[a]; cc += sj.dcol[a]; }
+                                else w *= 1.0 - sj.f[a];
+                            }
+                        if (w == 0.0) continue;
+                    }
                     acc = fma(w, bond_dot(X + rc * pa.r, Wt ? Wt + cc * pa.r : nullptr, pa.r, lane), acc);
                 }
             }
@@ -471,6 +454,8 @@ GatherArgs level_args(const Level& lv, const int64_t* tabs_dev, int64_t row) {
     return g;
 }
 
+}  // namespace
+
 int upload_tables(ndmps_ctx* ctx, const std::vector<int64_t>& tabs, int64_t** out) {
     NDMPS_TRY(ctx->ws.get<int64_t>(tabs.size(), out));
     // pageable source: staged before the call returns, so the host vector may go right after
@@ -478,7 +463,13 @@ int upload_tables(ndmps_ctx* ctx, const std::vector<int64_t>& tabs, int64_t** ou
     return NDMPS_OK;
 }
 
-}  // namespace
+int check_mps(const char* fn, const ndmps_plan* plan, const void* const* cores, int dtype, const int64_t* ranks) {
+    NDMPS_REQUIRE(dtype_ok(dtype), "%s: bad dtype %d", fn, dtype);
+    NDMPS_REQUIRE(plan->levels == 1 || ranks, "%s: ranks is NULL", fn);
+    for (int i = 0; i < plan->levels; i++) NDMPS_REQUIRE(cores[i], "%s: core %d is NULL", fn, i);
+    for (int i = 0; i + 1 < plan->levels; i++) NDMPS_REQUIRE(ranks[i] >= 1, "%s: bond %d is %lld", fn, i, (long long)ranks[i]);
+    return NDMPS_OK;
+}
 
 static int contract_region(ndmps_ctx* ctx, const ndmps_plan* p, const void* const* cores, int dtype, const int64_t* ranks,
                            const int64_t* lo, const int64_t* hi, void* out) {
@@ -591,21 +582,6 @@ static int point_setup(ndmps_ctx* ctx, const ndmps_plan* p, const void* const* c
     return NDMPS_OK;
 }
 
-static int evaluate_points(ndmps_ctx* ctx, const ndmps_plan* p, const void* const* cores, int dtype, const int64_t* ranks,
-                           const int64_t* coords, int64_t count, int idct, void* out) {
-    StageScope sc(ctx, ST_CONTRACT);
-    PointArgs pa;
-    const void *X = nullptr, *Wt = nullptr;
-    NDMPS_TRY(point_setup(ctx, p, cores, dtype, ranks, idct, &pa, &X, &Wt));
-    const int grid = warp_grid(ctx, (count + 31) / 32);   // a warp per 32 points
-    if (dtype == NDMPS_F32)
-        evaluate_points_kernel<float><<<grid, 256, 0, ctx->stream>>>((const float*)X, (const float*)Wt, coords, count, pa, (float*)out);
-    else
-        evaluate_points_kernel<double><<<grid, 256, 0, ctx->stream>>>((const double*)X, (const double*)Wt, coords, count, pa, (double*)out);
-    NDMPS_LAUNCH_CHECK(ctx);
-    return NDMPS_OK;
-}
-
 template <class Src>
 static int sample_points(ndmps_ctx* ctx, const ndmps_plan* p, const void* const* cores, int dtype, const int64_t* ranks,
                          const Src& src, int64_t count, int idct, void* out) {
@@ -613,23 +589,14 @@ static int sample_points(ndmps_ctx* ctx, const ndmps_plan* p, const void* const*
     PointArgs pa;
     const void *X = nullptr, *Wt = nullptr;
     NDMPS_TRY(point_setup(ctx, p, cores, dtype, ranks, idct, &pa, &X, &Wt));
-    const int grid = warp_grid(ctx, (count + 31) / 32, NDMPS_SAMPLE_WARPS);   // a warp per 32 samples
+    const int grid = warp_grid(ctx, (count + 31) / 32, Src::warps);   // a warp per 32 points
     if (dtype == NDMPS_F32)
-        sample_points_kernel<float, Src><<<grid, NDMPS_SAMPLE_WARPS * 32, 0, ctx->stream>>>((const float*)X, (const float*)Wt, src,
-                                                                                          count, pa, (float*)out);
+        sample_points_kernel<float, Src><<<grid, Src::warps * 32, 0, ctx->stream>>>((const float*)X, (const float*)Wt, src, count, pa,
+                                                                                  (float*)out);
     else
-        sample_points_kernel<double, Src><<<grid, NDMPS_SAMPLE_WARPS * 32, 0, ctx->stream>>>((const double*)X, (const double*)Wt,
-                                                                                           src, count, pa, (double*)out);
+        sample_points_kernel<double, Src><<<grid, Src::warps * 32, 0, ctx->stream>>>((const double*)X, (const double*)Wt, src, count,
+                                                                                   pa, (double*)out);
     NDMPS_LAUNCH_CHECK(ctx);
-    return NDMPS_OK;
-}
-
-// the argument checks every point entry point makes on the MPS itself
-static int check_mps(const char* fn, const ndmps_plan* plan, const void* const* cores, int dtype, const int64_t* ranks) {
-    NDMPS_REQUIRE(dtype_ok(dtype), "%s: bad dtype %d", fn, dtype);
-    NDMPS_REQUIRE(plan->levels == 1 || ranks, "%s: ranks is NULL", fn);
-    for (int i = 0; i < plan->levels; i++) NDMPS_REQUIRE(cores[i], "%s: core %d is NULL", fn, i);
-    for (int i = 0; i + 1 < plan->levels; i++) NDMPS_REQUIRE(ranks[i] >= 1, "%s: bond %d is %lld", fn, i, (long long)ranks[i]);
     return NDMPS_OK;
 }
 
@@ -642,10 +609,7 @@ extern "C" {
 int ndmps_contract_region(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void* const* cores, int dtype, const int64_t* ranks,
                           const int64_t* lo, const int64_t* hi, void* out) {
     NDMPS_REQUIRE(ctx && plan && cores && lo && hi, "ndmps_contract_region: NULL argument");
-    NDMPS_REQUIRE(dtype_ok(dtype), "ndmps_contract_region: bad dtype %d", dtype);
-    NDMPS_REQUIRE(plan->levels == 1 || ranks, "ndmps_contract_region: ranks is NULL");
-    for (int i = 0; i < plan->levels; i++) NDMPS_REQUIRE(cores[i], "ndmps_contract_region: core %d is NULL", i);
-    for (int i = 0; i + 1 < plan->levels; i++) NDMPS_REQUIRE(ranks[i] >= 1, "ndmps_contract_region: bond %d is %lld", i, (long long)ranks[i]);
+    NDMPS_TRY(check_mps("ndmps_contract_region", plan, cores, dtype, ranks));
     bool empty = false;
     NDMPS_TRY(check_box(plan, lo, hi, &empty));
     // an empty box writes nothing, so its output may be NULL (a zero-size tensor has no storage)
@@ -658,13 +622,13 @@ int ndmps_contract_region(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void
 int ndmps_evaluate_points(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void* const* cores, int dtype, const int64_t* ranks,
                           const int64_t* coords_dev, int64_t count, int idct_last_axis, void* out_dev) {
     NDMPS_REQUIRE(ctx && plan && cores && (count == 0 || (coords_dev && out_dev)), "ndmps_evaluate_points: NULL argument");
-    NDMPS_REQUIRE(dtype_ok(dtype) && count >= 0, "ndmps_evaluate_points: bad dtype or count");
-    NDMPS_REQUIRE(plan->levels == 1 || ranks, "ndmps_evaluate_points: ranks is NULL");
-    for (int i = 0; i < plan->levels; i++) NDMPS_REQUIRE(cores[i], "ndmps_evaluate_points: core %d is NULL", i);
-    for (int i = 0; i + 1 < plan->levels; i++) NDMPS_REQUIRE(ranks[i] >= 1, "ndmps_evaluate_points: bond %d is %lld", i, (long long)ranks[i]);
+    NDMPS_REQUIRE(count >= 0, "ndmps_evaluate_points: count %lld", (long long)count);
+    NDMPS_TRY(check_mps("ndmps_evaluate_points", plan, cores, dtype, ranks));
     if (count == 0) return NDMPS_OK;
     NDMPS_TRY(ctx->ws.reset(ctx->stream));
-    return evaluate_points(ctx, plan, cores, dtype, ranks, coords_dev, count, idct_last_axis ? 1 : 0, out_dev);
+    IntPoints src;
+    src.c = coords_dev;
+    return sample_points(ctx, plan, cores, dtype, ranks, src, count, idct_last_axis ? 1 : 0, out_dev);
 }
 
 int ndmps_sample_points(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void* const* cores, int dtype, const int64_t* ranks,

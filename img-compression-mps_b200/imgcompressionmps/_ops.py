@@ -370,13 +370,18 @@ def _dims_of(cores):
     return [int(cores[0].shape[0])] + [int(c.shape[1]) for c in cores[1:]]
 
 
+def _mps_args(cores):
+    """(cores checked by ``_dev``, their pointer array, dtype code, ranks array): an MPS as the C ABI takes it."""
+    cores = [_dev(c, "core") for c in cores]
+    return cores, N.ptr_array(cores), N.dtype_code(cores[0].dtype), N.i64_array(_ranks_of(cores))
+
+
 def contract_dense(cores):
     torch = _torch()
-    cores = [_dev(c, "core") for c in cores]
-    dims, ranks = _dims_of(cores), _ranks_of(cores)
+    cores, ptrs, code, ranks = _mps_args(cores)
+    dims = _dims_of(cores)
     out = torch.empty(dims, dtype=cores[0].dtype, device=cores[0].device)
-    N.check(N.load_library().ndmps_contract_dense(N.handle(), N.ptr_array(cores), N.dtype_code(cores[0].dtype),
-                                                  len(cores), N.i64_array(dims), N.i64_array(ranks), N.ptr(out)),
+    N.check(N.load_library().ndmps_contract_dense(N.handle(), ptrs, code, len(cores), N.i64_array(dims), ranks, N.ptr(out)),
             "ndmps_contract_dense")
     return out
 
@@ -431,12 +436,11 @@ def region_box(shape, index):
 def contract_region(cores, shape, lo, hi, plan=None):
     """Box [lo, hi) of the volume of ``shape`` that the cores encode, as a device tensor of shape hi - lo."""
     torch = _torch()
-    cores = [_dev(c, "core") for c in cores]
+    cores, ptrs, code, ranks = _mps_args(cores)
     plan = plan or plan_for(tuple(shape))
     out = torch.empty([int(h) - int(l) for l, h in zip(lo, hi)], dtype=cores[0].dtype, device=cores[0].device)
-    N.check(N.load_library().ndmps_contract_region(N.handle(), plan.handle, N.ptr_array(cores), N.dtype_code(cores[0].dtype),
-                                                   N.i64_array(_ranks_of(cores)), N.i64_array(lo), N.i64_array(hi),
-                                                   N.ptr(out)), "ndmps_contract_region")
+    N.check(N.load_library().ndmps_contract_region(N.handle(), plan.handle, ptrs, code, ranks, N.i64_array(lo),
+                                                   N.i64_array(hi), N.ptr(out)), "ndmps_contract_region")
     return out
 
 
@@ -444,16 +448,15 @@ def marginalize(cores, shape, levels):
     """Cores of the block mean of the volume of ``shape`` that ``cores`` encode, averaged over the finest ``levels``
     digits of each axis, in the layout of ``coarse_plan(shape, levels)``."""
     torch = _torch()
-    cores = [_dev(c, "core") for c in cores]
+    cores, ptrs, code, ranks = _mps_args(cores)
     shape = tuple(int(s) for s in shape)
     ks = coarse_levels(shape, levels)
     cplan = coarse_plan(shape, ks)
-    ranks = _ranks_of(cores)[:cplan.levels - 1]
-    shapes = [core_shape(i, cplan.levels, cplan.site_dims, ranks) for i in range(cplan.levels)]
+    kept = _ranks_of(cores)[:cplan.levels - 1]
+    shapes = [core_shape(i, cplan.levels, cplan.site_dims, kept) for i in range(cplan.levels)]
     out = [torch.empty(s, dtype=cores[0].dtype, device=cores[0].device) for s in shapes]
-    N.check(N.load_library().ndmps_marginalize(N.handle(), plan_for(shape).handle, N.ptr_array(cores),
-                                               N.dtype_code(cores[0].dtype), N.i64_array(_ranks_of(cores)),
-                                               N.i64_array(ks), N.ptr_array(out), N.i64_array([o.numel() for o in out])),
+    N.check(N.load_library().ndmps_marginalize(N.handle(), plan_for(shape).handle, ptrs, code, ranks, N.i64_array(ks),
+                                               N.ptr_array(out), N.i64_array([o.numel() for o in out])),
             "ndmps_marginalize")
     return out
 
@@ -461,15 +464,14 @@ def marginalize(cores, shape, levels):
 def evaluate_points(cores, shape, coords, idct_last_axis: bool = False):
     """Values of the volume of ``shape`` at ``coords`` (int64 device tensor, K x ndim), as a device tensor of K values."""
     torch = _torch()
-    cores = [_dev(c, "core") for c in cores]
+    cores, ptrs, code, ranks = _mps_args(cores)
     _dev(coords, "coords")
     if coords.dtype != torch.int64 or coords.ndim != 2 or coords.shape[1] != len(shape):
         raise ValueError("evaluate_points: coords must be an int64 (K, ndim) tensor")
     plan = plan_for(tuple(shape))
     count = int(coords.shape[0])
     out = torch.empty(count, dtype=cores[0].dtype, device=cores[0].device)
-    N.check(N.load_library().ndmps_evaluate_points(N.handle(), plan.handle, N.ptr_array(cores), N.dtype_code(cores[0].dtype),
-                                                   N.i64_array(_ranks_of(cores)), N.ptr(coords), count,
+    N.check(N.load_library().ndmps_evaluate_points(N.handle(), plan.handle, ptrs, code, ranks, N.ptr(coords), count,
                                                    int(bool(idct_last_axis)), N.ptr(out)), "ndmps_evaluate_points")
     return out
 
@@ -478,15 +480,14 @@ def sample_points(cores, shape, coords, idct_last_axis: bool = False):
     """Multilinear interpolation of the volume of ``shape`` at ``coords`` (float64 device tensor, K x ndim), each
     coordinate clamped to [0, extent - 1]; a device tensor of K values.  A non-finite coordinate gives NaN."""
     torch = _torch()
-    cores = [_dev(c, "core") for c in cores]
+    cores, ptrs, code, ranks = _mps_args(cores)
     _dev(coords, "coords")
     if coords.dtype != torch.float64 or coords.ndim != 2 or coords.shape[1] != len(shape):
         raise ValueError("sample_points: coords must be a float64 (K, ndim) tensor")
     plan = plan_for(tuple(shape))
     count = int(coords.shape[0])
     out = torch.empty(count, dtype=cores[0].dtype, device=cores[0].device)
-    N.check(N.load_library().ndmps_sample_points(N.handle(), plan.handle, N.ptr_array(cores), N.dtype_code(cores[0].dtype),
-                                                 N.i64_array(_ranks_of(cores)), N.ptr(coords), count,
+    N.check(N.load_library().ndmps_sample_points(N.handle(), plan.handle, ptrs, code, ranks, N.ptr(coords), count,
                                                  int(bool(idct_last_axis)), N.ptr(out)), "ndmps_sample_points")
     return out
 
@@ -534,29 +535,26 @@ def sample_grid(cores, shape, origin, steps, out_shape, idct_last_axis: bool = F
     """``sample_points`` at the affine grid origin + sum_j i_j steps[j] over ``out_shape`` (C order), with the
     coordinates computed in the kernel; a device tensor of ``out_shape``.  Arguments as ``grid_args`` returns them."""
     torch = _torch()
-    cores = [_dev(c, "core") for c in cores]
+    cores, ptrs, code, ranks = _mps_args(cores)
     plan = plan_for(tuple(shape))
     origin = np.ascontiguousarray(origin, dtype=np.float64)
     steps = np.ascontiguousarray(steps, dtype=np.float64)
     out = torch.empty(tuple(int(v) for v in out_shape), dtype=cores[0].dtype, device=cores[0].device)
-    N.check(N.load_library().ndmps_sample_grid(N.handle(), plan.handle, N.ptr_array(cores), N.dtype_code(cores[0].dtype),
-                                               N.i64_array(_ranks_of(cores)), origin.ctypes.data_as(N.p_f64),
+    N.check(N.load_library().ndmps_sample_grid(N.handle(), plan.handle, ptrs, code, ranks, origin.ctypes.data_as(N.p_f64),
                                                steps.ctypes.data_as(N.p_f64), N.i64_array(out_shape), len(out_shape),
                                                int(bool(idct_last_axis)), N.ptr(out)), "ndmps_sample_grid")
     return out
 
 
 def overlap(cores_a, cores_b) -> float:
-    cores_a = [_dev(c, "core") for c in cores_a]
-    cores_b = [_dev(c, "core") for c in cores_b]
+    cores_a, ptrs_a, code_a, ranks_a = _mps_args(cores_a)
+    cores_b, ptrs_b, code_b, ranks_b = _mps_args(cores_b)
     dims = _dims_of(cores_a)
     if dims != _dims_of(cores_b):
         raise ValueError("overlap: the two MPS have different site dimensions")
     out = C.c_double()
-    N.check(N.load_library().ndmps_overlap(N.handle(), N.ptr_array(cores_a), N.i64_array(_ranks_of(cores_a)),
-                                           N.dtype_code(cores_a[0].dtype), N.ptr_array(cores_b),
-                                           N.i64_array(_ranks_of(cores_b)), N.dtype_code(cores_b[0].dtype),
-                                           len(cores_a), N.i64_array(dims), C.byref(out)), "ndmps_overlap")
+    N.check(N.load_library().ndmps_overlap(N.handle(), ptrs_a, ranks_a, code_a, ptrs_b, ranks_b, code_b, len(cores_a),
+                                           N.i64_array(dims), C.byref(out)), "ndmps_overlap")
     return out.value
 
 

@@ -51,6 +51,21 @@ def _to_device(tensor, dtype=None, device=None):
     return torch.from_numpy(host).to(device or "cuda", non_blocking=False)
 
 
+def _coords_in(coords, ndim, name):
+    """(K, ndim) point coordinates as a caller passes them: (the numpy array or CUDA tensor, whether it is a CUDA
+    tensor, the function that turns a device result into the caller's form).  Anything but a numpy array (or what
+    ``np.asarray`` takes) or a CUDA tensor, and a wrong shape, raise ``ValueError``."""
+    torch = _torch()
+    on_device = isinstance(coords, torch.Tensor)
+    if on_device and not coords.is_cuda:
+        raise ValueError(f"{name}: coords must be a numpy array or a CUDA tensor")
+    if not on_device:
+        coords = np.asarray(coords)
+    if coords.ndim != 2 or int(coords.shape[1]) != ndim:
+        raise ValueError(f"{name}: coords must have shape (K, {ndim}), got {tuple(coords.shape)}")
+    return coords, on_device, (lambda out: out) if on_device else (lambda out: out.cpu().numpy())
+
+
 class NDMPS:
     """Class for storing and compressing N-dimensional tensors using MPS (device-resident)."""
 
@@ -159,15 +174,27 @@ class NDMPS:
                 print(f"Compression ratio at {c}: {self.compression_ratio()}")
 
     # ------------------------------------------------------------------ reconstruction
+    @staticmethod
+    def _decode_box(cores, plan, lo, hi, out_shape, last_axis=None):
+        """Box [lo, hi) (lists) of the tensor ``cores`` encode in ``plan``'s layout as a CUDA tensor of ``out_shape``: K7
+        for the whole tensor, else ``contract_region``.  ``last_axis`` (the inverse DCT or its block mean) maps whole
+        lines, so the box is decoded over the full last axis, mapped and cropped to [lo[-1], hi[-1]) after."""
+        shape = list(plan.shape)
+        if last_axis is not None:
+            crop = slice(lo[-1], hi[-1])
+            lo, hi = lo[:-1] + [0], hi[:-1] + [shape[-1]]
+        if lo == [0] * len(shape) and hi == shape:
+            rec = _ops.decode(_ops.contract_dense(cores), shape, plan=plan)           # core/ndmps.py:140-148
+        else:
+            rec = _ops.contract_region(cores, shape, lo, hi, plan=plan)
+        if last_axis is not None:
+            rec = last_axis(rec)                                                      # core/ndmps.py:153
+            rec = rec[..., crop].contiguous()
+        return rec.view(out_shape)
+
     def to_tensor_device(self):
-        """Reconstruction as a CUDA tensor of the original shape (no host copy)."""
-        dense = _ops.contract_dense(self.mps.cores)                       # core/ndmps.py:140-142
-        rec = _ops.decode(dense, self._shape)                             # core/ndmps.py:144-148
-        if self.mode == "Std":
-            return rec
-        if self.mode == "DCT":
-            return _ops.dct_last_axis(rec, inverse=True)                  # core/ndmps.py:153
-        return None
+        """Reconstruction as a CUDA tensor of the original shape (no host copy): the box of the whole volume."""
+        return self.to_tensor_region_device(())
 
     def to_tensor(self) -> np.ndarray:
         """MPS back to a numpy array (with inverse DCT in "DCT" mode); any other mode
@@ -190,13 +217,8 @@ class NDMPS:
         cores = self.mps.cores
         if any(h == l for l, h in zip(lo, hi)):
             return torch.empty(out_shape, dtype=cores[0].dtype, device=cores[0].device)
-        if self.mode == "Std":
-            return _ops.contract_region(cores, self._shape, lo, hi).view(out_shape)
-        n = self._shape[-1]
-        wide = _ops.contract_region(cores, self._shape, lo[:-1] + [0], hi[:-1] + [n])
-        rec = _ops.dct_last_axis(wide, inverse=True)
-        del wide
-        return rec[..., lo[-1]:hi[-1]].contiguous().view(out_shape)
+        return self._decode_box(cores, _ops.plan_for(self._shape), lo, hi, out_shape,
+                                (lambda x: _ops.dct_last_axis(x, inverse=True)) if self.mode == "DCT" else None)
 
     def to_tensor_region(self, index):
         """``to_tensor()[index]`` as a numpy array, without reconstructing the whole tensor (see
@@ -214,14 +236,7 @@ class NDMPS:
         mode it costs one per element of its last-axis line (the inverse DCT of that line evaluated at the point).
         Any other mode returns None."""
         torch = _torch()
-        ndim = len(self._shape)
-        on_device = isinstance(coords, torch.Tensor)
-        if on_device and not coords.is_cuda:
-            raise ValueError("values_at: coords must be a numpy array or a CUDA tensor")
-        if not on_device:
-            coords = np.asarray(coords)
-        if coords.ndim != 2 or int(coords.shape[1]) != ndim:
-            raise ValueError(f"values_at: coords must have shape (K, {ndim}), got {tuple(coords.shape)}")
+        coords, on_device, result = _coords_in(coords, len(self._shape), "values_at")
         integer = (not coords.dtype.is_floating_point and not coords.dtype.is_complex and coords.dtype != torch.bool
                    if on_device else np.issubdtype(coords.dtype, np.integer))
         if not integer:
@@ -240,8 +255,7 @@ class NDMPS:
             return None
         cores = self.mps.cores
         dev = coords if on_device else torch.from_numpy(coords).to(cores[0].device)
-        out = _ops.evaluate_points(cores, self._shape, dev, idct_last_axis=self.mode == "DCT")
-        return out if on_device else out.cpu().numpy()
+        return result(_ops.evaluate_points(cores, self._shape, dev, idct_last_axis=self.mode == "DCT"))
 
     # ------------------------------------------------------------------ interpolated sampling (extension)
     def sample(self, coords):
@@ -258,14 +272,7 @@ class NDMPS:
         a few in-between frames; the workspace is the decode chains and tables of ``values_at``, nothing of the
         size of the volume.  Any other mode returns None after the arguments are checked."""
         torch = _torch()
-        ndim = len(self._shape)
-        on_device = isinstance(coords, torch.Tensor)
-        if on_device and not coords.is_cuda:
-            raise ValueError("sample: coords must be a numpy array or a CUDA tensor")
-        if not on_device:
-            coords = np.asarray(coords)
-        if coords.ndim != 2 or int(coords.shape[1]) != ndim:
-            raise ValueError(f"sample: coords must have shape (K, {ndim}), got {tuple(coords.shape)}")
+        coords, on_device, result = _coords_in(coords, len(self._shape), "sample")
         if on_device:
             real = not coords.dtype.is_complex and coords.dtype != torch.bool
         else:
@@ -284,8 +291,7 @@ class NDMPS:
             return None
         cores = self.mps.cores
         dev = coords if on_device else torch.from_numpy(coords).to(cores[0].device)
-        out = _ops.sample_points(cores, self._shape, dev, idct_last_axis=self.mode == "DCT")
-        return out if on_device else out.cpu().numpy()
+        return result(_ops.sample_points(cores, self._shape, dev, idct_last_axis=self.mode == "DCT"))
 
     def sample_grid_device(self, origin, steps, shape):
         """``sample`` at an affine grid, as a CUDA tensor of ``shape``: the value at index (i_0, .., i_{m-1}) is the
@@ -344,22 +350,11 @@ class NDMPS:
         if any(h == l for l, h in zip(lo, hi)):
             return torch.empty(out_shape, dtype=cores[0].dtype, device=cores[0].device)
         if self.mode == "Std":
-            red = _ops.marginalize(cores, self._shape, ks)
-            if lo == [0] * len(cshape) and hi == list(cshape):
-                return _ops.decode(_ops.contract_dense(red), cshape, plan=cplan).view(out_shape)
-            return _ops.contract_region(red, cshape, lo, hi, plan=cplan).view(out_shape)
+            return self._decode_box(_ops.marginalize(cores, self._shape, ks), cplan, lo, hi, out_shape)
         dks = ks[:-1] + (0,)                     # the last axis holds DCT coefficients: averaged after the inverse
-        dplan = _ops.coarse_plan(self._shape, dks)
-        red = _ops.marginalize(cores, self._shape, dks)
-        n = self._shape[-1]
-        if lo[:-1] == [0] * (len(cshape) - 1) and hi[:-1] == list(cshape[:-1]):
-            wide = _ops.decode(_ops.contract_dense(red), dplan.shape, plan=dplan)
-        else:
-            wide = _ops.contract_region(red, dplan.shape, lo[:-1] + [0], hi[:-1] + [n], plan=dplan)
-        del red
-        rec = _ops.idct_block_mean_last_axis(wide, n // cshape[-1])
-        del wide
-        return rec[..., lo[-1]:hi[-1]].contiguous().view(out_shape)
+        block = self._shape[-1] // cshape[-1]
+        return self._decode_box(_ops.marginalize(cores, self._shape, dks), _ops.coarse_plan(self._shape, dks), lo, hi,
+                                out_shape, lambda x: _ops.idct_block_mean_last_axis(x, block))
 
     def to_tensor_coarse(self, levels, index=None):
         """``to_tensor_coarse_device(levels, index)`` as a numpy array; None for a mode other than "Std" / "DCT"."""

@@ -7,7 +7,8 @@ Workloads:
     values_at with 10^4 and 10^6 random points (CUDA coordinates);
   config 5-B - one (1920, 1080, 64) float32 DCT video chunk (bench.synthetic_video) at chi = 64:
     to_tensor_device(), one frame (last axis an int: decoded over all 64 frames, then inverse DCT, then cropped),
-    a 256 x 256 spatial crop (all 64 frames).
+    a 256 x 256 spatial crop (all 64 frames), values_at with 10^4 and 10^6 random points (CUDA coordinates; each
+    point sums the 64 coefficients of its line).
 Each call is warmed up, then timed with CUDA events around `--reps` calls (median and min reported), and its output
 is compared with the same part of the full reconstruction.  Peak torch allocation per call and the library's
 workspace high-water mark are recorded beside the times, with the card's name and power limit.
@@ -16,7 +17,6 @@ workspace high-water mark are recorded beside the times, with the card's name an
 """
 import argparse
 import json
-import subprocess
 import sys
 from pathlib import Path
 
@@ -29,44 +29,20 @@ for p in (str(ROOT), str(ROOT / "img-compression-mps_b200")):
         sys.path.insert(0, p)
 from bench import synthetic_video, synthetic_volume     # noqa: E402
 from imgcompressionmps.core.ndmps import NDMPS          # noqa: E402
-
-
-def card():
-    info = {"name": torch.cuda.get_device_name(0)}
-    try:
-        q = subprocess.run(["nvidia-smi", "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader", "-i", "0"],
-                           capture_output=True, text=True, timeout=30)
-        info["power_limit_and_max_sm_clock"] = q.stdout.strip()
-    except (OSError, subprocess.SubprocessError) as exc:
-        info["power_limit_and_max_sm_clock"] = f"unavailable: {exc}"
-    return info
-
-
-def timed(fn, reps, warmup):
-    for _ in range(warmup):
-        fn()
-    torch.cuda.synchronize()
-    ms = []
-    for _ in range(reps):
-        s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        s.record()
-        fn()
-        e.record()
-        e.synchronize()
-        ms.append(s.elapsed_time(e))
-    torch.cuda.reset_peak_memory_stats()
-    base = torch.cuda.memory_allocated()
-    out = fn()
-    torch.cuda.synchronize()
-    peak = torch.cuda.max_memory_allocated() - base
-    return out, {"median_ms": float(np.median(ms)), "min_ms": float(np.min(ms)), "reps": reps,
-                 "peak_torch_alloc_MB": peak / 2 ** 20}
+from probe_timing import card, timed                    # noqa: E402
 
 
 def rel_err(got, want):
     got = got if isinstance(got, torch.Tensor) else torch.as_tensor(got)
     got = got.to(want.device, torch.float64)
     return float((got - want.double()).abs().max() / want.double().abs().max())
+
+
+def random_points(shape, seed):
+    """10^4 and 10^6 seeded random points of a volume of ``shape``, as CUDA int64 (K, ndim) tensors."""
+    rng = np.random.default_rng(seed)
+    return {k: torch.as_tensor(np.stack([rng.integers(0, n, size=k) for n in shape], axis=1), device="cuda")
+            for k in (10 ** 4, 10 ** 6)}
 
 
 def probe(obj, full, items, reps, warmup):
@@ -100,9 +76,7 @@ def main():
     del vol
     full = obj.to_tensor_device()
     z, c = n // 2, n // 4
-    rng = np.random.default_rng(5)
-    pts = {k: torch.as_tensor(np.stack([rng.integers(0, n, size=k) for _ in range(3)], axis=1), device="cuda")
-           for k in (10 ** 4, 10 ** 6)}
+    pts = random_points((n, n, n), 5)
     items = [
         ("to_tensor_device()", obj.to_tensor_device, None),
         ("to_tensor()[z]", lambda: obj.to_tensor()[z], lambda: full[z]),
@@ -127,12 +101,13 @@ def main():
         full = obj.to_tensor_device()
         f = shape[2] // 3
         x0, y0 = shape[0] // 2 - 128, shape[1] // 2 - 128
+        pts = random_points(shape, 6)
         items = [
             ("to_tensor_device()", obj.to_tensor_device, None),
             ("region (..., f) one frame", lambda: obj.to_tensor_region_device((Ellipsis, f)), lambda: full[..., f]),
             ("region 256x256 crop, all frames", lambda: obj.to_tensor_region_device((slice(x0, x0 + 256), slice(y0, y0 + 256))),
              lambda: full[x0:x0 + 256, y0:y0 + 256]),
-        ]
+        ] + [(f"values_at {k} points", lambda k=k: obj.values_at(pts[k]), lambda k=k: full[tuple(pts[k].T)]) for k in pts]
         report["config5b"] = {"shape": list(shape), "chi": 64, "mode": "DCT", "bonds": obj.bond_sizes(),
                               "rows": probe(obj, full, items, args.reps, args.warmup)}
     report["workspace_high_water_MB"] = _native.context().stat("workspace_bytes") / 2 ** 20
