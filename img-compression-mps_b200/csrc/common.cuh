@@ -130,6 +130,22 @@ struct Arena {
         *out = static_cast<T*>(p);
         return rc;
     }
+    // Hand back everything allocated since mark() without a reset, so that a loop over blocks reuses one block's
+    // workspace (stream order makes the reuse safe: a later allocation is written by work enqueued after the last
+    // reader of the earlier one).  The high-water mark keeps the peak; cached pointers of the old generation die.
+    struct Mark { std::vector<size_t> used; size_t total = 0; };
+    Mark mark() const {
+        Mark m;
+        for (const auto& c : chunks) m.used.push_back(c.used);
+        m.total = cur_total;
+        return m;
+    }
+    void rewind(const Mark& m) {
+        if (cur_total > high_water) high_water = cur_total;
+        for (size_t i = 0; i < chunks.size(); i++) chunks[i].used = i < m.used.size() ? m.used[i] : 0;
+        cur_total = m.total;
+        generation++;
+    }
 };
 
 }  // namespace ndmps
@@ -269,6 +285,10 @@ int left_chain(ndmps_ctx* ctx, const void* const* cores, int dtype, int s, const
 int right_chain(ndmps_ctx* ctx, const void* const* cores, int dtype, int L, int s, const int64_t* dims, const int64_t* ranks,
                 const GatherArgs* gathers, const void** W_out, int64_t* cols_out);
 int chain_product(ndmps_ctx* ctx, int64_t rows, int64_t cols, int64_t r, const void* X, const void* W, int dtype, void* out);
+// the transform of ndmps_dct_last_axis (dct.cu) in two steps on workspace the caller has reset: dct_matrix puts the
+// n x n cosine matrix of one direction in the workspace, dct_lines applies it to `lines` lines of length n
+int dct_matrix(ndmps_ctx* ctx, int64_t n, int inverse, double** C_out);
+int dct_lines(ndmps_ctx* ctx, const void* src, void* dst, int64_t lines, int64_t n, int dtype, const double* C);
 
 #ifdef __CUDACC__
 __device__ __forceinline__ double warp_sum(double v) {

@@ -36,6 +36,28 @@ __global__ void __launch_bounds__(256) dct_block_mean_matrix_kernel(double* __re
     }
 }
 
+int dct_matrix(ndmps_ctx* ctx, int64_t n, int inverse, double** C_out) {
+    double* C = nullptr;
+    NDMPS_TRY(ctx->ws.get<double>((size_t)(n * n), &C));
+    int64_t want = (n * n + 255) / 256, cap = (int64_t)ctx->sm_count * 8;
+    dct_matrix_kernel<<<(int)(want < cap ? want : cap), 256, 0, ctx->stream>>>(C, n, inverse ? 0 : 1);
+    NDMPS_LAUNCH_CHECK(ctx);
+    *C_out = C;
+    return NDMPS_OK;
+}
+
+// forward: y[l, k] = sum_i x[l, i] C[k, i] = sum_i x[l, i] Ct[i, k]; inverse: x[l, i] = sum_k y[l, k] C[k, i].  Both are
+// dst = src . C with the matrix dct_matrix built for the direction.
+int dct_lines(ndmps_ctx* ctx, const void* src, void* dst, int64_t lines, int64_t n, int dtype, const double* C) {
+    if (ctx->opt_tc && dtype == NDMPS_F32 && lines * n >= (int64_t(1) << 20)) {
+        // float32 payload: the line x cosine-matrix product on tcgen05 (bf16x3 planes, tc_gemm.cu)
+        bool on_tc = false;
+        NDMPS_TRY(gemm_tc(ctx, lines, n, n, 1.0, src, dtype, n, 1, C, NDMPS_F64, n, 1, dst, dtype, n, false, &on_tc));
+        if (on_tc) return NDMPS_OK;
+    }
+    return gemm(ctx, lines, n, n, 1.0, src, dtype, n, 1, C, NDMPS_F64, n, 1, dst, dtype, n);
+}
+
 }  // namespace ndmps
 
 using namespace ndmps;
@@ -50,21 +72,8 @@ int ndmps_dct_last_axis(ndmps_ctx_t* ctx, const void* src, void* dst, int64_t li
     NDMPS_TRY(ctx->ws.reset(ctx->stream));
     StageScope sc(ctx, ST_DCT);
     double* C = nullptr;
-    NDMPS_TRY(ctx->ws.get<double>((size_t)(n * n), &C));
-    int64_t want = (n * n + 255) / 256, cap = (int64_t)ctx->sm_count * 8;
-    dct_matrix_kernel<<<(int)(want < cap ? want : cap), 256, 0, ctx->stream>>>(C, n, inverse ? 0 : 1);
-    NDMPS_LAUNCH_CHECK(ctx);
-    if (ctx->opt_tc && dtype == NDMPS_F32 && lines * n >= (int64_t(1) << 20)) {
-        // float32 payload: the line x cosine-matrix product on tcgen05 (bf16x3 planes, tc_gemm.cu); both directions are
-        // dst = src . C with the matrix the kernel above built for the direction
-        bool on_tc = false;
-        NDMPS_TRY(gemm_tc(ctx, lines, n, n, 1.0, src, dtype, n, 1, C, NDMPS_F64, n, 1, dst, dtype, n, false, &on_tc));
-        if (on_tc) return NDMPS_OK;
-    }
-    if (!inverse)   // y[l, k] = sum_i x[l, i] C[k, i] = sum_i x[l, i] Ct[i, k]
-        return gemm(ctx, lines, n, n, 1.0, src, dtype, n, 1, C, NDMPS_F64, n, 1, dst, dtype, n);
-    // x[l, i] = sum_k y[l, k] C[k, i]
-    return gemm(ctx, lines, n, n, 1.0, src, dtype, n, 1, C, NDMPS_F64, n, 1, dst, dtype, n);
+    NDMPS_TRY(dct_matrix(ctx, n, inverse, &C));
+    return dct_lines(ctx, src, dst, lines, n, dtype, C);
 }
 
 int ndmps_idct_block_mean_last_axis(ndmps_ctx_t* ctx, const void* src, void* dst, int64_t lines, int64_t n, int64_t block, int dtype) {

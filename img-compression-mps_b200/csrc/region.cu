@@ -18,6 +18,10 @@
 //   3. out[x] = T[iH(x), iC(x)] in volume order, one more gather_sum.
 // The workspace holds T, the restricted chains and the tables - nothing of the size of the volume.
 //
+// Projection path (ndmps_project_region): steps 1 and 2 of the region path, with T computed in row blocks of at most
+// 16 MB (whole axis-0 high parts), each reduced (max / min along one axis) into the output by project_reduce_kernel
+// as soon as it is written instead of being gathered into the box; the workspace holds one block at a time.
+//
 // Point path (ndmps_evaluate_points, ndmps_sample_points, ndmps_sample_grid): one kernel over three coordinate sources
 // (integer points, a list of real coordinates, an affine grid) on the full chains X (P_s x r) and W (r x Q_s) of
 // contract_dense, W transposed so that the column of a point is one contiguous bond vector; a warp works out the
@@ -272,6 +276,70 @@ sample_points_kernel(const T* __restrict__ X, const T* __restrict__ Wt, Src src,
     }
 }
 
+// max / min that propagate NaN as numpy's do (fmax / fmin drop it): a NaN on either side wins
+template <int OP, class T>
+__device__ __forceinline__ T proj_op(T a, T b) {
+    if (OP == NDMPS_PROJ_MAX) return (a != a || a > b) ? a : b;
+    return (a != a || a < b) ? a : b;
+}
+
+struct ProjectArgs {
+    int n = 0;                         // axes of the block
+    int ax = 0;                        // the projected one
+    int store = 1;                     // 0: combine with what out holds (axis 0 projected, a block after the first)
+    int64_t ext[8] = {0};
+    const int64_t* tab[8] = {nullptr}; // per-axis source offsets: the element at (i_0, ..) is src[sum_a tab[a][i_a]]
+    int64_t count = 0;                 // output elements: the product of ext over every axis but ax
+};
+
+// out[o] = OP over i_ax of src[sum_a tab[a][i_a]], o the C-order index over the other axes.  ax below the innermost
+// axis: a thread per output element, consecutive threads along the innermost axis; ax the innermost: a warp per output
+// element, lanes strided along the line and a shuffle reduction.
+template <class T, int OP>
+__global__ void __launch_bounds__(256)
+project_reduce_kernel(const T* __restrict__ src, T* __restrict__ out, ProjectArgs pa) {
+    const T ident = OP == NDMPS_PROJ_MAX ? (T)-INFINITY : (T)INFINITY;
+    const int64_t* tp = nullptr;
+    int64_t ne = 1;
+#pragma unroll
+    for (int a = 0; a < 8; a++)
+        if (a == pa.ax) { tp = pa.tab[a]; ne = pa.ext[a]; }
+    const bool per_warp = pa.ax == pa.n - 1;
+    const int lane = threadIdx.x & 31;
+    const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t step = per_warp ? ((int64_t)gridDim.x * blockDim.x) >> 5 : (int64_t)gridDim.x * blockDim.x;
+    for (int64_t o = per_warp ? gid >> 5 : gid; o < pa.count; o += step) {
+        int64_t rem = o, base = 0;
+#pragma unroll
+        for (int a = 7; a >= 0; a--)
+            if (a < pa.n && a != pa.ax) {
+                const int64_t q = rem / pa.ext[a];
+                base += pa.tab[a][rem - q * pa.ext[a]];
+                rem = q;
+            }
+        T v = ident;
+        if (per_warp) {
+            for (int64_t j = lane; j < ne; j += 32) v = proj_op<OP>(v, src[base + tp[j]]);
+#pragma unroll
+            for (int d = 16; d > 0; d >>= 1) v = proj_op<OP>(v, __shfl_xor_sync(0xffffffffu, v, d));
+            if (lane != 0) continue;
+        } else {
+            // four independent chains keep four loads in flight; max and min are exact, so the order is free
+            T v1 = ident, v2 = ident, v3 = ident;
+            int64_t j = 0;
+            for (; j + 4 <= ne; j += 4) {
+                v = proj_op<OP>(v, src[base + tp[j]]);
+                v1 = proj_op<OP>(v1, src[base + tp[j + 1]]);
+                v2 = proj_op<OP>(v2, src[base + tp[j + 2]]);
+                v3 = proj_op<OP>(v3, src[base + tp[j + 3]]);
+            }
+            for (; j < ne; j++) v = proj_op<OP>(v, src[base + tp[j]]);
+            v = proj_op<OP>(proj_op<OP>(v, v1), proj_op<OP>(v2, v3));
+        }
+        out[o] = pa.store ? v : proj_op<OP>(out[o], v);
+    }
+}
+
 static int warp_grid(const ndmps_ctx* ctx, int64_t warps, int warps_per_block = 8) {
     int64_t want = (warps + warps_per_block - 1) / warps_per_block, cap = (int64_t)ctx->sm_count * 16 * (8 / warps_per_block);
     if (want < 1) want = 1;
@@ -454,6 +522,117 @@ GatherArgs level_args(const Level& lv, const int64_t* tabs_dev, int64_t row) {
     return g;
 }
 
+// A projection decodes its box in blocks of T = X_H W_C that stay small (in L2 once written): a block is a range of
+// whole axis-0 high parts, i.e. a contiguous range of rows of X_H, and covers a contiguous range of the box's axis-0
+// positions.  The block's source is addressed by rp.tabs from one more Level, `src` (the box tables of the region path
+// with each axis-0 entry taken relative to its own block; for L = 1 the core offsets of rp.left[0]).  In DCT mode the
+// box covers the whole last axis and every block is gathered to volume order, transformed and reduced through the
+// Level `vol` (volume-order offsets in the block, the last axis starting at the caller's lo[-1]).
+constexpr int64_t PROJECT_BLOCK_BYTES = int64_t(16) << 20;
+
+struct ProjectBlock {
+    int64_t row0 = 0, rows = 0;        // rows of X_H
+    int64_t i0 = 0, n0 = 0;            // box positions along axis 0
+};
+
+struct ProjectPlan {
+    RegionPlan rp;                     // of the box widened to the whole last axis in DCT mode
+    Level src, vol;
+    std::vector<ProjectBlock> blocks;
+};
+
+// lo / hi: the caller's non-empty box; block_elems: the bound on the elements of a block of T
+void plan_project(const ndmps_plan* p, const int64_t* lo, const int64_t* hi, int idct, int64_t block_elems, ProjectPlan& pp) {
+    const int n = p->ndim, L = p->levels;
+    std::vector<int64_t> wlo(lo, lo + n), whi(hi, hi + n), nb((size_t)n);
+    if (idct) { wlo[(size_t)n - 1] = 0; whi[(size_t)n - 1] = p->shape[n - 1]; }
+    for (int a = 0; a < n; a++) nb[(size_t)a] = whi[(size_t)a] - wlo[(size_t)a];
+    RegionPlan& rp = pp.rp;
+    plan_region(p, wlo.data(), whi.data(), rp);
+    // blocks: high parts of axis 0 at the split (whole lines when axis 0 is the DCT axis, and the one core for L = 1)
+    std::vector<int64_t> pw, fs;
+    digit_products(p, pw, fs);
+    const int64_t g0 = pw[(size_t)(rp.s * n)], h_lo = wlo[0] / g0, nh = (whi[0] - 1) / g0 - h_lo + 1;
+    const int64_t per_h = rp.H / nh;   // rows of X_H in one axis-0 high part
+    int64_t hb = block_elems / (per_h * rp.C);
+    if (hb < 1) hb = 1;
+    if (L == 1 || (idct && n == 1)) hb = nh;
+    for (int64_t h = 0; h < nh; h += hb) {
+        ProjectBlock b;
+        const int64_t h1 = h + hb < nh ? h + hb : nh;
+        b.row0 = h * per_h;
+        b.rows = (h1 - h) * per_h;
+        const int64_t x0 = (h_lo + h) * g0 > wlo[0] ? (h_lo + h) * g0 : wlo[0], x1 = (h_lo + h1) * g0 < whi[0] ? (h_lo + h1) * g0 : whi[0];
+        b.i0 = x0 - wlo[0];
+        b.n0 = x1 - x0;
+        pp.blocks.push_back(b);
+    }
+    // src: the region path's box tables, or the core offsets of a single core; axis 0 relative to its block
+    const Level& from = L == 1 ? rp.left[0] : rp.box;
+    pp.src = add_level(rp, n, nb.data());
+    for (int a = 0; a < n; a++)
+        for (int64_t i = 0; i < nb[(size_t)a]; i++) rp.tabs[(size_t)(pp.src.off[a] + i)] = rp.tabs[(size_t)(from.off[a] + i)];
+    for (const ProjectBlock& b : pp.blocks)
+        for (int64_t i = b.i0; i < b.i0 + b.n0; i++) rp.tabs[(size_t)(pp.src.off[0] + i)] -= b.row0 * rp.C;
+    if (!idct) return;
+    // vol: volume order in the block's gathered lines (extents nb, axis 0 the block's), the caller's box on the last axis
+    std::vector<int64_t> ob((size_t)n);
+    for (int a = 0; a < n; a++) ob[(size_t)a] = hi[a] - lo[a];
+    pp.vol = add_level(rp, n, ob.data());
+    int64_t stride = 1;
+    for (int a = n - 1; a >= 0; a--) {
+        int64_t* t = rp.tabs.data() + pp.vol.off[a];
+        for (int64_t i = 0; i < ob[(size_t)a]; i++) t[i] = (a == n - 1 ? lo[a] - wlo[(size_t)a] + i : i) * stride;
+        stride *= nb[(size_t)a];
+    }
+    if (n == 1) return;                // one block, the whole line
+    for (const ProjectBlock& b : pp.blocks)
+        for (int64_t i = b.i0; i < b.i0 + b.n0; i++) rp.tabs[(size_t)(pp.vol.off[0] + i)] -= b.i0 * (stride / nb[0]);
+}
+
+// site-order prefix of every kept row (rowH) and suffix of every kept column (colC) of T, and Q = Q_s, the columns of
+// the full product: the flat site-order index of T[i, c] is rowH[i] * Q + colC[c]
+void region_sites(const ndmps_plan* plan, const RegionPlan& rp, std::vector<int64_t>& rowH, std::vector<int64_t>& colC,
+                  int64_t* Q_out) {
+    // level by level: row (parent, digit) of the gathered product
+    std::vector<int64_t> prev(1, 0), cur;
+    for (int l = 0; l < rp.s; l++) {
+        const int64_t d = plan->site_dims[l];
+        cur.assign((size_t)rp.left[(size_t)l].count(), 0);
+        walk(rp, rp.left[(size_t)l], [&](int64_t j, int64_t q) { cur[(size_t)j] = prev[(size_t)(q / d)] * d + q % d; });
+        prev.swap(cur);
+    }
+    rowH = prev;
+    // column (digit, child) of the gathered product
+    prev.assign(1, 0);
+    int64_t Q = 1;
+    for (int k = plan->levels - 1; k >= rp.s; k--) {
+        const int64_t mc = rp.m[(size_t)k + 1];
+        cur.assign((size_t)rp.m[(size_t)k], 0);
+        walk(rp, rp.right[(size_t)k], [&](int64_t j, int64_t q) { cur[(size_t)j] = (q / mc) * Q + prev[(size_t)(q % mc)]; });
+        prev.swap(cur);
+        Q *= plan->site_dims[k];
+    }
+    colC = prev;
+    *Q_out = Q;
+}
+
+// a Level restricted to one block: axis 0 is the block's range of positions
+Level block_level(const Level& lv, const ProjectBlock& b) {
+    Level r = lv;
+    r.ext[0] = b.n0;
+    r.off[0] += b.i0;
+    return r;
+}
+
+// the source of block b's reduction, the level the device path and ndmps_project_debug_offsets both read: src restricted
+// to the block, or in DCT mode vol restricted to it - except for a 1-D box, whose one block is the whole widened line
+// while vol is the caller's range of it, so vol is read as it stands
+Level reduce_level(const ProjectPlan& pp, int idct, const ProjectBlock& b) {
+    if (!idct) return block_level(pp.src, b);
+    return pp.vol.n == 1 ? pp.vol : block_level(pp.vol, b);
+}
+
 }  // namespace
 
 int upload_tables(ndmps_ctx* ctx, const std::vector<int64_t>& tabs, int64_t** out) {
@@ -471,23 +650,22 @@ int check_mps(const char* fn, const ndmps_plan* plan, const void* const* cores, 
     return NDMPS_OK;
 }
 
-static int contract_region(ndmps_ctx* ctx, const ndmps_plan* p, const void* const* cores, int dtype, const int64_t* ranks,
-                           const int64_t* lo, const int64_t* hi, void* out) {
-    const int L = p->levels, n = p->ndim;
-    const size_t esz = dtype_size(dtype);
-    RegionPlan rp;
-    plan_region(p, lo, hi, rp);
-    // the left bond of every right-chain level as the gather's outer axis: a -> a * (d_k * m[k+1])
-    std::vector<int64_t> bond_off((size_t)L, 0);
-    for (int k = rp.s; k < L; k++) {
+// the left bond of every right-chain level as the gather's outer axis, a -> a * (d_k * m[k+1]), appended to rp.tabs:
+// bond_off[k] (k >= s) is where level k's table starts
+static std::vector<int64_t> add_bond_tables(const ndmps_plan* p, const int64_t* ranks, RegionPlan& rp) {
+    std::vector<int64_t> bond_off((size_t)p->levels, 0);
+    for (int k = rp.s; k < p->levels; k++) {
         bond_off[(size_t)k] = (int64_t)rp.tabs.size();
         for (int64_t a = 0; a < ranks[k - 1]; a++) rp.tabs.push_back(a * p->site_dims[k] * rp.m[(size_t)k + 1]);
     }
-    int64_t* tabs = nullptr;
-    NDMPS_TRY(upload_tables(ctx, rp.tabs, &tabs));
-    StageScope sc(ctx, ST_CONTRACT);
-    if (L == 1)   // H is the box itself, in C order
-        return gather_sum(ctx, cores[0], out, dtype, level_args(rp.left[0], tabs, 1));
+    return bond_off;
+}
+
+// X_H (|H| x r) and W_C (r x |C|) of a planned box (L > 1), its tables uploaded to `tabs`
+static int region_chains(ndmps_ctx* ctx, const ndmps_plan* p, const void* const* cores, int dtype, const int64_t* ranks,
+                         const RegionPlan& rp, const int64_t* tabs, const std::vector<int64_t>& bond_off, const void** X,
+                         const void** W) {
+    const int L = p->levels, n = p->ndim;
     std::vector<GatherArgs> gl((size_t)rp.s), gr((size_t)L);
     for (int l = 0; l < rp.s; l++) gl[(size_t)l] = level_args(rp.left[(size_t)l], tabs, ranks[l]);
     for (int k = rp.s; k < L; k++) {
@@ -498,14 +676,103 @@ static int contract_region(ndmps_ctx* ctx, const ndmps_plan* p, const void* cons
         g.tab[0] = tabs + bond_off[(size_t)k];
         for (int a = 0; a < n; a++) { g.ext[a + 1] = lv.ext[a]; g.tab[a + 1] = tabs + lv.off[a]; }
     }
-    const void *X = nullptr, *W = nullptr;
     int64_t rows = 0, cols = 0;
-    NDMPS_TRY(left_chain(ctx, cores, dtype, rp.s, p->site_dims, ranks, gl.data(), &X, &rows));
-    NDMPS_TRY(right_chain(ctx, cores, dtype, L, rp.s, p->site_dims, ranks, gr.data(), &W, &cols));
+    NDMPS_TRY(left_chain(ctx, cores, dtype, rp.s, p->site_dims, ranks, gl.data(), X, &rows));
+    return right_chain(ctx, cores, dtype, L, rp.s, p->site_dims, ranks, gr.data(), W, &cols);
+}
+
+static int contract_region(ndmps_ctx* ctx, const ndmps_plan* p, const void* const* cores, int dtype, const int64_t* ranks,
+                           const int64_t* lo, const int64_t* hi, void* out) {
+    const int L = p->levels;
+    const size_t esz = dtype_size(dtype);
+    RegionPlan rp;
+    plan_region(p, lo, hi, rp);
+    const std::vector<int64_t> bond_off = add_bond_tables(p, ranks, rp);
+    int64_t* tabs = nullptr;
+    NDMPS_TRY(upload_tables(ctx, rp.tabs, &tabs));
+    StageScope sc(ctx, ST_CONTRACT);
+    if (L == 1)   // H is the box itself, in C order
+        return gather_sum(ctx, cores[0], out, dtype, level_args(rp.left[0], tabs, 1));
+    const void *X = nullptr, *W = nullptr;
+    NDMPS_TRY(region_chains(ctx, p, cores, dtype, ranks, rp, tabs, bond_off, &X, &W));
     void* T = nullptr;
-    NDMPS_TRY(ctx->ws.alloc((size_t)(rows * cols) * esz, &T));
-    NDMPS_TRY(chain_product(ctx, rows, cols, ranks[rp.s - 1], X, W, dtype, T));
+    NDMPS_TRY(ctx->ws.alloc((size_t)(rp.H * rp.C) * esz, &T));
+    NDMPS_TRY(chain_product(ctx, rp.H, rp.C, ranks[rp.s - 1], X, W, dtype, T));
     return gather_sum(ctx, T, out, dtype, level_args(rp.box, tabs, 1));
+}
+
+template <class T>
+static int launch_project(ndmps_ctx* ctx, const void* src, void* out, const GatherArgs& g, int ax, int op, int store) {
+    ProjectArgs pa;
+    pa.n = g.n;
+    pa.ax = ax;
+    pa.store = store;
+    pa.count = 1;
+    for (int a = 0; a < g.n; a++) {
+        pa.ext[a] = g.ext[a];
+        pa.tab[a] = g.tab[a];
+        if (a != ax) pa.count *= g.ext[a];
+    }
+    const int grid = ax == g.n - 1 ? warp_grid(ctx, pa.count) : warp_grid(ctx, (pa.count + 31) / 32);
+    if (op == NDMPS_PROJ_MAX)
+        project_reduce_kernel<T, NDMPS_PROJ_MAX><<<grid, 256, 0, ctx->stream>>>((const T*)src, (T*)out, pa);
+    else
+        project_reduce_kernel<T, NDMPS_PROJ_MIN><<<grid, 256, 0, ctx->stream>>>((const T*)src, (T*)out, pa);
+    NDMPS_LAUNCH_CHECK(ctx);
+    return NDMPS_OK;
+}
+
+// op over volume axis `ax` of the box [lo, hi) into out (C order over the other axes), a block of T at a time
+static int project_region(ndmps_ctx* ctx, const ndmps_plan* p, const void* const* cores, int dtype, const int64_t* ranks,
+                          const int64_t* lo, const int64_t* hi, int ax, int op, int idct, void* out) {
+    const int L = p->levels, n = p->ndim;
+    const size_t esz = dtype_size(dtype);
+    ProjectPlan pp;
+    plan_project(p, lo, hi, idct, PROJECT_BLOCK_BYTES / (int64_t)esz, pp);
+    const RegionPlan& rp = pp.rp;
+    const std::vector<int64_t> bond_off = add_bond_tables(p, ranks, pp.rp);
+    int64_t* tabs = nullptr;
+    NDMPS_TRY(upload_tables(ctx, rp.tabs, &tabs));
+    StageScope sc(ctx, ST_CONTRACT);
+    const void *X = nullptr, *W = nullptr;
+    if (L > 1) NDMPS_TRY(region_chains(ctx, p, cores, dtype, ranks, rp, tabs, bond_off, &X, &W));
+    const int64_t nl = p->shape[n - 1];
+    double* C = nullptr;
+    if (idct) NDMPS_TRY(dct_matrix(ctx, nl, 1, &C));
+    // output elements before a block's first axis-0 position (axis 0 projected: every block reduces into all of out)
+    int64_t out_per_i0 = 1;
+    for (int a = 1; a < n; a++)
+        if (a != ax) out_per_i0 *= hi[a] - lo[a];
+    const Arena::Mark mk = ctx->ws.mark();
+    for (size_t k = 0; k < pp.blocks.size(); k++) {
+        const ProjectBlock& b = pp.blocks[k];
+        const void* S = cores[0];      // L = 1: the core is the volume in C order
+        if (L > 1) {
+            void* T = nullptr;
+            NDMPS_TRY(ctx->ws.alloc((size_t)(b.rows * rp.C) * esz, &T));
+            NDMPS_TRY(chain_product(ctx, b.rows, rp.C, ranks[rp.s - 1], (const char*)X + (size_t)(b.row0 * ranks[rp.s - 1]) * esz, W,
+                                    dtype, T));
+            S = T;
+        }
+        if (idct) {                    // whole lines to volume order, inverse DCT, then reduced through vol
+            const GatherArgs g = level_args(block_level(pp.src, b), tabs, 1);
+            int64_t count = 1;
+            for (int a = 0; a < n; a++) count *= g.ext[a];
+            void *V = nullptr, *Y = nullptr;
+            NDMPS_TRY(ctx->ws.alloc((size_t)count * esz, &V));
+            NDMPS_TRY(ctx->ws.alloc((size_t)count * esz, &Y));
+            NDMPS_TRY(gather_sum(ctx, S, V, dtype, g));
+            NDMPS_TRY(dct_lines(ctx, V, Y, count / nl, nl, dtype, C));
+            S = Y;
+        }
+        const GatherArgs r = level_args(reduce_level(pp, idct, b), tabs, 1);
+        void* o = ax == 0 ? out : (char*)out + (size_t)(b.i0 * out_per_i0) * esz;
+        const int store = ax != 0 || k == 0;
+        if (dtype == NDMPS_F32) NDMPS_TRY(launch_project<float>(ctx, S, o, r, ax, op, store));
+        else NDMPS_TRY(launch_project<double>(ctx, S, o, r, ax, op, store));
+        ctx->ws.rewind(mk);
+    }
+    return NDMPS_OK;
 }
 
 // Set-up shared by the point and sampling paths: the per-axis row / column tables (uploaded in one copy), the full
@@ -619,6 +886,76 @@ int ndmps_contract_region(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void
     return contract_region(ctx, plan, cores, dtype, ranks, lo, hi, out);
 }
 
+// the checks ndmps_project_region and its debug twin share; *empty: an empty extent on an axis other than `axis`
+static int check_projection(const char* fn, const ndmps_plan* plan, const int64_t* lo, const int64_t* hi, int axis, bool* empty) {
+    NDMPS_TRY(check_box(plan, lo, hi, empty));
+    NDMPS_REQUIRE(axis >= 0 && axis < plan->ndim, "%s: axis %d outside 0..%d", fn, axis, plan->ndim - 1);
+    NDMPS_REQUIRE(hi[axis] > lo[axis], "%s: the box is empty along the projected axis %d", fn, axis);
+    return NDMPS_OK;
+}
+
+int ndmps_project_region(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void* const* cores, int dtype, const int64_t* ranks,
+                         const int64_t* lo, const int64_t* hi, int axis, int op, int idct_last_axis, void* out) {
+    NDMPS_REQUIRE(ctx && plan && cores && lo && hi, "ndmps_project_region: NULL argument");
+    NDMPS_TRY(check_mps("ndmps_project_region", plan, cores, dtype, ranks));
+    NDMPS_REQUIRE(op == NDMPS_PROJ_MAX || op == NDMPS_PROJ_MIN, "ndmps_project_region: op %d is not max or min", op);
+    bool empty = false;
+    NDMPS_TRY(check_projection("ndmps_project_region", plan, lo, hi, axis, &empty));
+    if (empty) return NDMPS_OK;
+    NDMPS_REQUIRE(out, "ndmps_project_region: out is NULL");
+    NDMPS_TRY(ctx->ws.reset(ctx->stream));
+    return project_region(ctx, plan, cores, dtype, ranks, lo, hi, axis, op, idct_last_axis ? 1 : 0, out);
+}
+
+int ndmps_project_debug_offsets(const ndmps_plan_t* plan, const int64_t* lo, const int64_t* hi, int axis, int64_t block_elems,
+                                int64_t* info_out, int64_t* offsets_out_host) {
+    NDMPS_REQUIRE(plan && lo && hi && info_out, "ndmps_project_debug_offsets: NULL argument");
+    NDMPS_REQUIRE(block_elems >= 1, "ndmps_project_debug_offsets: block_elems %lld", (long long)block_elems);
+    bool empty = false;
+    NDMPS_TRY(check_projection("ndmps_project_debug_offsets", plan, lo, hi, axis, &empty));
+    info_out[0] = split_of(plan);
+    info_out[1] = info_out[2] = info_out[3] = 0;
+    if (empty) return NDMPS_OK;
+    NDMPS_REQUIRE(offsets_out_host, "ndmps_project_debug_offsets: NULL argument");
+    const int n = plan->ndim;
+    ProjectPlan pp;
+    plan_project(plan, lo, hi, 0, block_elems, pp);
+    const RegionPlan& rp = pp.rp;
+    // compact row / column of T -> site-order prefix / suffix, as ndmps_region_debug_offsets derives them
+    std::vector<int64_t> rowH, colC;
+    int64_t Q = 1;
+    region_sites(plan, rp, rowH, colC, &Q);
+    const int64_t e = hi[axis] - lo[axis];
+    int64_t count = 1;
+    for (int a = 0; a < n; a++)
+        if (a != axis) count *= hi[a] - lo[a];
+    int64_t* block_of = offsets_out_host + count * e;   // -1: read by no block, -2: by more than one
+    for (int64_t i = 0; i < count * e; i++) block_of[i] = -1;
+    for (size_t k = 0; k < pp.blocks.size(); k++) {
+        const ProjectBlock& b = pp.blocks[k];
+        const Level lv = reduce_level(pp, 0, b);
+        int64_t per_i0 = 1;            // output elements and positions before the block's first axis-0 position
+        for (int a = 1; a < n; a++) per_i0 *= hi[a] - lo[a];
+        walk(rp, lv, [&](int64_t j, int64_t q) {
+            // j: C-order index in the block -> (output element, position along axis) of the whole box
+            int64_t rem = j + b.i0 * per_i0, o = 0, ostride = 1, pos = 0;
+            for (int a = n - 1; a >= 0; a--) {
+                const int64_t ext = hi[a] - lo[a], i = rem % ext;
+                rem /= ext;
+                if (a == axis) pos = i;
+                else { o += i * ostride; ostride *= ext; }
+            }
+            const int64_t t = b.row0 * rp.C + q;   // the element of the whole T the block's element is
+            offsets_out_host[o * e + pos] = plan->levels == 1 ? q : rowH[(size_t)(t / rp.C)] * Q + colC[(size_t)(t % rp.C)];
+            block_of[o * e + pos] = block_of[o * e + pos] == -1 ? (int64_t)k : -2;
+        });
+    }
+    info_out[1] = rp.H;
+    info_out[2] = rp.C;
+    info_out[3] = (int64_t)pp.blocks.size();
+    return NDMPS_OK;
+}
+
 int ndmps_evaluate_points(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void* const* cores, int dtype, const int64_t* ranks,
                           const int64_t* coords_dev, int64_t count, int idct_last_axis, void* out_dev) {
     NDMPS_REQUIRE(ctx && plan && cores && (count == 0 || (coords_dev && out_dev)), "ndmps_evaluate_points: NULL argument");
@@ -682,29 +1019,11 @@ int ndmps_region_debug_offsets(const ndmps_plan_t* plan, const int64_t* lo, cons
     info_out[1] = info_out[2] = 0;
     if (empty) return NDMPS_OK;
     NDMPS_REQUIRE(site_offsets_out_host, "ndmps_region_debug_offsets: NULL argument");
-    const int L = plan->levels;
     RegionPlan rp;
     plan_region(plan, lo, hi, rp);
-    // site-order prefix of every kept row, level by level: row (parent, digit) of the gathered product
-    std::vector<int64_t> prev(1, 0), cur;
-    for (int l = 0; l < rp.s; l++) {
-        const int64_t d = plan->site_dims[l];
-        cur.assign((size_t)rp.left[(size_t)l].count(), 0);
-        walk(rp, rp.left[(size_t)l], [&](int64_t j, int64_t q) { cur[(size_t)j] = prev[(size_t)(q / d)] * d + q % d; });
-        prev.swap(cur);
-    }
-    const std::vector<int64_t> rowH = prev;
-    // site-order suffix of every kept column: column (digit, child) of the gathered product
-    prev.assign(1, 0);
+    std::vector<int64_t> rowH, colC;
     int64_t Q = 1;
-    for (int k = L - 1; k >= rp.s; k--) {
-        const int64_t mc = rp.m[(size_t)k + 1];
-        cur.assign((size_t)rp.m[(size_t)k], 0);
-        walk(rp, rp.right[(size_t)k], [&](int64_t j, int64_t q) { cur[(size_t)j] = (q / mc) * Q + prev[(size_t)(q % mc)]; });
-        prev.swap(cur);
-        Q *= plan->site_dims[k];
-    }
-    const std::vector<int64_t>& colC = prev;
+    region_sites(plan, rp, rowH, colC, &Q);
     const int64_t C = rp.C;
     walk(rp, rp.box, [&](int64_t j, int64_t q) { site_offsets_out_host[j] = rowH[(size_t)(q / C)] * Q + colC[(size_t)(q % C)]; });
     info_out[1] = rp.H;

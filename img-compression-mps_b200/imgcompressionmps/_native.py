@@ -15,6 +15,7 @@ import numpy as np
 
 F32, F64 = 0, 1
 CUT_ABS, CUT_REL, CUT_SUM2, CUT_RSUM2, CUT_SUM1, CUT_RSUM1 = 1, 2, 3, 4, 5, 6
+PROJ_MAX, PROJ_MIN = 1, 2
 CUTOFF_MODES = {"abs": CUT_ABS, "rel": CUT_REL, "sum2": CUT_SUM2, "rsum2": CUT_RSUM2, "sum1": CUT_SUM1,
                 "rsum1": CUT_RSUM1}
 
@@ -75,6 +76,8 @@ PROTOTYPES = {
     "ndmps_sample_points": (ci, [vp, vp, p_vp, ci, p_i64, vp, i64, ci, vp]),
     "ndmps_sample_grid": (ci, [vp, vp, p_vp, ci, p_i64, p_f64, p_f64, p_i64, ci, ci, vp]),
     "ndmps_region_debug_offsets": (ci, [vp, p_i64, p_i64, p_i64, p_i64]),
+    "ndmps_project_region": (ci, [vp, vp, p_vp, ci, p_i64, p_i64, p_i64, ci, ci, ci, vp]),
+    "ndmps_project_debug_offsets": (ci, [vp, p_i64, p_i64, ci, i64, p_i64, p_i64]),
     "ndmps_marginalize": (ci, [vp, vp, p_vp, ci, p_i64, p_i64, p_vp, p_i64]),
     "ndmps_overlap": (ci, [vp, p_vp, p_i64, ci, p_vp, p_i64, ci, ci, p_i64, p_f64]),
     "ndmps_quantize": (ci, [vp, vp, i64, ci, f64, f64, ci, vp]),
@@ -272,6 +275,19 @@ class Plan:
         check(self.lib.ndmps_region_debug_offsets(self.handle, i64_array(lo), i64_array(hi), info,
                                                   out.ctypes.data_as(p_i64)), "ndmps_region_debug_offsets")
         return dict(zip(("s", "rows", "cols"), (int(v) for v in info))), out
+
+    def project_debug(self, lo, hi, axis: int, block_elems: int):
+        """(dict(s, rows, cols, blocks), site-order index read, block that reads it), both (output elements, extent along
+        ``axis``), as the projection of the box [lo, hi) along ``axis`` computes them with blocks of at most
+        ``block_elems`` elements of T (at least one axis-0 high part each)."""
+        ext = [int(h) - int(l) for l, h in zip(lo, hi)]
+        e = ext[axis] if 0 <= axis < len(ext) else 0
+        count = int(np.prod([x for a, x in enumerate(ext) if a != axis], dtype=np.int64))
+        out = np.empty((2, max(count, 0), max(e, 0)), dtype=np.int64)
+        info = (C.c_int64 * 4)()
+        check(self.lib.ndmps_project_debug_offsets(self.handle, i64_array(lo), i64_array(hi), int(axis), int(block_elems),
+                                                   info, out.ctypes.data_as(p_i64)), "ndmps_project_debug_offsets")
+        return dict(zip(("s", "rows", "cols", "blocks"), (int(v) for v in info))), out[0], out[1]
 
     def tile_info(self, inverse: bool) -> dict:
         out = (C.c_int64 * 6)()

@@ -386,8 +386,9 @@ def contract_dense(cores):
     return out
 
 
-def region_box(shape, index):
-    """numpy basic indexing with step 1 -> (lo, hi, result shape) of the box it selects in a volume of ``shape``.
+def region_box_axes(shape, index):
+    """numpy basic indexing with step 1 -> (lo, hi, result shape, kept axes) of the box it selects in a volume of
+    ``shape``; axis j of the result is volume axis ``kept[j]`` (an int drops its axis).
 
     ``index``: an int, a slice, ``Ellipsis`` or a tuple of them, with at most one ``Ellipsis`` and at most ``ndim``
     entries (missing trailing entries select whole axes).  Ints drop their axis and may be negative; slice bounds
@@ -413,7 +414,7 @@ def region_box(shape, index):
         at = items.index(Ellipsis)
         items = items[:at] + (slice(None),) * (ndim - len(items) + 1) + items[at + 1:]
     items = items + (slice(None),) * (ndim - len(items))
-    lo, hi, out_shape = [], [], []
+    lo, hi, out_shape, kept = [], [], [], []
     for axis, (it, n) in enumerate(zip(items, shape)):
         if isinstance(it, slice):
             if it.step is not None and operator.index(it.step) != 1:
@@ -423,6 +424,7 @@ def region_box(shape, index):
             lo.append(start)
             hi.append(stop)
             out_shape.append(stop - start)
+            kept.append(axis)
         else:
             i = operator.index(it)
             if not -n <= i < n:
@@ -430,7 +432,13 @@ def region_box(shape, index):
             i += n if i < 0 else 0
             lo.append(i)
             hi.append(i + 1)
-    return lo, hi, tuple(out_shape)
+    return lo, hi, tuple(out_shape), tuple(kept)
+
+
+def region_box(shape, index):
+    """numpy basic indexing with step 1 -> (lo, hi, result shape) of the box it selects in a volume of ``shape``;
+    ``region_box_axes`` without the kept axes."""
+    return region_box_axes(shape, index)[:3]
 
 
 def contract_region(cores, shape, lo, hi, plan=None):
@@ -441,6 +449,26 @@ def contract_region(cores, shape, lo, hi, plan=None):
     out = torch.empty([int(h) - int(l) for l, h in zip(lo, hi)], dtype=cores[0].dtype, device=cores[0].device)
     N.check(N.load_library().ndmps_contract_region(N.handle(), plan.handle, ptrs, code, ranks, N.i64_array(lo),
                                                    N.i64_array(hi), N.ptr(out)), "ndmps_contract_region")
+    return out
+
+
+PROJECTION_OPS = {"max": N.PROJ_MAX, "min": N.PROJ_MIN}
+
+
+def project_region(cores, shape, lo, hi, axis, op, idct_last_axis: bool = False):
+    """``op`` ("max" or "min", NaN propagating) over volume axis ``axis`` of the box [lo, hi) of the volume of ``shape``
+    that the cores encode, as a device tensor of the box's shape without ``axis``."""
+    torch = _torch()
+    cores, ptrs, code, ranks = _mps_args(cores)
+    plan = plan_for(tuple(shape))
+    ext = [int(h) - int(l) for l, h in zip(lo, hi)]
+    code_op = PROJECTION_OPS.get(op, 0)               # anything else: the library refuses it
+    # a bad axis gets an empty output: the library refuses the axis before it looks at out
+    out = torch.empty(ext[:axis] + ext[axis + 1:] if 0 <= axis < len(ext) else [0], dtype=cores[0].dtype,
+                      device=cores[0].device)
+    N.check(N.load_library().ndmps_project_region(N.handle(), plan.handle, ptrs, code, ranks, N.i64_array(lo),
+                                                  N.i64_array(hi), int(axis), code_op, int(bool(idct_last_axis)),
+                                                  N.ptr(out)), "ndmps_project_region")
     return out
 
 

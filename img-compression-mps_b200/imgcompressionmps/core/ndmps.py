@@ -323,6 +323,52 @@ class NDMPS:
         rec = self.sample_grid_device(origin, steps, shape)
         return None if rec is None else rec.cpu().numpy()
 
+    # ------------------------------------------------------------------ intensity projections (extension)
+    def _projection_args(self, axis, op, index):
+        """(lo, hi, volume axis, result shape) of ``project``; the argument errors of ``project_device``."""
+        import operator
+        if op not in _ops.PROJECTION_OPS:
+            raise ValueError(f"project: op must be 'max' or 'min', got {op!r}")
+        if isinstance(axis, (bool, np.bool_)) or not hasattr(axis, "__index__"):
+            raise TypeError(f"project: axis {axis!r} is not an integer")
+        axis = operator.index(axis)
+        lo, hi, out_shape, kept = _ops.region_box_axes(self._shape, () if index is None else index)
+        nd = len(out_shape)
+        if not -nd <= axis < nd:
+            raise ValueError(f"project: axis {axis} is out of bounds for an indexed result of {nd} dimensions")
+        axis %= nd
+        if out_shape[axis] == 0:
+            raise ValueError(f"project: zero-size extent along axis {axis}, which has no {op}")
+        return lo, hi, kept[axis], out_shape[:axis] + out_shape[axis + 1:]
+
+    def project_device(self, axis, op: str = "max", index=None):
+        """``getattr(np, op)(to_tensor()[index], axis=axis)`` as a CUDA tensor: a maximum (``op="max"``) or minimum
+        (``"min"``) intensity projection, computed from the cores without holding the box in memory.
+
+        ``index`` follows ``to_tensor_region``'s rules (ints, step-1 slices, ``...``; ``_ops.region_box``); None is the
+        whole tensor, so ``project(0, index=(slice(100, 140),))`` is a 40-slice thick-slab MIP.  ``axis`` counts the
+        axes of the indexed result and may be negative.  NaN propagates as in ``np.max`` / ``np.min``.  The result has
+        the cores' dtype and the indexed shape without ``axis`` (0-d for a 1-D indexed result).  Every voxel of the box
+        is still computed, but a block of at most 16 MB of the decode product at a time, each reduced into the result
+        as soon as it is written; in "DCT" mode each block covers whole last-axis lines and is inverse-transformed
+        first.  An ``op`` other than "max" / "min", an ``axis`` outside the indexed result's axes (a 0-d one has none)
+        and an empty extent along ``axis`` raise ``ValueError``; index errors are ``region_box``'s.  An empty extent on
+        another axis gives an empty result.  Any other mode returns None after the arguments are checked."""
+        torch = _torch()
+        lo, hi, vaxis, res_shape = self._projection_args(axis, op, index)
+        if self.mode not in ("Std", "DCT"):
+            return None
+        cores = self.mps.cores
+        if any(h == l for l, h in zip(lo, hi)):
+            return torch.empty(res_shape, dtype=cores[0].dtype, device=cores[0].device)
+        out = _ops.project_region(cores, self._shape, lo, hi, vaxis, op, idct_last_axis=self.mode == "DCT")
+        return out.view(res_shape)
+
+    def project(self, axis, op: str = "max", index=None):
+        """``project_device(axis, op, index)`` as a numpy array; None for a mode other than "Std" / "DCT"."""
+        rec = self.project_device(axis, op, index)
+        return None if rec is None else rec.cpu().numpy()
+
     # ------------------------------------------------------------------ block-mean reconstruction (extension)
     def coarse_shape(self, levels) -> tuple:
         """Shape of ``to_tensor_coarse(levels)`` with no index: axis a averaged over its finest ``k_a`` digits, i.e.

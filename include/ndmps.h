@@ -263,6 +263,31 @@ int ndmps_sample_grid(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void* co
 int ndmps_region_debug_offsets(const ndmps_plan_t* plan, const int64_t* lo, const int64_t* hi, int64_t* info_out,
                                int64_t* site_offsets_out_host);
 
+/* ---- K7d: maximum / minimum intensity projection of a box, without the box ------
+ * An extension beyond the reference: op(to_tensor()[box], axis) (numpy's max / min, NaN propagating) from the cores.
+ * out = op over volume axis `axis` of the box [lo, hi), C order over the other axes, in the cores' dtype.  The box is
+ * decoded as in ndmps_contract_region, but the product T = X_H W_C runs in row blocks of whole axis-0 high parts of at
+ * most 16 MB each, and every block is reduced into out as soon as it is written, so the workspace holds the two
+ * restricted chains and one block, never the box.  idct_last_axis = 1 (mode "DCT"): the box is widened to the whole
+ * last axis, and every block is gathered to volume order and inverse-transformed along it before the reduction.
+ * On the context's stream, no host synchronisation.  A box outside the volume, an axis outside 0..ndim-1, an op other
+ * than NDMPS_PROJ_MAX / NDMPS_PROJ_MIN, or an empty extent along `axis` return NDMPS_ERR_INVALID; an empty extent on
+ * another axis is a no-op (out may then be NULL). */
+#define NDMPS_PROJ_MAX 1
+#define NDMPS_PROJ_MIN 2
+int ndmps_project_region(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void* const* cores, int dtype,
+                         const int64_t* ranks, const int64_t* lo, const int64_t* hi, int axis, int op,
+                         int idct_last_axis, void* out);
+/* host-only index check of ndmps_project_region in Std mode (no device work), with the block bound `block_elems`
+ * (elements of T; the device path uses 16 MB): info_out[4] = {split site s, |H|, |C|, blocks}; for every output
+ * element o (C order over the box without `axis`) and position j along `axis`, offsets_out_host[o * e + j] (e = the
+ * box's extent along `axis`) = the flat site-order index (row * Q_s + column) the reduction reads, and
+ * offsets_out_host[count * e + o * e + j] (count = the output elements) = the block that reads it (-1: none, -2: more
+ * than one).  The arguments are
+ * checked as ndmps_project_region checks them; an empty box writes {s, 0, 0, 0} and nothing else. */
+int ndmps_project_debug_offsets(const ndmps_plan_t* plan, const int64_t* lo, const int64_t* hi, int axis,
+                                int64_t block_elems, int64_t* info_out, int64_t* offsets_out_host);
+
 /* ---- K7c: block-mean (coarse) MPS, without the whole tensor -------------------
  * An extension beyond the reference: the mean of to_tensor() over non-overlapping blocks, from the cores.
  * drop_levels (ndim values, 0 <= k_a <= levels): axis a is averaged over its finest k_a digits, i.e. over blocks of
