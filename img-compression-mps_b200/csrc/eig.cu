@@ -792,12 +792,6 @@ eigh_small_kernel(const double* __restrict__ G, int n, int max_sweeps, double to
     int sweep = 0;
     int done = rank < 2 ? 1 : 0;
     float relmax = 0.f;
-#ifdef NDMPS_EIG_PROF
-    long long pt[4] = {0, 0, 0, 0}, pl = clock64();
-#define EPROF(i) do { long long now_ = clock64(); pt[i] += now_ - pl; pl = now_; } while (0)
-#else
-#define EPROF(i) do { } while (0)
-#endif
     while (!done && sweep < max_sweeps) {
         bool any = false;
         for (int lr = 0; lr < P - 1; lr++) {
@@ -807,12 +801,9 @@ eigh_small_kernel(const double* __restrict__ G, int n, int max_sweeps, double to
                 if (m < matches) tournament_pair(P, lr, m, s1, s2);
                 const bool valid = m < matches && s1 < rank && s2 < rank;
                 const int c1 = valid ? piv[s1] : 0, c2 = valid ? piv[s2] : 0;
-                EPROF(0);
                 any |= rotate_group<NR, 8>(S + (size_t)c1 * ld, S + (size_t)c2 * ld, n, li, valid, tol2, floor2, relmax);
-                EPROF(1);
             }
             __syncthreads();
-            EPROF(2);
         }
         sweep++;
         done = !__syncthreads_or(any ? 1 : 0);
@@ -849,9 +840,6 @@ eigh_small_kernel(const double* __restrict__ G, int n, int max_sweeps, double to
         const double* col = S + (size_t)piv[c] * ld;
         for (int i = lane; i < n; i += 32) evecs[(size_t)i * n + cnt] = col[i] * invn;
     }
-#ifdef NDMPS_EIG_PROF
-    if (tid == 0) printf("[eig prof] n=%d rank=%d sweeps=%d cycles: pairing %lld rotate %lld sync %lld\n", n, rank, sweep, pt[0], pt[1], pt[2]);
-#endif
     if (tid == 0) { info[0] = done ? sweep : -(sweep + 1); info[1] = rank; }
 }
 

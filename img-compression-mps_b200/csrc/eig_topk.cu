@@ -94,18 +94,6 @@ __device__ __forceinline__ double block_sum_all(double v, double* scratch) {
     return s[0];
 }
 
-// per-phase cycle counts of one thread (build with -DNDMPS_TOPK_PROF): register accumulators, written once at the end
-#ifdef NDMPS_TOPK_PROF
-__device__ unsigned long long g_prof[8];
-#define PROF_DECL unsigned long long prof_acc[8] = {0, 0, 0, 0, 0, 0, 0, 0}; long long prof_last = clock64()
-#define PROF_MARK(i) do { long long now = clock64(); if (jn < NDMPS_TOPK_PROF) prof_acc[i] += (unsigned long long)(now - prof_last); prof_last = now; } while (0)
-#define PROF_FLUSH() do { if (tid == 224 && cta == 0) { for (int i_ = 0; i_ < 8; i_++) g_prof[i_] += prof_acc[i_]; } } while (0)
-#else
-#define PROF_DECL do { } while (0)
-#define PROF_MARK(i) do { } while (0)
-#define PROF_FLUSH() do { } while (0)
-#endif
-
 // The inner pass of the tridiagonalisation for the chunks Q0 .. NEQ-1 of a warp's RPW rows: A -= u w^T + w u^T on
 // these columns, acc += A u'.  No predicates and no branches: the loads of u, w, u' are hoisted ahead of the
 // dependent DFMA pairs by the compiler, which a per-chunk `if` prevented (each chunk then cost a full
@@ -185,7 +173,6 @@ tridiag_kernel(const double* __restrict__ G, int n, int ldv, double* __restrict_
     unsigned epoch = 0;
     __syncthreads();
     if constexpr (CL) cluster_barrier();                 // every CTA of the cluster is resident before the first remote store
-    PROF_DECL;
     for (int jn = 0; jn <= n - 2; jn++) {
         const int par = jn & 1;
         double r[KM];                                    // row jn of the current matrix, columns >= jn
@@ -224,9 +211,7 @@ tridiag_kernel(const double* __restrict__ G, int n, int ldv, double* __restrict_
             double part = 0.0;
 #pragma unroll
             for (int m = 0; m < KM; m++) part = fma(pf[m], u[tid + m * NT], part);
-            PROF_MARK(0);
             const double s = block_sum_all<NT / 32>(part, red0);
-            PROF_MARK(1);
             const double K = -0.5 * tau * tau * s;
             const double wj = fma(tau, pj, K);           // u[jn] = 1
 #pragma unroll
@@ -266,9 +251,7 @@ tridiag_kernel(const double* __restrict__ G, int n, int ldv, double* __restrict_
             const int k = tid + m * NT;
             if (k >= jn + 2 && k < n) part = fma(r[m], r[m], part);
         }
-        PROF_MARK(2);
         const double sigma = block_sum_all<NT / 32>(part, red1);  // the barrier inside also publishes s_alpha and wv
-        PROF_MARK(3);
         const double alpha = s_alpha;
         double beta = alpha, taun = 0.0, scal = 0.0;
         if (sigma > 1e-280) {
@@ -286,7 +269,6 @@ tridiag_kernel(const double* __restrict__ G, int n, int ldv, double* __restrict_
         }
         if (cta == 0 && tid == 0) { e_g[jn] = beta; tau_g[jn] = taun; }
         __syncthreads();
-        PROF_MARK(4);
         // fused rank-2 update (reflector jn-1) + product with reflector jn, this warp's rows, column chunks >= jn+1.
         // Straight-line code from the first live quarter of the chunks on (fused_pass): dead columns and dead rows
         // are updated with whatever finite values the vectors hold there and multiply u'[k] = 0.
@@ -356,18 +338,15 @@ tridiag_kernel(const double* __restrict__ G, int n, int ldv, double* __restrict_
                     if (live[t] && lane == 0) __stcg(pw + gi[t], acc[t]);
             }
         }
-        PROF_MARK(5);
         if constexpr (CL) {
             cluster_barrier();
         } else {
             epoch++;
             grid_barrier(ctrl, epoch * C);
         }
-        PROF_MARK(6);
         double* t = u; u = un; un = t;
         tau = taun;
     }
-    PROF_FLUSH();
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1232,17 +1211,6 @@ int eigh_topk(ndmps_ctx* ctx, const double* G, int64_t n64, int64_t k64, double*
                 NDMPS_TRY(coop_launch(ctx, fn, dim3(C), dim3(TDT), args, 0));
             }
         }
-#ifdef NDMPS_TOPK_PROF
-        {
-            unsigned long long h[8];
-            cudaStreamSynchronize(ctx->stream);
-            cudaMemcpyFromSymbol(h, g_prof, sizeof(h));
-            fprintf(stderr, "[prof] n=%d cycles: load+dot %llu, sum_s %llu, w,r %llu, sum_sigma %llu, householder+sync %llu, fused %llu, barrier %llu\n",
-                    n, h[0], h[1], h[2], h[3], h[4], h[5], h[6]);
-            unsigned long long z[8] = {0};
-            cudaMemcpyToSymbol(g_prof, z, sizeof(z));
-        }
-#endif
     }
     // 2. shifts
     const int passes = 8;

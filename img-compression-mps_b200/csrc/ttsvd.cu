@@ -190,36 +190,21 @@ static double renorm_factor(const double* s, int64_t n, int64_t keep, int power)
     return pow((k + l) / k, 1.0 / power);
 }
 
-// The tcgen05 Gram decides ON THE DEVICE whether its digits are exact enough (tc_gemm.cu); the projection needs that
-// answer on the host to pick its kernel.  It rides along with the eigenvalue readback every sweep step does anyway:
-// the 4-byte flag is copied into an unused slot of the pinned scratch before the same synchronisation.
-static int fetch_exact_flag(ndmps_ctx* ctx, size_t slot) {
+// Copy `count` doubles from the device into the pinned scratch and wait for them.  The tcgen05 Gram decides ON THE
+// DEVICE whether its digits are exact enough (tc_gemm.cu); the projection needs that answer on the host to pick its
+// kernel.  While it is pending, the 4-byte flag rides along in an unused slot of the scratch before the same wait.
+static int read_back(ndmps_ctx* ctx, const double* src, int64_t count) {
+    const size_t slot = (size_t)count + 8;
+    NDMPS_TRY(ensure_pinned(ctx, (size_t)count + 64));
+    NDMPS_TRY(readback(ctx, ctx->pinned, src, (size_t)count * sizeof(double)));
     auto& dg = ctx->tc_digits;
-    if (dg.use_exact == nullptr || dg.gen != ctx->ws.generation || dg.exact_host >= 0) return NDMPS_OK;
-    NDMPS_TRY(readback(ctx, ctx->pinned + slot, dg.use_exact, sizeof(int)));
-    dg.exact_host = -2;                                  // in flight
-    return NDMPS_OK;
-}
-static void note_exact_flag(ndmps_ctx* ctx, size_t slot) {
-    auto& dg = ctx->tc_digits;
-    if (dg.exact_host == -2) dg.exact_host = *reinterpret_cast<const int*>(ctx->pinned + slot) != 0 ? 1 : 0;
-}
-
-// copy n eigenvalues to the host, return sqrt(max(l, 0)) in sv (host vector)
-static int fetch_svals(ndmps_ctx* ctx, const double* evals_dev, int64_t n, std::vector<double>& sv) {
-    NDMPS_TRY(ensure_pinned(ctx, (size_t)n + 64));
-    NDMPS_TRY(readback(ctx, ctx->pinned, evals_dev, (size_t)n * sizeof(double)));
-    NDMPS_TRY(fetch_exact_flag(ctx, (size_t)n + 8));
+    const bool flag = dg.use_exact != nullptr && dg.gen == ctx->ws.generation && dg.exact_host < 0;
+    if (flag) NDMPS_TRY(readback(ctx, ctx->pinned + slot, dg.use_exact, sizeof(int)));
     NDMPS_CUDA_TRY(stream_wait(ctx));
-    note_exact_flag(ctx, (size_t)n + 8);
-    sv.resize((size_t)n);
-    for (int64_t i = 0; i < n; i++) sv[i] = ctx->pinned[i] > 0.0 ? sqrt(ctx->pinned[i]) : 0.0;
+    if (flag) dg.exact_host = *reinterpret_cast<const int*>(ctx->pinned + slot) != 0 ? 1 : 0;
     return NDMPS_OK;
 }
 
-// ---------------------------------------------------------------------------------
-// the sweep
-// ---------------------------------------------------------------------------------
 struct TrimOpts {
     double cutoff;
     int mode;
@@ -227,16 +212,17 @@ struct TrimOpts {
     int renorm;
 };
 
+struct Bond { std::vector<double> sv; int64_t n = 0; double f = 1.0; };   // singular values (host), kept, renorm factor
+
 // Bond cap set and the matrix much larger than the cap: try the leading-eigenpair solver
 // (eig_topk.cu).  It is used only when the host can PROVE from its output that the trimming rule
 // (n_keep above) lands on the cap: the weight outside the k leading eigenvalues, trace(G) minus
 // their sum, must exceed the cutoff target with a margin far above the rounding error of that
 // difference, and lambda_k must be well above the absolute error floor of the tridiagonal
-// reduction (~ n eps lambda_1).  Anything else: *capped = false and the caller runs the full
+// reduction (~ n eps lambda_1).  Anything else leaves *b as it is and the caller runs the full
 // solver, so ranks never depend on which solver ran.  U: mj x mj buffer, eigenvector t in column t.
 static int capped_eigh(ndmps_ctx* ctx, const double* Gj, int64_t mj, int64_t nmax, const TrimOpts& opt, double* evals_dev,
-                       double* U, std::vector<double>& sv, int64_t* n_out, double* f_out, bool* capped) {
-    *capped = false;
+                       double* U, Bond* b) {
     const int64_t k = opt.max_bond;
     if (!ctx->opt_eig_topk || k <= 0 || mj < 4 * k || mj < 96 || nmax <= k) return NDMPS_OK;
     const bool sum2 = opt.mode == NDMPS_CUT_SUM2 || opt.mode == NDMPS_CUT_RSUM2;
@@ -247,11 +233,7 @@ static int capped_eigh(ndmps_ctx* ctx, const double* Gj, int64_t mj, int64_t nma
     bool done = false;
     { StageScope sc(ctx, ST_EIG); NDMPS_TRY(eigh_topk(ctx, Gj, mj, k, out, U, mj, &done)); }
     if (!done) return NDMPS_OK;
-    NDMPS_TRY(ensure_pinned(ctx, (size_t)k + 64));
-    NDMPS_TRY(readback(ctx, ctx->pinned, out, (size_t)(k + 2) * sizeof(double)));
-    NDMPS_TRY(fetch_exact_flag(ctx, (size_t)k + 8));
-    NDMPS_CUDA_TRY(stream_wait(ctx));
-    note_exact_flag(ctx, (size_t)k + 8);
+    NDMPS_TRY(read_back(ctx, out, k + 2));
     const double* ev = ctx->pinned;
     const double trace = ev[k], rank_loss = ev[k + 1];
     double kept = 0.0;
@@ -266,16 +248,34 @@ static int capped_eigh(ndmps_ctx* ctx, const double* Gj, int64_t mj, int64_t nma
                 (long long)mj, (long long)k, ev[0] > 0.0 ? ev[k - 1] / ev[0] : 0.0, trace > 0.0 ? tail / trace : 0.0,
                 ok ? "cap binds" : "full solver");
     if (!ok) return NDMPS_OK;
-    sv.assign((size_t)mj, 0.0);
-    for (int64_t i = 0; i < k; i++) sv[(size_t)i] = sqrt(ev[i]);
-    *n_out = k;
-    *f_out = opt.renorm == 2 ? sqrt(trace / kept) : 1.0;
-    // the kept eigenvalues also on the device, where the column-side branch scales by them
+    b->sv.assign((size_t)mj, 0.0);
+    for (int64_t i = 0; i < k; i++) b->sv[(size_t)i] = sqrt(ev[i]);
+    b->n = k;
+    b->f = opt.renorm == 2 ? sqrt(trace / kept) : 1.0;
+    // the kept eigenvalues also on the device, where the column-side step scales by them
     NDMPS_TRY(copy_small(ctx, evals_dev, out, (size_t)k * sizeof(double)));
-    *capped = true;
     return NDMPS_OK;
 }
 
+// The truncation of one bond with one host wait: evals (m) and U (m x m, eigenvector t in column t) of its float64 Gram
+// matrix G on the device, *b on the host.  nmax bounds the rank; try_capped opens the leading-eigenpair route.
+static int decide_bond(ndmps_ctx* ctx, double* G, int64_t m, int64_t nmax, const TrimOpts& opt, bool try_capped, double eig_tol,
+                       double* evals, double* U, Bond* b) {
+    *b = Bond();
+    if (try_capped) NDMPS_TRY(capped_eigh(ctx, G, m, nmax, opt, evals, U, b));
+    if (b->n > 0) return NDMPS_OK;                       // the cap binds
+    { StageScope sc(ctx, ST_EIG); NDMPS_TRY(eigh(ctx, G, m, evals, U, eig_tol)); }
+    NDMPS_TRY(read_back(ctx, evals, m));
+    b->sv.resize((size_t)m);
+    for (int64_t i = 0; i < m; i++) b->sv[i] = ctx->pinned[i] > 0.0 ? sqrt(ctx->pinned[i]) : 0.0;
+    b->n = n_keep(b->sv.data(), nmax, opt.cutoff, opt.mode, opt.max_bond);
+    b->f = renorm_factor(b->sv.data(), nmax, b->n, opt.renorm);
+    return NDMPS_OK;
+}
+
+// ---------------------------------------------------------------------------------
+// the sweep
+// ---------------------------------------------------------------------------------
 // Column-sharded sweep (SURVEY section 8e, row 2): this rank holds the slice of the dense site array
 // with the last site index in its block, i.e. a column block of every unfolding.  The left factor
 // of a step depends only on G = M M^T, a SUM over column blocks: local Gram, allreduce through the
@@ -291,12 +291,144 @@ struct ShardCtl {
     int64_t remainder_rows = 1, remainder_cols = 0;
 };
 
+// what every step of one sweep shares
+struct Sweep {
+    ndmps_ctx* ctx;
+    int dtype;
+    const int64_t* dims;
+    TrimOpts opt;
+    double eig_tol;
+    void* const* cores;
+    const int64_t* core_cap;
+    int64_t* ranks;
+    double* svals;                 // optional: singular values of bond i at svals + i * svals_stride
+    int64_t svals_stride;
+    const ShardCtl* sh;            // optional
+};
+
+// rank and singular values (times the renorm factor) of bond `site`, and the capacity of its core (rows x b.n)
+static int record_site(const Sweep& s, int site, int64_t rows, const Bond& b) {
+    s.ranks[site] = b.n;
+    if (s.svals)
+        for (int64_t t = 0; t < b.n && t < s.svals_stride; t++) s.svals[(int64_t)site * s.svals_stride + t] = b.sv[t] * b.f;
+    if (s.core_cap[site] < rows * b.n) {
+        set_error("ttsvd: core %d needs %lld elements, capacity %lld", site, (long long)(rows * b.n), (long long)s.core_cap[site]);
+        return NDMPS_ERR_CAPACITY;
+    }
+    return NDMPS_OK;
+}
+
+// Sites site .. site+k-1 from ONE row-side Gram pass over the unfolding M (D x C, D <= C) and ONE projection:
+// *T = P^T M (*r_out x C), P the accumulated isometry of the group
+static int row_group_step(const Sweep& s, const void* M, int64_t D, int64_t C, int site, int k, int64_t r_prev, void** T,
+                          int64_t* r_out) {
+    ndmps_ctx* ctx = s.ctx;
+    const int dtype = s.dtype;
+    const ShardCtl* sh = s.sh;
+    double* G = nullptr;
+    NDMPS_TRY(ctx->ws.get<double>((size_t)(D * D), &G));
+    { StageScope sc(ctx, ST_GRAM); NDMPS_TRY(gram(ctx, M, D, C, C, dtype, 0, G)); }
+    if (sh && sh->world > 1) {
+        const int rc_hook = sh->allreduce(sh->user, G, D * D, (void*)ctx->stream);
+        if (rc_hook != 0) { set_error("ttsvd: the allreduce hook failed (%d)", rc_hook); return NDMPS_ERR_CUDA; }
+    }
+    double* P = nullptr;       // (pd x rc) accumulated isometry (times renorm factors); nullptr = identity
+    int64_t pd = r_prev, rc = r_prev;
+    for (int j = 0; j < k; j++) {
+        const int64_t d = s.dims[site + j];
+        const int64_t X = pd * d, rest = D / X, mj = rc * d;
+        double* Gt = G;
+        if (rest > 1) {
+            NDMPS_TRY(ctx->ws.get<double>((size_t)(X * X), &Gt));
+            partial_trace_kernel<<<ew_grid(ctx, X * X), 256, 0, ctx->stream>>>(G, D, X, rest, Gt);
+            NDMPS_LAUNCH_CHECK(ctx);
+        }
+        double* Gj = Gt;
+        double* K = nullptr;
+        if (P != nullptr) {
+            NDMPS_TRY(ctx->ws.get<double>((size_t)(X * mj), &K));
+            kron_identity_kernel<<<ew_grid(ctx, X * mj), 256, 0, ctx->stream>>>(P, pd, rc, d, K);
+            NDMPS_LAUNCH_CHECK(ctx);
+            double* tmp = nullptr;
+            NDMPS_TRY(ctx->ws.get<double>((size_t)(X * mj), &tmp));
+            NDMPS_TRY(gemm(ctx, X, mj, X, 1.0, Gt, NDMPS_F64, X, 1, K, NDMPS_F64, mj, 1, tmp, NDMPS_F64, mj));
+            NDMPS_TRY(ctx->ws.get<double>((size_t)(mj * mj), &Gj));
+            NDMPS_TRY(gemm(ctx, mj, mj, X, 1.0, K, NDMPS_F64, 1, mj, tmp, NDMPS_F64, mj, 1, Gj, NDMPS_F64, mj));
+        }
+        double *evals = nullptr, *U = nullptr;
+        NDMPS_TRY(ctx->ws.get<double>((size_t)mj, &evals));
+        NDMPS_TRY(ctx->ws.get<double>((size_t)(mj * mj), &U));
+        const int64_t cols_j = C * rest * (sh ? sh->world : 1);     // the rank is at most min(rows, cols)
+        Bond b;
+        NDMPS_TRY(decide_bond(ctx, Gj, mj, mj < cols_j ? mj : cols_j, s.opt, true, s.eig_tol, evals, U, &b));
+        NDMPS_TRY(record_site(s, site + j, mj, b));
+        NDMPS_TRY(scale_convert(ctx, U, mj, b.n, mj, nullptr, nullptr, 1.0, s.cores[site + j], dtype, b.n));
+        // P_next = f * K * U[:, :n]   (X x n)
+        double* Pn = nullptr;
+        NDMPS_TRY(ctx->ws.get<double>((size_t)(X * b.n), &Pn));
+        if (K == nullptr) NDMPS_TRY(scale_convert(ctx, U, X, b.n, mj, nullptr, nullptr, b.f, Pn, NDMPS_F64, b.n));
+        else NDMPS_TRY(gemm(ctx, X, b.n, mj, b.f, K, NDMPS_F64, mj, 1, U, NDMPS_F64, mj, 1, Pn, NDMPS_F64, b.n));
+        P = Pn;
+        pd = X;
+        rc = b.n;
+    }
+    // T = P^T M   (rc x C)
+    *r_out = rc;
+    NDMPS_TRY(ctx->ws.alloc((size_t)(rc * C) * dtype_size(dtype), T));
+    StageScope sc(ctx, ST_PROJECT);
+    bool on_tc = false;
+    if (ctx->tc_sweep && C >= 2048) {
+        // the digits the Gram of this step sliced, when it ran on the integer tensor cores (exact accumulation) ...
+        NDMPS_TRY(proj_tc_digits(ctx, M, D, C, C, P, rc, *T, dtype, C, &on_tc));
+        // ... else T^T = M^T P on bf16x3 planes: the unfolding is the MN-major operand, T leaves transposed
+        if (!on_tc) NDMPS_TRY(gemm_tc(ctx, C, rc, D, 1.0, M, dtype, 1, C, P, NDMPS_F64, rc, 1, *T, dtype, C, true, &on_tc));
+    }
+    if (!on_tc) {
+        // P^T made explicit (r x D, tiny) so the big product reads both operands along their rows
+        double* Pt = nullptr;
+        NDMPS_TRY(ctx->ws.get<double>((size_t)(rc * D), &Pt));
+        NDMPS_TRY(scaled_transpose(ctx, P, rc, D, rc, nullptr, 1.0, Pt, NDMPS_F64));
+        NDMPS_TRY(gemm(ctx, rc, C, D, 1.0, Pt, NDMPS_F64, D, 1, M, dtype, C, 1, *T, dtype, C));
+    }
+    return NDMPS_OK;
+}
+
+// Site `site` when its unfolding M (D x C) has more rows than columns: Gram on the column side, G' = M^T M = V s^2 V^T,
+// core M V[:, :n] / s (D x n), *T = f diag(s) V[:, :n]^T (n x C).  The sharded sweep hands back before such a step.
+static int column_step(const Sweep& s, const void* M, int64_t D, int64_t C, int site, void** T, int64_t* r_out) {
+    ndmps_ctx* ctx = s.ctx;
+    const int dtype = s.dtype;
+    double *G = nullptr, *evals = nullptr, *V = nullptr;
+    NDMPS_TRY(ctx->ws.get<double>((size_t)(C * C), &G));
+    { StageScope sc(ctx, ST_GRAM); NDMPS_TRY(gram(ctx, M, D, C, C, dtype, 1, G)); }
+    NDMPS_TRY(ctx->ws.get<double>((size_t)C, &evals));
+    NDMPS_TRY(ctx->ws.get<double>((size_t)(C * C), &V));
+    // the capped route leaves all but the k leading eigenvalues as they are; col_scale below reads all C
+    NDMPS_CUDA_TRY(cudaMemsetAsync(evals, 0, (size_t)C * sizeof(double), ctx->stream));
+    Bond b;
+    NDMPS_TRY(decide_bond(ctx, G, C, C, s.opt, true, s.eig_tol, evals, V, &b));   // rank <= min(D, C) = C
+    const int64_t n = b.n;
+    NDMPS_TRY(record_site(s, site, D, b));
+    double *inv_s = nullptr, *s_f = nullptr, *MV = nullptr;
+    NDMPS_TRY(ctx->ws.get<double>((size_t)C, &inv_s));
+    NDMPS_TRY(ctx->ws.get<double>((size_t)C, &s_f));
+    NDMPS_TRY(col_scale(ctx, evals, C, 1, 1.0, 1e-14, inv_s));
+    NDMPS_TRY(col_scale(ctx, evals, C, 0, b.f, 0.0, s_f));
+    // U = M V[:, :n] / s   (D x n)
+    NDMPS_TRY(ctx->ws.get<double>((size_t)(D * n), &MV));
+    NDMPS_TRY(gemm(ctx, D, n, C, 1.0, M, dtype, C, 1, V, NDMPS_F64, C, 1, MV, NDMPS_F64, n));
+    NDMPS_TRY(scale_convert(ctx, MV, D, n, n, nullptr, inv_s, 1.0, s.cores[site], dtype, n));
+    // T = f diag(s) V[:, :n]^T   (n x C)
+    *r_out = n;
+    NDMPS_TRY(ctx->ws.alloc((size_t)(n * C) * dtype_size(dtype), T));
+    NDMPS_TRY(scaled_transpose(ctx, V, n, C, C, s_f, 1.0, *T, dtype));
+    return NDMPS_OK;
+}
+
 static int ttsvd(ndmps_ctx* ctx, const void* dense, int dtype, int L, const int64_t* dims, const TrimOpts& opt,
                  void* const* cores_out, const int64_t* core_cap, int64_t* ranks_out, double* svals_out,
                  int64_t svals_stride, ShardCtl* sh = nullptr) {
     const size_t esz = dtype_size(dtype);
-    // cores stored in float32 need eigenvectors orthogonal to ~1e-8, not 1e-15: one sweep less
-    const double eig_tol = dtype == NDMPS_F32 ? 1e-10 : 0.0;
     int64_t total = 1;
     for (int i = 0; i < L; i++) total *= dims[i];
     if (svals_out)
@@ -306,6 +438,8 @@ static int ttsvd(ndmps_ctx* ctx, const void* dense, int dtype, int L, const int6
         NDMPS_CUDA_TRY(cudaMemcpyAsync(cores_out[0], dense, (size_t)total * esz, cudaMemcpyDeviceToDevice, ctx->stream));
         return NDMPS_OK;
     }
+    // cores stored in float32 need eigenvectors orthogonal to ~1e-8, not 1e-15: one sweep less
+    const Sweep s{ctx, dtype, dims, opt, dtype == NDMPS_F32 ? 1e-10 : 0.0, cores_out, core_cap, ranks_out, svals_out, svals_stride, sh};
     // float32 payload with a bond cap: the long Gram and projection passes run on tcgen05 (tc_gemm.cu); the rank
     // decisions of an UNCAPPED sweep sit at lambda / lambda_1 ~ 1e-10 and keep the exact FP64-pipe path
     struct TcScope { ndmps_ctx* c; ~TcScope() { c->tc_sweep = false; } } tc_scope{ctx};
@@ -313,7 +447,6 @@ static int ttsvd(ndmps_ctx* ctx, const void* dense, int dtype, int L, const int6
     const void* M = dense;         // current remainder, (r_prev * remaining) elements
     int64_t r_prev = 1;
     int64_t remaining = total;     // elements of the remainder divided by r_prev
-    std::vector<double> sv;
     int site = 0;
     while (site < L - 1) {
         // ---- choose the group of sites sharing one Gram pass ----
@@ -338,132 +471,10 @@ static int ttsvd(ndmps_ctx* ctx, const void* dense, int dtype, int L, const int6
         if (ctx->opt_verbose)
             fprintf(stderr, "[ndmps] sweep site %d: group of %d, unfolding %lld x %lld (%s Gram)%s\n", site, k,
                     (long long)D, (long long)C, D <= C ? "row" : "column", sh ? " [column shard]" : "");
-        int64_t r_out = 0;
         void* T = nullptr;
-        if (D <= C) {
-            double* G = nullptr;
-            NDMPS_TRY(ctx->ws.get<double>((size_t)(D * D), &G));
-            { StageScope sc(ctx, ST_GRAM); NDMPS_TRY(gram(ctx, M, D, C, C, dtype, 0, G)); }
-            if (sh && sh->world > 1) {
-                const int rc_hook = sh->allreduce(sh->user, G, D * D, (void*)ctx->stream);
-                if (rc_hook != 0) { set_error("ttsvd: the allreduce hook failed (%d)", rc_hook); return NDMPS_ERR_CUDA; }
-            }
-            double* P = nullptr;       // (pd x rc) accumulated isometry (times renorm factors); nullptr = identity
-            int64_t pd = r_prev, rc = r_prev;
-            for (int j = 0; j < k; j++) {
-                const int64_t d = dims[site + j];
-                const int64_t X = pd * d, rest = D / X, mj = rc * d;
-                double* Gt = G;
-                if (rest > 1) {
-                    NDMPS_TRY(ctx->ws.get<double>((size_t)(X * X), &Gt));
-                    partial_trace_kernel<<<ew_grid(ctx, X * X), 256, 0, ctx->stream>>>(G, D, X, rest, Gt);
-                    NDMPS_LAUNCH_CHECK(ctx);
-                }
-                double* Gj = Gt;
-                double* K = nullptr;
-                if (P != nullptr) {
-                    NDMPS_TRY(ctx->ws.get<double>((size_t)(X * mj), &K));
-                    kron_identity_kernel<<<ew_grid(ctx, X * mj), 256, 0, ctx->stream>>>(P, pd, rc, d, K);
-                    NDMPS_LAUNCH_CHECK(ctx);
-                    double* tmp = nullptr;
-                    NDMPS_TRY(ctx->ws.get<double>((size_t)(X * mj), &tmp));
-                    NDMPS_TRY(gemm(ctx, X, mj, X, 1.0, Gt, NDMPS_F64, X, 1, K, NDMPS_F64, mj, 1, tmp, NDMPS_F64, mj));
-                    NDMPS_TRY(ctx->ws.get<double>((size_t)(mj * mj), &Gj));
-                    NDMPS_TRY(gemm(ctx, mj, mj, X, 1.0, K, NDMPS_F64, 1, mj, tmp, NDMPS_F64, mj, 1, Gj, NDMPS_F64, mj));
-                }
-                double *evals = nullptr, *U = nullptr;
-                NDMPS_TRY(ctx->ws.get<double>((size_t)mj, &evals));
-                NDMPS_TRY(ctx->ws.get<double>((size_t)(mj * mj), &U));
-                // rank of this unfolding is at most min(rows, cols)
-                int64_t cols_j = C * rest * (sh ? sh->world : 1);
-                int64_t nmax = mj < cols_j ? mj : cols_j;
-                int64_t n = 0;
-                double f = 1.0;
-                bool capped = false;
-                NDMPS_TRY(capped_eigh(ctx, Gj, mj, nmax, opt, evals, U, sv, &n, &f, &capped));
-                if (!capped) {
-                    { StageScope sc(ctx, ST_EIG); NDMPS_TRY(eigh(ctx, Gj, mj, evals, U, eig_tol)); }
-                    NDMPS_TRY(fetch_svals(ctx, evals, mj, sv));
-                    n = n_keep(sv.data(), nmax, opt.cutoff, opt.mode, opt.max_bond);
-                    f = renorm_factor(sv.data(), nmax, n, opt.renorm);
-                }
-                const int s_idx = site + j;
-                ranks_out[s_idx] = n;
-                if (svals_out)
-                    for (int64_t t = 0; t < n && t < svals_stride; t++) svals_out[(int64_t)s_idx * svals_stride + t] = sv[t] * f;
-                if (core_cap[s_idx] < mj * n) {
-                    set_error("ttsvd: core %d needs %lld elements, capacity %lld", s_idx, (long long)(mj * n), (long long)core_cap[s_idx]);
-                    return NDMPS_ERR_CAPACITY;
-                }
-                NDMPS_TRY(scale_convert(ctx, U, mj, n, mj, nullptr, nullptr, 1.0, cores_out[s_idx], dtype, n));
-                // P_next = f * K * U[:, :n]   (X x n)
-                double* Pn = nullptr;
-                NDMPS_TRY(ctx->ws.get<double>((size_t)(X * n), &Pn));
-                if (K == nullptr) NDMPS_TRY(scale_convert(ctx, U, X, n, mj, nullptr, nullptr, f, Pn, NDMPS_F64, n));
-                else NDMPS_TRY(gemm(ctx, X, n, mj, f, K, NDMPS_F64, mj, 1, U, NDMPS_F64, mj, 1, Pn, NDMPS_F64, n));
-                P = Pn;
-                pd = X;
-                rc = n;
-            }
-            // T = P^T M   (rc x C)
-            r_out = rc;
-            NDMPS_TRY(ctx->ws.alloc((size_t)(r_out * C) * esz, &T));
-            {
-                StageScope sc(ctx, ST_PROJECT);
-                bool on_tc = false;
-                if (ctx->tc_sweep && C >= 2048) {
-                    // the digits the Gram of this step sliced, when it ran on the integer tensor cores (exact accumulation) ...
-                    NDMPS_TRY(proj_tc_digits(ctx, M, D, C, C, P, r_out, T, dtype, C, &on_tc));
-                    // ... else T^T = M^T P on bf16x3 planes: the unfolding is the MN-major operand, T leaves transposed
-                    if (!on_tc) NDMPS_TRY(gemm_tc(ctx, C, r_out, D, 1.0, M, dtype, 1, C, P, NDMPS_F64, r_out, 1, T, dtype, C, true, &on_tc));
-                }
-                if (!on_tc) {
-                    // P^T made explicit (r x D, tiny) so the big product reads both operands along their rows
-                    double* Pt = nullptr;
-                    NDMPS_TRY(ctx->ws.get<double>((size_t)(r_out * D), &Pt));
-                    NDMPS_TRY(scaled_transpose(ctx, P, r_out, D, r_out, nullptr, 1.0, Pt, NDMPS_F64));
-                    NDMPS_TRY(gemm(ctx, r_out, C, D, 1.0, Pt, NDMPS_F64, D, 1, M, dtype, C, 1, T, dtype, C));
-                }
-            }
-        } else {
-            // more rows than columns: Gram on the column side, G' = M^T M = V s^2 V^T
-            double *G = nullptr, *evals = nullptr, *V = nullptr;
-            NDMPS_TRY(ctx->ws.get<double>((size_t)(C * C), &G));
-            { StageScope sc(ctx, ST_GRAM); NDMPS_TRY(gram(ctx, M, D, C, C, dtype, 1, G)); }
-            NDMPS_TRY(ctx->ws.get<double>((size_t)C, &evals));
-            NDMPS_TRY(ctx->ws.get<double>((size_t)(C * C), &V));
-            int64_t n = 0;
-            double f = 1.0;
-            bool capped = false;
-            NDMPS_CUDA_TRY(cudaMemsetAsync(evals, 0, (size_t)C * sizeof(double), ctx->stream));
-            if (!sh) NDMPS_TRY(capped_eigh(ctx, G, C, C < D ? C : D, opt, evals, V, sv, &n, &f, &capped));
-            if (!capped) {
-                { StageScope sc(ctx, ST_EIG); NDMPS_TRY(eigh(ctx, G, C, evals, V, eig_tol)); }
-                NDMPS_TRY(fetch_svals(ctx, evals, C, sv));
-                n = n_keep(sv.data(), C, opt.cutoff, opt.mode, opt.max_bond);
-                f = renorm_factor(sv.data(), C, n, opt.renorm);
-            }
-            ranks_out[site] = n;
-            if (svals_out)
-                for (int64_t t = 0; t < n && t < svals_stride; t++) svals_out[(int64_t)site * svals_stride + t] = sv[t] * f;
-            if (core_cap[site] < D * n) {
-                set_error("ttsvd: core %d needs %lld elements, capacity %lld", site, (long long)(D * n), (long long)core_cap[site]);
-                return NDMPS_ERR_CAPACITY;
-            }
-            double *inv_s = nullptr, *s_f = nullptr, *MV = nullptr;
-            NDMPS_TRY(ctx->ws.get<double>((size_t)C, &inv_s));
-            NDMPS_TRY(ctx->ws.get<double>((size_t)C, &s_f));
-            NDMPS_TRY(col_scale(ctx, evals, C, 1, 1.0, 1e-14, inv_s));
-            NDMPS_TRY(col_scale(ctx, evals, C, 0, f, 0.0, s_f));
-            // U = M V[:, :n] / s   (D x n)
-            NDMPS_TRY(ctx->ws.get<double>((size_t)(D * n), &MV));
-            NDMPS_TRY(gemm(ctx, D, n, C, 1.0, M, dtype, C, 1, V, NDMPS_F64, C, 1, MV, NDMPS_F64, n));
-            NDMPS_TRY(scale_convert(ctx, MV, D, n, n, nullptr, inv_s, 1.0, cores_out[site], dtype, n));
-            // T = f diag(s) V[:, :n]^T   (n x C)
-            r_out = n;
-            NDMPS_TRY(ctx->ws.alloc((size_t)(r_out * C) * esz, &T));
-            NDMPS_TRY(scaled_transpose(ctx, V, n, C, C, s_f, 1.0, T, dtype));
-        }
+        int64_t r_out = 0;
+        if (D <= C) NDMPS_TRY(row_group_step(s, M, D, C, site, k, r_prev, &T, &r_out));
+        else NDMPS_TRY(column_step(s, M, D, C, site, &T, &r_out));
         M = T;
         r_prev = r_out;
         remaining = C;
@@ -513,17 +524,15 @@ static int compress_bond(ndmps_ctx* ctx, const void* t1, const void* t2, int dty
     NDMPS_TRY(gram(ctx, t2, r, b, b, dtype, 0, G2));
     NDMPS_TRY(gemm(ctx, r, r, r, 1.0, S1, NDMPS_F64, r, 1, G2, NDMPS_F64, r, 1, tmp, NDMPS_F64, r));
     NDMPS_TRY(gemm(ctx, r, r, r, 1.0, tmp, NDMPS_F64, r, 1, S1, NDMPS_F64, 1, r, H, NDMPS_F64, r));
-    NDMPS_TRY(eigh(ctx, H, r, sig2, Up));
-    std::vector<double> sv;
-    NDMPS_TRY(fetch_svals(ctx, sig2, r, sv));
     int64_t nmax = r < a ? r : a;
     if (b < nmax) nmax = b;
-    int64_t n = n_keep(sv.data(), nmax, opt.cutoff, opt.mode, opt.max_bond);
-    double f = renorm_factor(sv.data(), nmax, n, opt.renorm);
+    Bond bond;
+    NDMPS_TRY(decide_bond(ctx, H, r, nmax, opt, false, 0.0, sig2, Up, &bond));
+    const int64_t n = bond.n;
     *new_rank = n;
     if (svals_out)
-        for (int64_t t = 0; t < r; t++) svals_out[t] = t < n ? sv[t] * f : 0.0;
-    const double rf = sqrt(f);
+        for (int64_t t = 0; t < r; t++) svals_out[t] = t < n ? bond.sv[t] * bond.f : 0.0;
+    const double rf = sqrt(bond.f);
     // Y = S1^T U'[:, :n]   (r x n)
     NDMPS_TRY(ctx->ws.get<double>((size_t)(r * n), &Y));
     NDMPS_TRY(gemm(ctx, r, n, r, 1.0, S1, NDMPS_F64, 1, r, Up, NDMPS_F64, r, 1, Y, NDMPS_F64, n));
@@ -851,7 +860,6 @@ int ndmps_roundtrip_host(ndmps_ctx_t* ctx, const ndmps_plan_t* plan, const void*
         }
         for (int i = 0; i < L; i++) {
             int64_t l = i == 0 ? 1 : bound[(size_t)i - 1], r = i == L - 1 ? 1 : bound[(size_t)i];
-            // a bond can never exceed (left bond * d): tighten so lossless capacities stay finite
             cap[(size_t)i] = l * plan->site_dims[i] * r;
             NDMPS_TRY(ctx->ws.alloc((size_t)cap[(size_t)i] * esz, &cores[(size_t)i]));
         }

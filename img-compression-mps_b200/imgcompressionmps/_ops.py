@@ -237,32 +237,48 @@ def core_shape(i, L, dims, ranks):
     return (int(ranks[i - 1]), int(dims[i]), int(ranks[i]))
 
 
-def ttsvd(dense, dims, cutoff=1e-10, cutoff_mode="rsum2", max_bond=None, renorm=None):
-    """Left-canonical MPS cores of ``dense`` (site order); returns (cores, ranks, svals)."""
-    torch = _torch()
-    _dev(dense, "dense")
-    dims = [int(d) for d in dims]
-    L = len(dims)
+def _trim_mode(cutoff_mode, renorm):
+    """Mode code and renorm power of a sweep; ``renorm=None`` takes the mode's default."""
     mode = N.CUTOFF_MODES[cutoff_mode]
-    if renorm is None:
-        renorm = {N.CUT_RSUM2: 2, N.CUT_SUM2: 2, N.CUT_RSUM1: 1, N.CUT_SUM1: 1}.get(mode, 0)
+    default = {N.CUT_RSUM2: 2, N.CUT_SUM2: 2, N.CUT_RSUM1: 1, N.CUT_SUM1: 1}.get(mode, 0)
+    return mode, int(default if renorm is None else renorm)
+
+
+def _sweep_args(dims, cutoff, cutoff_mode, renorm, max_bond, like):
+    """Arguments cutoff .. svals_stride of both sweep entry points, and the buffers (like ``like``) they point to."""
+    torch = _torch()
+    L = len(dims)
     bounds = bond_bounds(dims, max_bond)
     caps = [int(np.prod(core_shape(i, L, dims, bounds), dtype=np.int64)) for i in range(L)]
-    bufs = [torch.empty(c, dtype=dense.dtype, device=dense.device) for c in caps]
+    bufs = [torch.empty(c, dtype=like.dtype, device=like.device) for c in caps]
     ranks = (C.c_int64 * max(L - 1, 1))()
-    stride = max(bounds) if bounds else 1
-    svals = np.zeros((max(L - 1, 1), stride), dtype=np.float64)
-    N.check(N.load_library().ndmps_ttsvd(N.handle(), N.ptr(dense), N.dtype_code(dense.dtype), L, N.i64_array(dims),
-                                         float(cutoff), mode, int(max_bond or 0), int(renorm),
-                                         N.ptr_array(bufs), N.i64_array(caps), ranks,
-                                         svals.ctypes.data_as(N.p_f64), stride), "ndmps_ttsvd")
-    ranks = [int(r) for r in ranks][:L - 1]
+    svals = np.zeros((max(L - 1, 1), max(bounds) if bounds else 1), dtype=np.float64)
+    mode, renorm = _trim_mode(cutoff_mode, renorm)
+    args = (float(cutoff), mode, int(max_bond or 0), renorm, N.ptr_array(bufs), N.i64_array(caps), ranks,
+            svals.ctypes.data_as(N.p_f64), svals.shape[1])
+    return args, bufs, ranks, svals
+
+
+def _sweep_out(bufs, ranks, svals, dims, bonds, sites):
+    """(cores, ranks, singular values) of the first ``sites`` cores and ``bonds`` bonds of a sweep, cut from its buffers;
+    a core smaller than its buffer is copied so that the buffer is freed."""
+    ranks = [int(r) for r in ranks][:bonds]
     cores = []
-    for i in range(L):
-        shp = core_shape(i, L, dims, ranks)
-        n = int(np.prod(shp, dtype=np.int64))
-        cores.append(bufs[i][:n].view(shp) if n == caps[i] else bufs[i][:n].clone().view(shp))
-    return cores, ranks, [svals[i, :ranks[i]].copy() for i in range(L - 1)]
+    for i in range(sites):
+        shp = core_shape(i, len(dims), dims, ranks)
+        core = bufs[i][:int(np.prod(shp, dtype=np.int64))].view(shp)
+        cores.append(core if core.numel() == bufs[i].numel() else core.clone())
+    return cores, ranks, [svals[i, :ranks[i]].copy() for i in range(bonds)]
+
+
+def ttsvd(dense, dims, cutoff=1e-10, cutoff_mode="rsum2", max_bond=None, renorm=None):
+    """Left-canonical MPS cores of ``dense`` (site order); returns (cores, ranks, svals)."""
+    _dev(dense, "dense")
+    dims = [int(d) for d in dims]
+    args, bufs, ranks, svals = _sweep_args(dims, cutoff, cutoff_mode, renorm, max_bond, dense)
+    N.check(N.load_library().ndmps_ttsvd(N.handle(), N.ptr(dense), N.dtype_code(dense.dtype), len(dims), N.i64_array(dims),
+                                         *args), "ndmps_ttsvd")
+    return _sweep_out(bufs, ranks, svals, dims, len(dims) - 1, len(dims))
 
 
 class _DevicePointer:
@@ -282,17 +298,8 @@ def ttsvd_sharded(dense_local, dims_local, world: int, allreduce=None, stop_byte
     torch = _torch()
     _dev(dense_local, "dense_local")
     dims = [int(d) for d in dims_local]
-    L = len(dims)
-    mode = N.CUTOFF_MODES[cutoff_mode]
-    if renorm is None:
-        renorm = {N.CUT_RSUM2: 2, N.CUT_SUM2: 2, N.CUT_RSUM1: 1, N.CUT_SUM1: 1}.get(mode, 0)
     gdims = dims[:-1] + [dims[-1] * int(world)]
-    bounds = bond_bounds(gdims, max_bond)
-    caps = [int(np.prod(core_shape(i, L, gdims, bounds), dtype=np.int64)) for i in range(L)]
-    bufs = [torch.empty(c, dtype=dense_local.dtype, device=dense_local.device) for c in caps]
-    ranks = (C.c_int64 * max(L - 1, 1))()
-    stride = max(bounds) if bounds else 1
-    svals = np.zeros((max(L - 1, 1), stride), dtype=np.float64)
+    args, bufs, ranks, svals = _sweep_args(gdims, cutoff, cutoff_mode, renorm, max_bond, dense_local)
     remainder = torch.empty(dense_local.numel(), dtype=dense_local.dtype, device=dense_local.device)
     sites_done = C.c_int(0)
     rshape = (C.c_int64 * 2)()
@@ -310,21 +317,15 @@ def ttsvd_sharded(dense_local, dims_local, world: int, allreduce=None, stop_byte
     if world > 1 and allreduce is None:
         raise ValueError("ttsvd_sharded: world > 1 needs an allreduce callable")
     rc = N.load_library().ndmps_ttsvd_sharded(
-        N.handle(), N.ptr(dense_local), N.dtype_code(dense_local.dtype), L, N.i64_array(dims), int(world), cb, None,
-        int(stop_bytes), float(cutoff), mode, int(max_bond or 0), int(renorm), N.ptr_array(bufs), N.i64_array(caps), ranks,
-        svals.ctypes.data_as(N.p_f64), stride, C.byref(sites_done), N.ptr(remainder), remainder.numel(), rshape)
+        N.handle(), N.ptr(dense_local), N.dtype_code(dense_local.dtype), len(dims), N.i64_array(dims), int(world), cb,
+        None, int(stop_bytes), *args, C.byref(sites_done), N.ptr(remainder), remainder.numel(), rshape)
     if failure:
         raise failure[0]
     N.check(rc, "ndmps_ttsvd_sharded")
     done = sites_done.value
-    rk = [int(r) for r in ranks][:done]
-    cores = []
-    for i in range(done):                              # done < L - 1: never the last core
-        shp = (gdims[0], rk[0]) if i == 0 else (rk[i - 1], gdims[i], rk[i])
-        n = int(np.prod(shp, dtype=np.int64))
-        cores.append(bufs[i][:n].clone().view(shp))
+    cores, rk, sv = _sweep_out(bufs, ranks, svals, gdims, done, done)    # done < len(dims) - 1: never the last core
     rows, cols = int(rshape[0]), int(rshape[1])
-    return cores, rk, [svals[i, :rk[i]].copy() for i in range(done)], remainder[:rows * cols].view(rows, cols)
+    return cores, rk, sv, remainder[:rows * cols].view(rows, cols)
 
 
 def interleave_shards(gathered, world: int, rows: int, cmid: int, dl: int):
@@ -661,9 +662,7 @@ def roundtrip_host(src: np.ndarray, max_bond=None, cutoff=1e-10, cutoff_mode="rs
         raise ValueError("roundtrip_host expects a float32 or float64 array")
     src = np.ascontiguousarray(src)
     plan = plan_for(tuple(src.shape))
-    mode = N.CUTOFF_MODES[cutoff_mode]
-    if renorm is None:
-        renorm = {N.CUT_RSUM2: 2, N.CUT_SUM2: 2, N.CUT_RSUM1: 1, N.CUT_SUM1: 1}.get(mode, 0)
+    mode, renorm = _trim_mode(cutoff_mode, renorm)
     if out is None:
         out = np.empty_like(src)
     ranks = (C.c_int64 * max(plan.levels - 1, 1))()
@@ -672,7 +671,7 @@ def roundtrip_host(src: np.ndarray, max_bond=None, cutoff=1e-10, cutoff_mode="rs
     bounds = np.zeros((plan.levels, 2), dtype=np.float64)
     N.check(N.load_library().ndmps_roundtrip_host(N.handle(), plan.handle, src.ctypes.data_as(C.c_void_p),
                                                   out.ctypes.data_as(C.c_void_p), code, float(cutoff), mode,
-                                                  int(max_bond or 0), int(renorm), ranks, C.byref(norm),
+                                                  int(max_bond or 0), renorm, ranks, C.byref(norm),
                                                   bounds.ctypes.data_as(N.p_f64)), "ndmps_roundtrip_host")
     if extras is not None:
         extras["norm"] = norm.value
