@@ -26,7 +26,6 @@ void Arena::release() {
 }
 
 int Arena::reset(cudaStream_t stream) {
-    generation++;
     if (cur_total > high_water) high_water = cur_total;
     cur_total = 0;
     if (chunks.size() > 1) {

@@ -119,7 +119,6 @@ struct Arena {
     std::vector<Chunk> chunks;
     size_t high_water = 0;
     size_t cur_total = 0;
-    uint64_t generation = 0;            // bumped by reset(): cached workspace pointers of an older generation are dead
 
     int reset(cudaStream_t stream);
     int alloc(size_t bytes, void** out);
@@ -132,7 +131,7 @@ struct Arena {
     }
     // Hand back everything allocated since mark() without a reset, so that a loop over blocks reuses one block's
     // workspace (stream order makes the reuse safe: a later allocation is written by work enqueued after the last
-    // reader of the earlier one).  The high-water mark keeps the peak; cached pointers of the old generation die.
+    // reader of the earlier one).  The high-water mark keeps the peak.
     struct Mark { std::vector<size_t> used; size_t total = 0; };
     Mark mark() const {
         Mark m;
@@ -144,7 +143,6 @@ struct Arena {
         if (cur_total > high_water) high_water = cur_total;
         for (size_t i = 0; i < chunks.size(); i++) chunks[i].used = i < m.used.size() ? m.used[i] : 0;
         cur_total = m.total;
-        generation++;
     }
 };
 
@@ -167,14 +165,6 @@ struct ndmps_ctx {
     int64_t opt_gram_path = 0;      // 0 auto, 2 SIMT, 3 tcgen05
     int64_t opt_tc = 1;             // tcgen05 contractions for float32 payloads
     int64_t opt_gemm_out_t = 0;     // test hook: ndmps_gemm writes C transposed
-    // int8 digit planes of the unfolding the tcgen05 Gram sliced last (workspace memory: valid until the next ws.reset);
-    // the projection of the same sweep step multiplies the same digits.  exact_host: the device-side "use the FP64 pipe"
-    // flag once it has been copied to the host beside the eigenvalues (-1: not yet known)
-    struct {
-        const void* src = nullptr; int64_t rows = 0, cols = 0, ld = 0; void* digits = nullptr; int64_t ldp = 0, pstride = 0;
-        const int* sc = nullptr; const int* use_exact = nullptr; uint64_t gen = 0; int exact_host = -1;
-    } tc_digits;
-    bool tc_sweep = false;          // set by the sweep while the tcgen05 Gram / projection are admissible (float32, bond cap)
     int64_t opt_gemm_path = 0;      // 0 auto, 2 SIMT
     int64_t opt_permute_path = 0;   // 0 auto, 1 tiles, 2 gather
     int64_t opt_eig_topk = 1;             // leading-eigenpair solver for capped bonds
@@ -239,11 +229,35 @@ int gemm(ndmps_ctx* ctx, int64_t m, int64_t n, int64_t k, double alpha,
          const void* a, int dtype_a, int64_t a_rs, int64_t a_cs,
          const void* b, int dtype_b, int64_t b_rs, int64_t b_cs,
          void* c, int dtype_c, int64_t ldc);
-int gram(ndmps_ctx* ctx, const void* m, int64_t rows, int64_t cols, int64_t ld, int dtype, int side, double* g_dev);
+// C = A B whose float32 payload (`payload` elements, as the caller measures it) is large: on tcgen05 when the shape allows
+int payload_gemm(ndmps_ctx* ctx, int64_t payload, int64_t m, int64_t n, int64_t k,
+                 const void* a, int dtype_a, int64_t a_rs, int64_t a_cs,
+                 const void* b, int dtype_b, int64_t b_rs, int64_t b_cs,
+                 void* c, int dtype_c, int64_t ldc);
+// The int8 digit planes ([digit][rows][ldp], planes pstride apart; workspace memory) the sliced-integer Gram made of an
+// unfolding (rows x cols), kept by the sweep step whose projection multiplies the same digits.  use_exact: the device-side
+// "use the FP64 pipe" flag; exact_host: its value once it has been copied to the host beside the eigenvalues (-1: not yet)
+struct TcDigits {
+    int8_t* digits = nullptr;
+    const int* sc = nullptr;            // power-of-two row scales
+    const int* use_exact = nullptr;
+    int64_t ldp = 0, pstride = 0, rows = 0, cols = 0;
+    int exact_host = -1;
+};
+// tc != nullptr: the caller accepts the sliced-integer Gram on tcgen05 and takes its digits (when it ran) in *tc
+int gram(ndmps_ctx* ctx, const void* m, int64_t rows, int64_t cols, int64_t ld, int dtype, int side, double* g_dev,
+         TcDigits* tc = nullptr);
+// FP64 tensor-pipe paths (gemm_dmma.cu, gram_dmma.cu); *done = false when the shape is not eligible.
+// run_flag (device, optional): the Gram's kernels return at once unless run_flag[0] != 0
+int gemm_dmma(ndmps_ctx* ctx, int64_t m, int64_t n, int64_t k, double alpha, const void* a, int dtype_a, int64_t a_rs,
+              int64_t a_cs, const void* b, int dtype_b, int64_t b_rs, int64_t b_cs, void* c, int dtype_c, int64_t ldc,
+              bool* done);
+int gram_dmma(ndmps_ctx* ctx, const void* mat, int64_t rows, int64_t cols, int64_t ld, int dtype, double* g_dev, bool* done,
+              const int* run_flag = nullptr);
 // tcgen05 paths (tc_gemm.cu); *done = false when the shape is not eligible
-int gram_tc(ndmps_ctx* ctx, const void* mat, int64_t rows, int64_t cols, int64_t ld, int dtype, double* g_dev, bool* done);
-int proj_tc_digits(ndmps_ctx* ctx, const void* mat, int64_t D, int64_t C, int64_t ld, const double* P, int64_t r, void* T, int dtype_t,
-                   int64_t ldt, bool* done);
+int gram_tc(ndmps_ctx* ctx, const void* mat, int64_t rows, int64_t cols, int64_t ld, int dtype, double* g_dev, TcDigits* dg,
+            bool* done);
+int proj_tc_digits(ndmps_ctx* ctx, const TcDigits& dg, const double* P, int64_t r, void* T, int dtype_t, int64_t ldt, bool* done);
 int gemm_tc(ndmps_ctx* ctx, int64_t m, int64_t n, int64_t k, double alpha, const void* a, int dtype_a, int64_t a_rs, int64_t a_cs,
             const void* b, int dtype_b, int64_t b_rs, int64_t b_cs, void* c, int dtype_c, int64_t ldc, bool out_t, bool* done);
 // tol_override > 0 loosens the relative off-diagonal threshold (float32 payloads do not need 1e-15)
@@ -305,6 +319,19 @@ __device__ __forceinline__ double warp_min(double v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v = fmin(v, __shfl_xor_sync(0xffffffffu, v, o));
     return v;
+}
+// D (8 x 8, two per thread) += A (8 x 4) B (4 x 8) on the FP64 tensor pipe, one element of A and of B per thread
+__device__ __forceinline__ void mma_f64(double& d0, double& d1, double a, double b) {
+    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
+                 : "+d"(d0), "+d"(d1)
+                 : "d"(a), "d"(b));
+}
+// tile index -> (ti, tj) with tj >= ti, tiles enumerated row by row over the upper triangle
+__device__ __forceinline__ void upper_tile(int t, int nt, int& ti, int& tj) {
+    int row = 0, left = t;
+    while (left >= nt - row) { left -= nt - row; row++; }
+    ti = row;
+    tj = row + left;
 }
 // block reductions; `scratch` must hold 32 doubles; result valid in thread 0
 __device__ __forceinline__ double block_sum(double v, double* scratch) {

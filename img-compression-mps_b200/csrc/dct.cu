@@ -49,13 +49,7 @@ int dct_matrix(ndmps_ctx* ctx, int64_t n, int inverse, double** C_out) {
 // forward: y[l, k] = sum_i x[l, i] C[k, i] = sum_i x[l, i] Ct[i, k]; inverse: x[l, i] = sum_k y[l, k] C[k, i].  Both are
 // dst = src . C with the matrix dct_matrix built for the direction.
 int dct_lines(ndmps_ctx* ctx, const void* src, void* dst, int64_t lines, int64_t n, int dtype, const double* C) {
-    if (ctx->opt_tc && dtype == NDMPS_F32 && lines * n >= (int64_t(1) << 20)) {
-        // float32 payload: the line x cosine-matrix product on tcgen05 (bf16x3 planes, tc_gemm.cu)
-        bool on_tc = false;
-        NDMPS_TRY(gemm_tc(ctx, lines, n, n, 1.0, src, dtype, n, 1, C, NDMPS_F64, n, 1, dst, dtype, n, false, &on_tc));
-        if (on_tc) return NDMPS_OK;
-    }
-    return gemm(ctx, lines, n, n, 1.0, src, dtype, n, 1, C, NDMPS_F64, n, 1, dst, dtype, n);
+    return payload_gemm(ctx, lines * n, lines, n, n, src, dtype, n, 1, C, NDMPS_F64, n, 1, dst, dtype, n);
 }
 
 }  // namespace ndmps
@@ -91,12 +85,8 @@ int ndmps_idct_block_mean_last_axis(ndmps_ctx_t* ctx, const void* src, void* dst
     int64_t want = (n * m + 255) / 256, cap = (int64_t)ctx->sm_count * 8;
     dct_block_mean_matrix_kernel<<<(int)(want < cap ? want : cap), 256, 0, ctx->stream>>>(B, n, block);
     NDMPS_LAUNCH_CHECK(ctx);
-    if (ctx->opt_tc && dtype == NDMPS_F32 && lines * n >= (int64_t(1) << 20)) {   // same rule as ndmps_dct_last_axis
-        bool on_tc = false;
-        NDMPS_TRY(gemm_tc(ctx, lines, m, n, 1.0, src, dtype, n, 1, B, NDMPS_F64, m, 1, dst, dtype, m, false, &on_tc));
-        if (on_tc) return NDMPS_OK;
-    }
-    return gemm(ctx, lines, m, n, 1.0, src, dtype, n, 1, B, NDMPS_F64, m, 1, dst, dtype, m);
+    // the payload is the input (lines x n), as for ndmps_dct_last_axis
+    return payload_gemm(ctx, lines * n, lines, m, n, src, dtype, n, 1, B, NDMPS_F64, m, 1, dst, dtype, m);
 }
 
 }  // extern "C"

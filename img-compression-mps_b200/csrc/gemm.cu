@@ -138,10 +138,6 @@ splitk_reduce_kernel(const double* __restrict__ partial, int splits, int64_t M, 
     }
 }
 
-int gemm_dmma(ndmps_ctx* ctx, int64_t m, int64_t n, int64_t k, double alpha, const void* a, int dtype_a, int64_t a_rs,
-              int64_t a_cs, const void* b, int dtype_b, int64_t b_rs, int64_t b_cs, void* c, int dtype_c, int64_t ldc,
-              bool* done);
-
 int gemm(ndmps_ctx* ctx, int64_t m, int64_t n, int64_t k, double alpha,
          const void* a, int dtype_a, int64_t a_rs, int64_t a_cs,
          const void* b, int dtype_b, int64_t b_rs, int64_t b_cs,
@@ -157,7 +153,7 @@ int gemm(ndmps_ctx* ctx, int64_t m, int64_t n, int64_t k, double alpha,
         if (done) return NDMPS_OK;
         NDMPS_REQUIRE(ctx->opt_gemm_out_t == 0, "gemm: transposed output needs the tcgen05 path (shape not eligible)");
     }
-    {   // large row-major products go to the FP64 tensor pipe (gemm_dmma.cu)
+    if (ctx->opt_gemm_path != 2) {   // large row-major products go to the FP64 tensor pipe (gemm_dmma.cu)
         bool done = false;
         NDMPS_TRY(gemm_dmma(ctx, m, n, k, alpha, a, dtype_a, a_rs, a_cs, b, dtype_b, b_rs, b_cs, c, dtype_c, ldc, &done));
         if (done) return NDMPS_OK;
@@ -201,15 +197,26 @@ int gemm(ndmps_ctx* ctx, int64_t m, int64_t n, int64_t k, double alpha,
     return NDMPS_OK;
 }
 
-int gram_dmma(ndmps_ctx* ctx, const void* mat, int64_t rows, int64_t cols, int64_t ld, int dtype, double* g_dev, bool* done,
-              const int* run_flag = nullptr);
+// float32 payloads from 2^20 elements on: the product on tcgen05 (bf16x3 planes, tc_gemm.cu)
+int payload_gemm(ndmps_ctx* ctx, int64_t payload, int64_t m, int64_t n, int64_t k,
+                 const void* a, int dtype_a, int64_t a_rs, int64_t a_cs,
+                 const void* b, int dtype_b, int64_t b_rs, int64_t b_cs,
+                 void* c, int dtype_c, int64_t ldc) {
+    if (ctx->opt_tc && dtype_c == NDMPS_F32 && payload >= (int64_t(1) << 20)) {
+        bool done = false;
+        NDMPS_TRY(gemm_tc(ctx, m, n, k, 1.0, a, dtype_a, a_rs, a_cs, b, dtype_b, b_rs, b_cs, c, dtype_c, ldc, false, &done));
+        if (done) return NDMPS_OK;
+    }
+    return gemm(ctx, m, n, k, 1.0, a, dtype_a, a_rs, a_cs, b, dtype_b, b_rs, b_cs, c, dtype_c, ldc);
+}
 
-int gram(ndmps_ctx* ctx, const void* mat, int64_t rows, int64_t cols, int64_t ld, int dtype, int side, double* g_dev) {
-    if (side == 0 && (ctx->opt_gram_path == 3 || (ctx->opt_gram_path == 0 && ctx->opt_tc && ctx->tc_sweep))) {
+int gram(ndmps_ctx* ctx, const void* mat, int64_t rows, int64_t cols, int64_t ld, int dtype, int side, double* g_dev, TcDigits* tc) {
+    if (side == 0 && (ctx->opt_gram_path == 3 || (ctx->opt_gram_path == 0 && tc != nullptr))) {
         // sliced-integer Gram on tcgen05 kind::i8 (tc_gemm.cu): float32 unfoldings of a capped sweep.  Exact accumulation,
         // five 7-bit digits; rows too heavy-tailed for five digits go to the FP64-pipe kernel through a device-side flag
+        TcDigits dropped;
         bool done = false;
-        NDMPS_TRY(gram_tc(ctx, mat, rows, cols, ld, dtype, g_dev, &done));
+        NDMPS_TRY(gram_tc(ctx, mat, rows, cols, ld, dtype, g_dev, tc ? tc : &dropped, &done));
         if (done) return NDMPS_OK;
     }
     if (side == 0 && ctx->opt_gram_path != 2) {   // FP64 tensor-pipe path when the shape allows (gram_dmma.cu)

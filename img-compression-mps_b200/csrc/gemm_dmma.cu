@@ -15,12 +15,6 @@ namespace gdm {
 
 constexpr int BN = 128, BK = 16, LDA = BK + 4, LDB = BN + 4;   // strides chosen so the fragment reads are bank-conflict free
 
-__device__ __forceinline__ void mma_f64(double& d0, double& d1, double a, double b) {
-    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
-                 : "+d"(d0), "+d"(d1)
-                 : "d"(a), "d"(b));
-}
-
 template <int BM, class TA, class TB, class TC>
 __global__ void __launch_bounds__(BM * 4, BM == 64 ? 2 : 1)
 gemm_dmma_kernel(int64_t M, int64_t N, int64_t K, const TA* __restrict__ A, int64_t lda, const TB* __restrict__ B, int64_t ldb,
@@ -138,7 +132,6 @@ int gemm_dmma(ndmps_ctx* ctx, int64_t m, int64_t n, int64_t k, double alpha, con
               int64_t a_cs, const void* b, int dtype_b, int64_t b_rs, int64_t b_cs, void* c, int dtype_c, int64_t ldc,
               bool* done) {
     *done = false;
-    if (ctx->opt_gemm_path == 2) return NDMPS_OK;
     if (a_cs != 1 || b_cs != 1 || m < 48 || n < 64 || k < 4) return NDMPS_OK;   // n = 64: half of the 128-wide tile idles, still ahead of SIMT
     const int64_t tiles64 = ((m + 63) / 64) * ((n + gdm::BN - 1) / gdm::BN);
     if (tiles64 < ctx->sm_count) return NDMPS_OK;          // would need split-K: SIMT path has it

@@ -26,20 +26,6 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N)); }
 
-__device__ __forceinline__ void mma_f64(double& d0, double& d1, double a, double b) {
-    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
-                 : "+d"(d0), "+d"(d1)
-                 : "d"(a), "d"(b));
-}
-
-// tile index -> (ti, tj) with tj >= ti, tiles enumerated row by row over the upper triangle
-__device__ __forceinline__ void upper_tile(int t, int nt, int& ti, int& tj) {
-    int row = 0, left = t;
-    while (left >= nt - row) { left -= nt - row; row++; }
-    ti = row;
-    tj = row + left;
-}
-
 __global__ void __launch_bounds__(THREADS, 1)
 gram_dmma_kernel(const float* __restrict__ M, int m, int64_t K, int64_t ld, int nt, int64_t k_per, double* __restrict__ partial,
                  const int* __restrict__ run_flag) {
@@ -149,7 +135,6 @@ gram_dmma_reduce_kernel(const double* __restrict__ partial, int m, int nt, int n
 }  // namespace dmma
 
 // returns NDMPS_OK and sets *done = true when the fast path ran
-// run_flag (device, optional): the kernels return at once unless run_flag[0] != 0
 int gram_dmma(ndmps_ctx* ctx, const void* mat, int64_t rows, int64_t cols, int64_t ld, int dtype, double* g_dev, bool* done,
               const int* run_flag) {
     using namespace dmma;

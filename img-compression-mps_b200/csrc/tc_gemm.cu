@@ -141,13 +141,6 @@ __host__ __device__ constexpr uint32_t instr_desc(int m, int n, int a_mn, int b_
            ((uint32_t)(m >> 4) << 24);
 }
 
-__device__ __forceinline__ void upper_tile(int t, int nt, int& ti, int& tj) {
-    int row = 0, left = t;
-    while (left >= nt - row) { left -= nt - row; row++; }
-    ti = row;
-    tj = row + left;
-}
-
 // ---------------------------------------------------------------------------------------------
 // float32 / float64 -> three bfloat16 planes (x = h + m + l, every step round-to-nearest)
 // ---------------------------------------------------------------------------------------------
@@ -160,9 +153,9 @@ __device__ __forceinline__ void split3(T x, __nv_bfloat16& h, __nv_bfloat16& m, 
     l = __float2bfloat16_rn((float)r);
 }
 
-// src: rows x cols (row stride ld_src, optional transpose: element (r, c) read from src[c * ld_src + r]);
-// dst: bf16[3][rows][ldp], columns cols..ldp-1 zeroed.  Eight elements per thread (16-byte stores).
-template <class T, bool TRANSPOSE>
+// src: rows x cols (row stride ld_src); dst: bf16[3][rows][ldp], columns cols..ldp-1 zeroed.  Eight elements per thread
+// (16-byte stores).
+template <class T>
 __global__ void __launch_bounds__(256)
 split_planes_kernel(const T* __restrict__ src, int64_t rows, int64_t cols, int64_t ld_src, double alpha,
                     __nv_bfloat16* __restrict__ dst, int64_t ldp, int64_t plane_stride) {
@@ -171,18 +164,13 @@ split_planes_kernel(const T* __restrict__ src, int64_t rows, int64_t cols, int64
         const int64_t r = i / groups, c0 = (i - r * groups) << 3;
         __align__(16) __nv_bfloat16 h[8], m[8], l[8];
         T v[8];
-        if constexpr (!TRANSPOSE) {
-            const T* p = src + r * ld_src + c0;
-            if (sizeof(T) == 4 && c0 + 8 <= cols && ((reinterpret_cast<uintptr_t>(p) & 15) == 0)) {
-                const float4 a = __ldcs(reinterpret_cast<const float4*>(p)), b = __ldcs(reinterpret_cast<const float4*>(p) + 1);
-                v[0] = (T)a.x; v[1] = (T)a.y; v[2] = (T)a.z; v[3] = (T)a.w; v[4] = (T)b.x; v[5] = (T)b.y; v[6] = (T)b.z; v[7] = (T)b.w;
-            } else {
-#pragma unroll
-                for (int j = 0; j < 8; j++) v[j] = c0 + j < cols ? p[j] : (T)0;
-            }
+        const T* p = src + r * ld_src + c0;
+        if (sizeof(T) == 4 && c0 + 8 <= cols && ((reinterpret_cast<uintptr_t>(p) & 15) == 0)) {
+            const float4 a = __ldcs(reinterpret_cast<const float4*>(p)), b = __ldcs(reinterpret_cast<const float4*>(p) + 1);
+            v[0] = (T)a.x; v[1] = (T)a.y; v[2] = (T)a.z; v[3] = (T)a.w; v[4] = (T)b.x; v[5] = (T)b.y; v[6] = (T)b.z; v[7] = (T)b.w;
         } else {
 #pragma unroll
-            for (int j = 0; j < 8; j++) v[j] = c0 + j < cols ? src[(c0 + j) * ld_src + r] : (T)0;
+            for (int j = 0; j < 8; j++) v[j] = c0 + j < cols ? p[j] : (T)0;
         }
 #pragma unroll
         for (int j = 0; j < 8; j++) split3<T>(v[j] * (T)alpha, h[j], m[j], l[j]);
@@ -899,28 +887,37 @@ static EncodeTiledFn encode_fn() {
     return fn;
 }
 
-// planes: bf16[3][rows][ldp]; box = 64 columns x box_rows rows x 1 plane, 128-byte swizzle, zero fill outside
-static int make_plane_map(CUtensorMap* map, const void* planes, int64_t rows, int64_t cols, int64_t ldp, int64_t plane_stride,
-                          int box_rows) {
+// 3-d tensor map of a stack of planes: dims {cols, rows, planes}, strides {row, plane} in bytes, zero fill outside.
+// `what` names the operand in the error text.
+static int encode_map(CUtensorMap* map, CUtensorMapDataType type, const void* base, const cuuint64_t (&dims)[3],
+                      const cuuint64_t (&strides)[2], const cuuint32_t (&box)[3], CUtensorMapSwizzle swizzle, const char* what) {
     EncodeTiledFn fn = encode_fn();
     if (!fn) { set_error("tc: cuTensorMapEncodeTiled is not available from the driver"); return NDMPS_ERR_CUDA; }
-    const cuuint64_t dims[3] = {(cuuint64_t)cols, (cuuint64_t)rows, 3};
-    const cuuint64_t strides[2] = {(cuuint64_t)ldp * 2, (cuuint64_t)plane_stride * 2};
-    const cuuint32_t box[3] = {64, (cuuint32_t)box_rows, 1};
     const cuuint32_t estr[3] = {1, 1, 1};
-    CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(planes), dims, strides, box, estr,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { set_error("tc: cuTensorMapEncodeTiled failed (%d) rows %lld cols %lld ld %lld", (int)r, (long long)rows, (long long)cols, (long long)ldp); return NDMPS_ERR_CUDA; }
+    CUresult r = fn(map, type, 3, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle,
+                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) {
+        set_error("tc: cuTensorMapEncodeTiled (%s) failed (%d): %llu x %llu x %llu, row pitch %llu B", what, (int)r,
+                  (unsigned long long)dims[0], (unsigned long long)dims[1], (unsigned long long)dims[2], (unsigned long long)strides[0]);
+        return NDMPS_ERR_CUDA;
+    }
     return NDMPS_OK;
+}
+
+// planes: bf16[3][rows][ldp]; box = 64 columns x box_rows rows x 1 plane, 128-byte swizzle
+static int make_plane_map(CUtensorMap* map, const void* planes, int64_t rows, int64_t cols, int64_t ldp, int64_t plane_stride,
+                          int box_rows) {
+    return encode_map(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, planes, {(cuuint64_t)cols, (cuuint64_t)rows, 3},
+                      {(cuuint64_t)ldp * 2, (cuuint64_t)plane_stride * 2}, {64, (cuuint32_t)box_rows, 1}, CU_TENSOR_MAP_SWIZZLE_128B,
+                      "bf16x3 planes");
 }
 
 static inline int64_t round8(int64_t x) { return (x + 7) & ~int64_t(7); }
 
 }  // namespace tc
 
-// Split `src` (rows x cols, optionally read transposed) into planes in the workspace.
-int tc_split(ndmps_ctx* ctx, const void* src, int dtype, int64_t rows, int64_t cols, int64_t ld_src, bool transpose, double alpha,
+// Split `src` (rows x cols, row stride ld_src) into planes in the workspace.
+int tc_split(ndmps_ctx* ctx, const void* src, int dtype, int64_t rows, int64_t cols, int64_t ld_src, double alpha,
              __nv_bfloat16** planes_out, int64_t* ldp_out, int64_t* plane_stride_out) {
     using namespace tc;
     const int64_t ldp = round8(cols), pstride = rows * ldp;
@@ -929,10 +926,10 @@ int tc_split(ndmps_ctx* ctx, const void* src, int dtype, int64_t rows, int64_t c
     const int64_t total = rows * (ldp >> 3);
     int64_t want = (total + 255) / 256, cap = (int64_t)ctx->sm_count * 16;
     const int g = (int)(want < 1 ? 1 : (want < cap ? want : cap));
-#define NDMPS_SPLIT(T, TR) split_planes_kernel<T, TR><<<g, 256, 0, ctx->stream>>>((const T*)src, rows, cols, ld_src, alpha, planes, ldp, pstride)
-    if (dtype == NDMPS_F32) { if (transpose) NDMPS_SPLIT(float, true); else NDMPS_SPLIT(float, false); }
-    else { if (transpose) NDMPS_SPLIT(double, true); else NDMPS_SPLIT(double, false); }
-#undef NDMPS_SPLIT
+    if (dtype == NDMPS_F32)
+        split_planes_kernel<float><<<g, 256, 0, ctx->stream>>>((const float*)src, rows, cols, ld_src, alpha, planes, ldp, pstride);
+    else
+        split_planes_kernel<double><<<g, 256, 0, ctx->stream>>>((const double*)src, rows, cols, ld_src, alpha, planes, ldp, pstride);
     NDMPS_LAUNCH_CHECK(ctx);
     *planes_out = planes;
     *ldp_out = ldp;
@@ -940,13 +937,12 @@ int tc_split(ndmps_ctx* ctx, const void* src, int dtype, int64_t rows, int64_t c
     return NDMPS_OK;
 }
 
-int gram_dmma(ndmps_ctx* ctx, const void* mat, int64_t rows, int64_t cols, int64_t ld, int dtype, double* g_dev, bool* done,
-              const int* run_flag);
-
 // G = M M^T from the float32 unfolding `mat` (rows x cols, row stride ld).  *done = false: shape not eligible.
 // Launches BOTH the sliced-integer tensor-core Gram and the exact FP64-pipe Gram; a device-side flag set by the
 // row-scaling pass lets exactly one of them run (the other returns at once), so no host round trip is needed.
-int gram_tc(ndmps_ctx* ctx, const void* mat, int64_t rows, int64_t cols, int64_t ld, int dtype, double* g_dev, bool* done) {
+// *dg receives the digits and the flag, for a projection of the same unfolding (proj_tc_digits).
+int gram_tc(ndmps_ctx* ctx, const void* mat, int64_t rows, int64_t cols, int64_t ld, int dtype, double* g_dev, TcDigits* dg,
+            bool* done) {
     using namespace tc;
     *done = false;
     if (dtype != NDMPS_F32 || rows < 64 || rows > 4096 || cols < 2048) return NDMPS_OK;
@@ -983,17 +979,8 @@ int gram_tc(ndmps_ctx* ctx, const void* mat, int64_t rows, int64_t cols, int64_t
     }
     // 3. digit products on the integer tensor cores
     CUtensorMap map;
-    {
-        EncodeTiledFn fn = encode_fn();
-        if (!fn) { set_error("tc: cuTensorMapEncodeTiled is not available from the driver"); return NDMPS_ERR_CUDA; }
-        const cuuint64_t dims[3] = {(cuuint64_t)cols, (cuuint64_t)rows, (cuuint64_t)I8_PLANES};
-        const cuuint64_t strides[2] = {(cuuint64_t)ldp, (cuuint64_t)pstride};
-        const cuuint32_t box[3] = {(cuuint32_t)I8_BK, 64, 1};
-        const cuuint32_t estr[3] = {1, 1, 1};
-        CUresult r = fn(&map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, digits, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) { set_error("tc: cuTensorMapEncodeTiled (int8 digits) failed (%d)", (int)r); return NDMPS_ERR_CUDA; }
-    }
+    NDMPS_TRY(encode_map(&map, CU_TENSOR_MAP_DATA_TYPE_UINT8, digits, {(cuuint64_t)cols, (cuuint64_t)rows, (cuuint64_t)I8_PLANES},
+                         {(cuuint64_t)ldp, (cuuint64_t)pstride}, {(cuuint32_t)I8_BK, 64, 1}, CU_TENSOR_MAP_SWIZZLE_64B, "int8 digits"));
     const int m = (int)rows, ntr = (m + TILE - 1) / TILE, ntc = (m + I8_TN - 1) / I8_TN;
     int ntiles = 0;
     for (int ti = 0; ti < ntr; ti++) ntiles += ntc - 2 * ti > 0 ? ntc - 2 * ti : 0;
@@ -1014,10 +1001,7 @@ int gram_tc(ndmps_ctx* ctx, const void* mat, int64_t rows, int64_t cols, int64_t
     dim3 rgrid(8, (unsigned)ntiles);
     gram_i8_reduce_kernel<<<rgrid, 256, 0, ctx->stream>>>(partial, m, ntc, ntiles, (int)splits, use_exact, g_dev);
     NDMPS_LAUNCH_CHECK(ctx);
-    // the projection of this sweep step can reuse the digits (proj_tc_digits below)
-    ctx->tc_digits.src = mat; ctx->tc_digits.rows = rows; ctx->tc_digits.cols = cols; ctx->tc_digits.ld = ld;
-    ctx->tc_digits.digits = digits; ctx->tc_digits.ldp = ldp; ctx->tc_digits.pstride = pstride; ctx->tc_digits.sc = sc;
-    ctx->tc_digits.use_exact = use_exact; ctx->tc_digits.gen = ctx->ws.generation; ctx->tc_digits.exact_host = -1;
+    *dg = {digits, sc, use_exact, ldp, pstride, rows, cols};
     // 4. the exact kernel: runs only when the flag is set
     bool exact_ok = false;
     NDMPS_TRY(gram_dmma(ctx, mat, rows, cols, ld, dtype, g_dev, &exact_ok, use_exact));
@@ -1027,17 +1011,13 @@ int gram_tc(ndmps_ctx* ctx, const void* mat, int64_t rows, int64_t cols, int64_t
 }
 
 // T (r x C, row-major ldt) = P^T M on the digit planes gram_tc made of M (rows D x cols C), P: D x r float64 row-major.
-// *done = false: no digits for this unfolding (the Gram fell back to the FP64 pipe, or another matrix) - the caller
-// takes the bf16x3 route.  The exactness flag must have reached the host (ttsvd copies it beside the eigenvalues).
-int proj_tc_digits(ndmps_ctx* ctx, const void* mat, int64_t D, int64_t C, int64_t ld, const double* P, int64_t r, void* T, int dtype_t,
-                   int64_t ldt, bool* done) {
+// *done = false: the digits are not known to be exact (the Gram fell back to the FP64 pipe, or did not slice M) - the
+// caller takes the bf16x3 route.  The exactness flag must have reached the host (ttsvd copies it beside the eigenvalues).
+int proj_tc_digits(ndmps_ctx* ctx, const TcDigits& dg, const double* P, int64_t r, void* T, int dtype_t, int64_t ldt, bool* done) {
     using namespace tc;
     *done = false;
-    const auto& dg = ctx->tc_digits;
-    if (!dg.digits || dg.gen != ctx->ws.generation || dg.src != mat || dg.rows != D || dg.cols != C || dg.ld != ld) return NDMPS_OK;
+    const int64_t D = dg.rows, C = dg.cols;
     if (dg.exact_host != 0 || D > 4096 || r < 1 || C < TILE) return NDMPS_OK;
-    EncodeTiledFn fn = encode_fn();
-    if (!fn) { set_error("tc: cuTensorMapEncodeTiled is not available from the driver"); return NDMPS_ERR_CUDA; }
     // digits of the scaled columns of P: [digit][i][k], k padded to 16
     const int64_t ldk = (D + 15) & ~int64_t(15), bstride = r * ldk;
     int8_t* bdig = nullptr;
@@ -1047,24 +1027,11 @@ int proj_tc_digits(ndmps_ctx* ctx, const void* mat, int64_t D, int64_t C, int64_
     split_i8_proj_kernel<<<(unsigned)r, 256, 0, ctx->stream>>>(P, D, r, dg.sc, bdig, ldk, bstride, tcs);
     NDMPS_LAUNCH_CHECK(ctx);
     CUtensorMap map_y, map_b;
-    {
-        const cuuint64_t dims[3] = {(cuuint64_t)C, (cuuint64_t)D, (cuuint64_t)I8_PLANES};
-        const cuuint64_t strides[2] = {(cuuint64_t)dg.ldp, (cuuint64_t)dg.pstride};
-        const cuuint32_t box[3] = {(cuuint32_t)TILE, (cuuint32_t)I8_BK, 1};
-        const cuuint32_t estr[3] = {1, 1, 1};
-        CUresult rc = fn(&map_y, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, dg.digits, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                         CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (rc != CUDA_SUCCESS) { set_error("tc: cuTensorMapEncodeTiled (projection digits) failed (%d)", (int)rc); return NDMPS_ERR_CUDA; }
-    }
-    {
-        const cuuint64_t dims[3] = {(cuuint64_t)D, (cuuint64_t)r, (cuuint64_t)I8_PLANES};
-        const cuuint64_t strides[2] = {(cuuint64_t)ldk, (cuuint64_t)bstride};
-        const cuuint32_t box[3] = {(cuuint32_t)I8_BK, 64, 1};
-        const cuuint32_t estr[3] = {1, 1, 1};
-        CUresult rc = fn(&map_b, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, bdig, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                         CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (rc != CUDA_SUCCESS) { set_error("tc: cuTensorMapEncodeTiled (projector digits) failed (%d)", (int)rc); return NDMPS_ERR_CUDA; }
-    }
+    NDMPS_TRY(encode_map(&map_y, CU_TENSOR_MAP_DATA_TYPE_UINT8, dg.digits, {(cuuint64_t)C, (cuuint64_t)D, (cuuint64_t)I8_PLANES},
+                         {(cuuint64_t)dg.ldp, (cuuint64_t)dg.pstride}, {(cuuint32_t)TILE, (cuuint32_t)I8_BK, 1}, CU_TENSOR_MAP_SWIZZLE_128B,
+                         "projection digits"));
+    NDMPS_TRY(encode_map(&map_b, CU_TENSOR_MAP_DATA_TYPE_UINT8, bdig, {(cuuint64_t)D, (cuuint64_t)r, (cuuint64_t)I8_PLANES},
+                         {(cuuint64_t)ldk, (cuuint64_t)bstride}, {(cuuint32_t)I8_BK, 64, 1}, CU_TENSOR_MAP_SWIZZLE_64B, "projector digits"));
     dim3 grid((unsigned)((C + TILE - 1) / TILE), (unsigned)((r + I8_TN - 1) / I8_TN));
     if (dtype_t == NDMPS_F32) {
         NDMPS_TRY(raise_dynamic_smem((const void*)proj_i8_kernel<float>, ctx->device, ProjI8Smem::TOTAL));
@@ -1110,10 +1077,10 @@ int gemm_tc(ndmps_ctx* ctx, int64_t m, int64_t n, int64_t k, double alpha, const
     // plane matrices as stored: K-major A planes are [m][k]; MN-major A planes are [k][m]; same for B with n
     __nv_bfloat16 *pa = nullptr, *pb = nullptr;
     int64_t lda = 0, sa = 0, ldb = 0, sb = 0;
-    if (a_mn) NDMPS_TRY(tc_split(ctx, a, dtype_a, k, m, a_cs, false, alpha, &pa, &lda, &sa));
-    else NDMPS_TRY(tc_split(ctx, a, dtype_a, m, k, a_rs, false, alpha, &pa, &lda, &sa));
-    if (b_mn) NDMPS_TRY(tc_split(ctx, b, dtype_b, k, n, b_rs, false, 1.0, &pb, &ldb, &sb));
-    else NDMPS_TRY(tc_split(ctx, b, dtype_b, n, k, b_cs, false, 1.0, &pb, &ldb, &sb));
+    if (a_mn) NDMPS_TRY(tc_split(ctx, a, dtype_a, k, m, a_cs, alpha, &pa, &lda, &sa));
+    else NDMPS_TRY(tc_split(ctx, a, dtype_a, m, k, a_rs, alpha, &pa, &lda, &sa));
+    if (b_mn) NDMPS_TRY(tc_split(ctx, b, dtype_b, k, n, b_rs, 1.0, &pb, &ldb, &sb));
+    else NDMPS_TRY(tc_split(ctx, b, dtype_b, n, k, b_cs, 1.0, &pb, &ldb, &sb));
     CUtensorMap ma, mb;
     if (a_mn) NDMPS_TRY(make_plane_map(&ma, pa, k, m, lda, sa, 64));
     else NDMPS_TRY(make_plane_map(&ma, pa, m, k, lda, sa, TILE));

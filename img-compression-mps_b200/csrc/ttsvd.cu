@@ -192,16 +192,16 @@ static double renorm_factor(const double* s, int64_t n, int64_t keep, int power)
 
 // Copy `count` doubles from the device into the pinned scratch and wait for them.  The tcgen05 Gram decides ON THE
 // DEVICE whether its digits are exact enough (tc_gemm.cu); the projection needs that answer on the host to pick its
-// kernel.  While it is pending, the 4-byte flag rides along in an unused slot of the scratch before the same wait.
-static int read_back(ndmps_ctx* ctx, const double* src, int64_t count) {
+// kernel.  While it is pending (dg: the Gram's digits, optional), the 4-byte flag rides along in an unused slot of the
+// scratch before the same wait.
+static int read_back(ndmps_ctx* ctx, const double* src, int64_t count, TcDigits* dg) {
     const size_t slot = (size_t)count + 8;
     NDMPS_TRY(ensure_pinned(ctx, (size_t)count + 64));
     NDMPS_TRY(readback(ctx, ctx->pinned, src, (size_t)count * sizeof(double)));
-    auto& dg = ctx->tc_digits;
-    const bool flag = dg.use_exact != nullptr && dg.gen == ctx->ws.generation && dg.exact_host < 0;
-    if (flag) NDMPS_TRY(readback(ctx, ctx->pinned + slot, dg.use_exact, sizeof(int)));
+    const bool flag = dg != nullptr && dg->use_exact != nullptr && dg->exact_host < 0;
+    if (flag) NDMPS_TRY(readback(ctx, ctx->pinned + slot, dg->use_exact, sizeof(int)));
     NDMPS_CUDA_TRY(stream_wait(ctx));
-    if (flag) dg.exact_host = *reinterpret_cast<const int*>(ctx->pinned + slot) != 0 ? 1 : 0;
+    if (flag) dg->exact_host = *reinterpret_cast<const int*>(ctx->pinned + slot) != 0 ? 1 : 0;
     return NDMPS_OK;
 }
 
@@ -221,8 +221,8 @@ struct Bond { std::vector<double> sv; int64_t n = 0; double f = 1.0; };   // sin
 // difference, and lambda_k must be well above the absolute error floor of the tridiagonal
 // reduction (~ n eps lambda_1).  Anything else leaves *b as it is and the caller runs the full
 // solver, so ranks never depend on which solver ran.  U: mj x mj buffer, eigenvector t in column t.
-static int capped_eigh(ndmps_ctx* ctx, const double* Gj, int64_t mj, int64_t nmax, const TrimOpts& opt, double* evals_dev,
-                       double* U, Bond* b) {
+static int capped_eigh(ndmps_ctx* ctx, const double* Gj, int64_t mj, int64_t nmax, const TrimOpts& opt, TcDigits* dg,
+                       double* evals_dev, double* U, Bond* b) {
     const int64_t k = opt.max_bond;
     if (!ctx->opt_eig_topk || k <= 0 || mj < 4 * k || mj < 96 || nmax <= k) return NDMPS_OK;
     const bool sum2 = opt.mode == NDMPS_CUT_SUM2 || opt.mode == NDMPS_CUT_RSUM2;
@@ -233,7 +233,7 @@ static int capped_eigh(ndmps_ctx* ctx, const double* Gj, int64_t mj, int64_t nma
     bool done = false;
     { StageScope sc(ctx, ST_EIG); NDMPS_TRY(eigh_topk(ctx, Gj, mj, k, out, U, mj, &done)); }
     if (!done) return NDMPS_OK;
-    NDMPS_TRY(read_back(ctx, out, k + 2));
+    NDMPS_TRY(read_back(ctx, out, k + 2, dg));
     const double* ev = ctx->pinned;
     const double trace = ev[k], rank_loss = ev[k + 1];
     double kept = 0.0;
@@ -258,14 +258,15 @@ static int capped_eigh(ndmps_ctx* ctx, const double* Gj, int64_t mj, int64_t nma
 }
 
 // The truncation of one bond with one host wait: evals (m) and U (m x m, eigenvector t in column t) of its float64 Gram
-// matrix G on the device, *b on the host.  nmax bounds the rank; try_capped opens the leading-eigenpair route.
+// matrix G on the device, *b on the host.  nmax bounds the rank; try_capped opens the leading-eigenpair route.  dg
+// (optional): the digits the tcgen05 Gram made for G, whose exactness flag the same wait brings to the host.
 static int decide_bond(ndmps_ctx* ctx, double* G, int64_t m, int64_t nmax, const TrimOpts& opt, bool try_capped, double eig_tol,
-                       double* evals, double* U, Bond* b) {
+                       TcDigits* dg, double* evals, double* U, Bond* b) {
     *b = Bond();
-    if (try_capped) NDMPS_TRY(capped_eigh(ctx, G, m, nmax, opt, evals, U, b));
+    if (try_capped) NDMPS_TRY(capped_eigh(ctx, G, m, nmax, opt, dg, evals, U, b));
     if (b->n > 0) return NDMPS_OK;                       // the cap binds
     { StageScope sc(ctx, ST_EIG); NDMPS_TRY(eigh(ctx, G, m, evals, U, eig_tol)); }
-    NDMPS_TRY(read_back(ctx, evals, m));
+    NDMPS_TRY(read_back(ctx, evals, m, dg));
     b->sv.resize((size_t)m);
     for (int64_t i = 0; i < m; i++) b->sv[i] = ctx->pinned[i] > 0.0 ? sqrt(ctx->pinned[i]) : 0.0;
     b->n = n_keep(b->sv.data(), nmax, opt.cutoff, opt.mode, opt.max_bond);
@@ -295,6 +296,9 @@ struct ShardCtl {
 struct Sweep {
     ndmps_ctx* ctx;
     int dtype;
+    // float32 payload with a bond cap: the long Gram and projection passes run on tcgen05 (tc_gemm.cu); the rank
+    // decisions of an UNCAPPED sweep sit at lambda / lambda_1 ~ 1e-10 and keep the exact FP64-pipe path
+    bool tc;
     const int64_t* dims;
     TrimOpts opt;
     double eig_tol;
@@ -327,7 +331,9 @@ static int row_group_step(const Sweep& s, const void* M, int64_t D, int64_t C, i
     const ShardCtl* sh = s.sh;
     double* G = nullptr;
     NDMPS_TRY(ctx->ws.get<double>((size_t)(D * D), &G));
-    { StageScope sc(ctx, ST_GRAM); NDMPS_TRY(gram(ctx, M, D, C, C, dtype, 0, G)); }
+    TcDigits digits;                                  // of M, when the Gram runs on the integer tensor cores
+    TcDigits* dg = s.tc ? &digits : nullptr;
+    { StageScope sc(ctx, ST_GRAM); NDMPS_TRY(gram(ctx, M, D, C, C, dtype, 0, G, dg)); }
     if (sh && sh->world > 1) {
         const int rc_hook = sh->allreduce(sh->user, G, D * D, (void*)ctx->stream);
         if (rc_hook != 0) { set_error("ttsvd: the allreduce hook failed (%d)", rc_hook); return NDMPS_ERR_CUDA; }
@@ -360,7 +366,7 @@ static int row_group_step(const Sweep& s, const void* M, int64_t D, int64_t C, i
         NDMPS_TRY(ctx->ws.get<double>((size_t)(mj * mj), &U));
         const int64_t cols_j = C * rest * (sh ? sh->world : 1);     // the rank is at most min(rows, cols)
         Bond b;
-        NDMPS_TRY(decide_bond(ctx, Gj, mj, mj < cols_j ? mj : cols_j, s.opt, true, s.eig_tol, evals, U, &b));
+        NDMPS_TRY(decide_bond(ctx, Gj, mj, mj < cols_j ? mj : cols_j, s.opt, true, s.eig_tol, dg, evals, U, &b));
         NDMPS_TRY(record_site(s, site + j, mj, b));
         NDMPS_TRY(scale_convert(ctx, U, mj, b.n, mj, nullptr, nullptr, 1.0, s.cores[site + j], dtype, b.n));
         // P_next = f * K * U[:, :n]   (X x n)
@@ -377,9 +383,9 @@ static int row_group_step(const Sweep& s, const void* M, int64_t D, int64_t C, i
     NDMPS_TRY(ctx->ws.alloc((size_t)(rc * C) * dtype_size(dtype), T));
     StageScope sc(ctx, ST_PROJECT);
     bool on_tc = false;
-    if (ctx->tc_sweep && C >= 2048) {
+    if (s.tc && C >= 2048) {
         // the digits the Gram of this step sliced, when it ran on the integer tensor cores (exact accumulation) ...
-        NDMPS_TRY(proj_tc_digits(ctx, M, D, C, C, P, rc, *T, dtype, C, &on_tc));
+        NDMPS_TRY(proj_tc_digits(ctx, digits, P, rc, *T, dtype, C, &on_tc));
         // ... else T^T = M^T P on bf16x3 planes: the unfolding is the MN-major operand, T leaves transposed
         if (!on_tc) NDMPS_TRY(gemm_tc(ctx, C, rc, D, 1.0, M, dtype, 1, C, P, NDMPS_F64, rc, 1, *T, dtype, C, true, &on_tc));
     }
@@ -406,7 +412,7 @@ static int column_step(const Sweep& s, const void* M, int64_t D, int64_t C, int 
     // the capped route leaves all but the k leading eigenvalues as they are; col_scale below reads all C
     NDMPS_CUDA_TRY(cudaMemsetAsync(evals, 0, (size_t)C * sizeof(double), ctx->stream));
     Bond b;
-    NDMPS_TRY(decide_bond(ctx, G, C, C, s.opt, true, s.eig_tol, evals, V, &b));   // rank <= min(D, C) = C
+    NDMPS_TRY(decide_bond(ctx, G, C, C, s.opt, true, s.eig_tol, nullptr, evals, V, &b));   // rank <= min(D, C) = C
     const int64_t n = b.n;
     NDMPS_TRY(record_site(s, site, D, b));
     double *inv_s = nullptr, *s_f = nullptr, *MV = nullptr;
@@ -439,11 +445,8 @@ static int ttsvd(ndmps_ctx* ctx, const void* dense, int dtype, int L, const int6
         return NDMPS_OK;
     }
     // cores stored in float32 need eigenvectors orthogonal to ~1e-8, not 1e-15: one sweep less
-    const Sweep s{ctx, dtype, dims, opt, dtype == NDMPS_F32 ? 1e-10 : 0.0, cores_out, core_cap, ranks_out, svals_out, svals_stride, sh};
-    // float32 payload with a bond cap: the long Gram and projection passes run on tcgen05 (tc_gemm.cu); the rank
-    // decisions of an UNCAPPED sweep sit at lambda / lambda_1 ~ 1e-10 and keep the exact FP64-pipe path
-    struct TcScope { ndmps_ctx* c; ~TcScope() { c->tc_sweep = false; } } tc_scope{ctx};
-    ctx->tc_sweep = ctx->opt_tc && dtype == NDMPS_F32 && opt.max_bond > 0;
+    const bool tc = ctx->opt_tc && dtype == NDMPS_F32 && opt.max_bond > 0;
+    const Sweep s{ctx, dtype, tc, dims, opt, dtype == NDMPS_F32 ? 1e-10 : 0.0, cores_out, core_cap, ranks_out, svals_out, svals_stride, sh};
     const void* M = dense;         // current remainder, (r_prev * remaining) elements
     int64_t r_prev = 1;
     int64_t remaining = total;     // elements of the remainder divided by r_prev
@@ -527,7 +530,7 @@ static int compress_bond(ndmps_ctx* ctx, const void* t1, const void* t2, int dty
     int64_t nmax = r < a ? r : a;
     if (b < nmax) nmax = b;
     Bond bond;
-    NDMPS_TRY(decide_bond(ctx, H, r, nmax, opt, false, 0.0, sig2, Up, &bond));
+    NDMPS_TRY(decide_bond(ctx, H, r, nmax, opt, false, 0.0, nullptr, sig2, Up, &bond));
     const int64_t n = bond.n;
     *new_rank = n;
     if (svals_out)
@@ -651,12 +654,7 @@ int right_chain(ndmps_ctx* ctx, const void* const* cores, int dtype, int L, int 
 
 // out (rows x cols) = X (rows x r) W (r x cols)
 int chain_product(ndmps_ctx* ctx, int64_t rows, int64_t cols, int64_t r, const void* X, const void* W, int dtype, void* out) {
-    if (ctx->opt_tc && dtype == NDMPS_F32 && rows * cols >= (int64_t(1) << 20)) {   // float32 payload: the one big product on tcgen05
-        bool on_tc = false;
-        NDMPS_TRY(gemm_tc(ctx, rows, cols, r, 1.0, X, dtype, r, 1, W, dtype, cols, 1, out, dtype, cols, false, &on_tc));
-        if (on_tc) return NDMPS_OK;
-    }
-    return gemm(ctx, rows, cols, r, 1.0, X, dtype, r, 1, W, dtype, cols, 1, out, dtype, cols);
+    return payload_gemm(ctx, rows * cols, rows, cols, r, X, dtype, r, 1, W, dtype, cols, 1, out, dtype, cols);
 }
 
 static int contract_dense(ndmps_ctx* ctx, const void* const* cores, int dtype, int L, const int64_t* dims,

@@ -9,6 +9,7 @@ seeded inputs.
 * the capped float32 sweep with and without the tensor-core kernels (`tc`): same bonds, singular values within 1e-8 of
   sigma_1, reconstructions within 1e-5 (the parity bar of the path)."""
 import ctypes as C
+import re
 
 import numpy as np
 import pytest
@@ -150,3 +151,59 @@ def test_capped_sweep_tc_on_off(lib, ctx, shape, chi):
     for s0, s1 in zip(o0.singular_values, o1.singular_values):
         assert np.max(np.abs(np.asarray(s0) - np.asarray(s1))) <= 1e-8 * np.asarray(s0)[0]
     assert float(torch.linalg.vector_norm((r1 - r0).double()) / torch.linalg.vector_norm(r0.double())) <= 1e-5
+
+
+# ---- the sweep's digit hand-off ------------------------------------------------------------------------------------
+def _sweep_kernels(ctx, v, **kw):
+    """NDMPS.from_tensor(v, **kw), the names of the CUDA kernels a trace of it recorded, and how many tcgen05 kernels it
+    launched (the library's own count: it holds even where the trace misses a record)."""
+    from imgcompressionmps.core.ndmps import NDMPS
+    launches0 = ctx.stat("tc_launches")
+    torch.cuda.synchronize()
+    with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
+        torch.cuda.synchronize()
+        obj = NDMPS.from_tensor(v, **kw)
+        torch.cuda.synchronize()
+    return obj, [e.name for e in prof.events()], ctx.stat("tc_launches") - launches0
+
+
+def test_capped_sweep_hands_the_gram_digits_to_its_projection(lib, ctx):
+    # (32, 64, 4096) -> sites [32, 16, 16, 16, 64]: the first group's unfolding is 512 x 16384, eligible for the
+    # sliced-integer Gram; every later unfolding has fewer than 2048 columns, so only the first step can use tcgen05:
+    # its Gram on kind::i8 and its projection, two tcgen05 launches
+    shape, chi = (32, 64, 4096), 16
+    rng = np.random.default_rng(5)
+    z, y, x = np.meshgrid(*[np.linspace(-1, 1, s) for s in shape], indexing="ij")
+    vol = (np.exp(-3 * (x * x + 0.5 * y * y + 2 * z * z)) + 0.3 * np.sin(5 * x + 3 * y) * np.cos(4 * z)
+           + 0.02 * rng.standard_normal(shape)).astype(np.float32)
+    smooth = torch.from_numpy(vol).cuda()
+    out_t = re.compile(r"gemm_tc_kernel<\d+, \d+, \w+, \w+, true, float>")    # bf16x3 product with transposed output
+
+    # smooth rows: five digits are exact, the projection multiplies the digits the Gram made
+    _, names, tc = _sweep_kernels(ctx, smooth, max_bond=chi)
+    assert tc == 2
+    for k in ("split_i8_proj_kernel", "proj_i8_kernel"):
+        assert any(k in n for n in names), f"{k} did not run; kernels: {names}"
+    assert not any(out_t.search(n) for n in names), names
+
+    # one element 1e4 x the RMS: its row is too heavy-tailed for five digits, the device flag hands the Gram to the
+    # FP64-pipe kernel and the projection to bf16x3 planes (the unfolding as the MN-major operand, T written transposed)
+    spiky = smooth.clone()
+    spiky[7, 33, 1000] = 1e4 * float(smooth.double().square().mean().sqrt())
+    obj1, names, tc = _sweep_kernels(ctx, spiky, max_bond=chi)
+    assert tc == 2
+    assert not any("proj_i8_kernel" in n or "split_i8_proj_kernel" in n for n in names), names
+    assert any(out_t.search(n) for n in names), names
+    # the Gram the exact kernel computed is the one the sweep without tcgen05 computes: same first bonds
+    ctx.set_option("tc", 0)
+    obj0, _, tc = _sweep_kernels(ctx, spiky, max_bond=chi)
+    ctx.set_option("tc", 1)
+    assert tc == 0
+    assert obj0.bond_sizes() == obj1.bond_sizes()
+    s0, s1 = np.asarray(obj0.singular_values[0]), np.asarray(obj1.singular_values[0])
+    assert np.max(np.abs(s0 - s1)) <= 1e-12 * s0[0]
+
+    # an uncapped sweep and a float64 one keep to the FP64 pipe: no kernel of tc_gemm.cu (namespace ndmps::tc) runs
+    for v, kw in ((smooth, {}), (smooth.double(), {"max_bond": chi})):
+        _, names, tc = _sweep_kernels(ctx, v, **kw)
+        assert tc == 0 and not any("ndmps::tc::" in n for n in names), names
